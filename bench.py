@@ -2,7 +2,7 @@
 """bench.py — KMC site-updates/s of the sublattice sweep on the 512^3 lattice (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cetkmc|reference]
-                    [--scaling strong|weak] [--L 512] [--thermal cet|laser]
+                    [--scaling strong|weak] [--L 512] [--thermal cet|laser] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one synchronous-sublattice sweep over the whole lattice (csrc/sweep.cu): thermal stencil
@@ -24,6 +24,12 @@ CUDA-event timing), roofline_all, cpu_baseline (the oracle port on the host core
 e2e (the sweep API call with host buffers, copies inside the timed region), api_e2e (the reference-
 signature calls run_kmc / update_temperature_cet / get_event_rates, host arrays in, host arrays out),
 clocks, gpu_launches.
+
+--dump-outputs DIR (N = 1) writes, after the timed sweeps, what they left on the device as DIR/<name>.npy:
+the lattice a caller of the sweep receives (state, defects, theta, phi, T) and the resident site rate sums
+at a fixed seeded sample of sites (site_index), the deposition rates of the top plane (dep_rate, 0 where a
+site offers no deposition), and the counters the timed sweep call returned (sweep_<name>).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -192,6 +198,34 @@ def pinned(shape, dtype):
         return np.empty(shape, dtype=dtype), None
 
 
+DUMP_SITES = 1 << 20            # sampled sites: 48 B each over 7 arrays, ~50 MB in all with dep_rate at 512^2
+
+
+def dump_outputs(ctx, res, out_dir):
+    """--dump-outputs: the resident lattice and rate sums at a fixed seeded sample of DUMP_SITES sites
+    (all of them on a smaller lattice), the deposition rates of the top plane, and the sweep counters.
+    Every value written is finite; a non-finite one is an error."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(np.prod(ctx.owned_shape))
+    idx = np.arange(n) if n <= DUMP_SITES else np.unique(np.random.default_rng(0).integers(0, n, DUMP_SITES))
+    packed = ctx.download_packed().reshape(-1)[idx]
+    out = {"site_index": idx.astype(np.float64), "state": (packed & 15).astype(np.float32),
+           "defects": (packed >> 4).astype(np.float32)}
+    for name in ("theta", "phi", "T"):
+        out[name] = ctx.download(**{name: True})[name].reshape(-1)[idx]
+    sr, dr = ctx.rates_download()
+    # the device marks a top-plane site without a deposition event (occupied, or rate at or below the
+    # threshold) with NaN; such a site offers rate 0, as kmc_exact.cu reads it
+    out["site_rate_sum"], out["dep_rate"] = sr.reshape(-1)[idx], np.where(np.isnan(dr), 0.0, dr)
+    for k, v in res.items():
+        out["sweep_" + k] = np.float64(v)
+    bad = [name for name, a in out.items() if not np.all(np.isfinite(a))]
+    if bad:
+        raise RuntimeError(f"--dump-outputs: non-finite values in {bad}")
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def api_e2e():
     """The reference-signature calls (host NumPy arrays in, host NumPy arrays out), wall clock around
     the call as a user makes it: run_kmc at the main.py default lattice, update_temperature_cet at
@@ -253,7 +287,10 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-api-e2e", action="store_true")
     ap.add_argument("--debug-flags", type=int, default=0, help="refresh variant for A/B runs (cet_debug_flags)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed sweeps computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -264,6 +301,8 @@ def main():
             raise SystemExit("launch with torch.distributed.run --nproc-per-node N for --gpus N")
     if args.thermal == "laser" and world > 1:
         raise SystemExit("--thermal laser is the single-GPU configuration (BASELINE configs[2])")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs is the single-GPU configuration")
     warm = max(args.warmup, 3)
 
     import cetkmc
@@ -333,11 +372,10 @@ def main():
             if laser:
                 laser_step()
             r = ctx.sweep_run(blk, sp, tp)
-            if tot is None:
-                tot = dict(r)
-            else:
+            if tot is not None:                     # counts add up over the blocks; the clock is the last block's
                 for k in ("events_applied", "events_fired", "sites_refreshed", "sweeps_done"):
-                    tot[k] += r[k]
+                    r[k] += tot[k]
+            tot = r
             done += blk
         return tot
 
@@ -366,6 +404,8 @@ def main():
     clocks = sampler.stop()
     ctx.profile_enable(False)
     barrier()
+    if args.dump_outputs:
+        dump_outputs(ctx, res, args.dump_outputs)
     if dist is not None:
         import torch
         t = torch.tensor([ms], dtype=torch.float64, device="cuda")

@@ -101,6 +101,8 @@ SIGNATURES = {
     "cet_sweep_set_state": [_VP, _I64, _F64, _F64],
     "cet_sweep_run": [_VP, _I64, C.POINTER(SweepParams), C.POINTER(ThermalParams),
                       C.POINTER(SweepResult)],
+    "cet_sweep_run_group": [C.POINTER(_VP), _I32, _I64, C.POINTER(SweepParams), C.POINTER(ThermalParams),
+                            C.POINTER(SweepResult)],
     "cet_comm_unique_id": [_VP],
     "cet_comm_init": [_VP, _VP, C.c_int, C.c_int],
     "cet_comm_destroy": [_VP],
@@ -496,6 +498,33 @@ class Context:
         ms = C.c_float(0.0)
         check(lib().cet_timer_end_ms(self._h, C.byref(ms)), "cet_timer_end_ms")
         return ms.value
+
+
+GROUP_MAX = 64                                      # cet_sweep_run_group's limit on n_ctx
+
+
+def sweep_run_group(ctxs, n_sweeps, sps, tps=None):
+    """Advance the lattices of `ctxs` (whole-lattice Contexts of one L on one device) by n_sweeps sweeps each,
+    with one launch per kernel for the whole group.  sps: one SweepParams per context; tps: one
+    ThermalParams per context, or None when no context has a thermal step.  Every context ends exactly as
+    its own ctx.sweep_run(n_sweeps, sps[q], tps[q]) would leave it.  Returns one result dict per context,
+    with the keys of Context.sweep_run."""
+    ctxs, sps = list(ctxs), list(sps)
+    n = len(ctxs)
+    if len(sps) != n:
+        raise ValueError(f"sweep_run_group: {len(sps)} sweep params for {n} contexts")
+    if tps is not None:
+        tps = list(tps)
+        if len(tps) != n:
+            raise ValueError(f"sweep_run_group: {len(tps)} thermal params for {n} contexts")
+    if any(not isinstance(c, Context) for c in ctxs):
+        raise TypeError("sweep_run_group: ctxs must be Context objects")
+    handles = (C.c_void_p * n)(*[c._h.value for c in ctxs])
+    sp_arr = (SweepParams * n)(*sps)
+    tp_arr = None if tps is None else (ThermalParams * n)(*tps)
+    res = (SweepResult * n)()
+    check(lib().cet_sweep_run_group(handles, n, int(n_sweeps), sp_arr, tp_arr, res), "cet_sweep_run_group")
+    return [{f: getattr(r, f) for f, _ in SweepResult._fields_ if f != "pad_"} for r in res]
 
 
 def comm_unique_id() -> bytes:

@@ -111,6 +111,54 @@ def _slab_comm(world):
     return all_gather, bcast_bytes
 
 
+def _upload_initial(ctx, L, n_seeds, temp, impurity_c, lattice, i_begin, i_end):
+    """The run's initial lattice on the device: initialize_lattice + introduce_defects (NumPy's global stream,
+    seeded by the caller), or the given `lattice`."""
+    if lattice is None:
+        state, theta, phi, T, atom_type = _ks.initialize_lattice(lattice_size=L, n_seeds=n_seeds, T_sub=temp,
+                                                                 impurity_c=impurity_c)
+        defects_mask, _ = _ks.introduce_defects(state, atom_type, T, apply_to_state=False)
+    else:
+        state, theta, phi, T, atom_type = lattice[:5]
+        defects_mask = lattice[5] if len(lattice) > 5 else None
+    own = slice(i_begin, i_end)
+    ctx.upload(state=np.ascontiguousarray(state[own], dtype=np.int64), theta=theta[own], phi=phi[own], T=T[own],
+               defects=None if defects_mask is None else defects_mask[own])
+
+
+def _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction, thermal_every):
+    """Sweep and thermal parameters of a run (thermal_every 0: no update_temperature_cet in the sweeps)."""
+    sp = _lib.SweepParams()
+    sp.seed = seed
+    sp.events_per_sweep = float(events_per_sweep if events_per_sweep is not None else 0.005 * L ** 3)
+    sp.p_max, sp.defect_fraction = float(p_max), float(defect_fraction)
+    sp.thermal_every = int(thermal_every)
+    tp = None if not thermal_every else thermal_params(_ks.THERMAL_DT, nan_to_num=True, t_floor=temp)
+    return sp, tp
+
+
+def _stop_at(sweep, every, n_sweeps):
+    """The last sweep of the next metrics interval (run_kmc's cadence)."""
+    return min(((sweep + every - 1) // every) * every, n_sweeps - 1)
+
+
+def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_count, cet_detected, consts,
+             verbose, all_gather=None):
+    """What follows the sweeps of a metrics interval that ended at sweep `last`: the defect-mask refresh on
+    multiples of `every` (kmc_simulation.py:335-338) and the metrics row.  Returns (row, cet_detected)."""
+    if last % every == 0:
+        if not philox_mask:
+            _defects.refresh_resident(ctx)
+        else:
+            ctx.defects_refresh(draws=None, seed=seed, epoch=last // every, prob_base=constants.DEFECT_PROB_BASE,
+                                e_mig=_defects.E_MIGRATION, kT=constants.K_T, T_default=constants.T_SUB,
+                                carbon_id=_defects.CARBON_ID, defect_id=constants.DEFECT_ID)
+            if world > 1:
+                ctx.halo_exchange(1)                                          # the ghost copies of the mask nibble
+    return _ks._metrics_row(last, total_time, nucleation_count, cet_detected, consts, ctx, verbose=verbose,
+                            all_gather=all_gather)
+
+
 def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_seeds=5, impurity_c=0.0,
                        output_prefix="cet_sublattice", metrics_every=None, events_per_sweep=None, p_max=0.1,
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
@@ -164,26 +212,12 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             nucleation_count, cet_detected = int(meta.get("nucleation_count", 0)), bool(meta.get("cet_detected", False))
             rows = list(meta.get("rows", []))
         else:
-            if lattice is None:
-                state, theta, phi, T, atom_type = _ks.initialize_lattice(lattice_size=L, n_seeds=n_seeds, T_sub=temp,
-                                                                         impurity_c=impurity_c)
-                defects_mask, _ = _ks.introduce_defects(state, atom_type, T, apply_to_state=False)
-            else:
-                state, theta, phi, T, atom_type = lattice[:5]
-                defects_mask = lattice[5] if len(lattice) > 5 else None
-            own = slice(i_begin, i_end)
-            ctx.upload(state=np.ascontiguousarray(state[own], dtype=np.int64), theta=theta[own], phi=phi[own], T=T[own],
-                       defects=None if defects_mask is None else defects_mask[own])
+            _upload_initial(ctx, L, n_seeds, temp, impurity_c, lattice, i_begin, i_end)
         if world > 1:
             all_gather, bcast_bytes = _slab_comm(world)
             ctx.comm_init(bcast_bytes(_lib.comm_unique_id() if rank == 0 else None), rank, world)
             ctx.halo_exchange(7)
-        sp = _lib.SweepParams()
-        sp.seed = seed
-        sp.events_per_sweep = float(events_per_sweep if events_per_sweep is not None else 0.005 * L ** 3)
-        sp.p_max, sp.defect_fraction = float(p_max), float(defect_fraction)
-        sp.thermal_every = 0 if laser else int(thermal_every)
-        tp = None if laser else thermal_params(_ks.THERMAL_DT, nan_to_num=True, t_floor=temp)
+        sp, tp = _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction, 0 if laser else thermal_every)
         if laser and int(thermal_every) <= 0:
             raise ValueError("run_cet_sublattice: the laser variant needs thermal_every >= 1")
         if laser:
@@ -217,21 +251,10 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             ctx.snapshot_state()
         terminated = False
         while sweep < n_sweeps and not terminated:
-            stop_at = min(((sweep + every - 1) // every) * every, n_sweeps - 1)      # run_kmc's cadence
-            done, terminated = advance(stop_at - sweep + 1)
+            done, terminated = advance(_stop_at(sweep, every, n_sweeps) - sweep + 1)
             sweep += done
-            last = sweep - 1
-            if last % every == 0:                                                     # kmc_simulation.py:335-338
-                if not philox_mask:
-                    _defects.refresh_resident(ctx)
-                else:
-                    ctx.defects_refresh(draws=None, seed=seed, epoch=last // every, prob_base=constants.DEFECT_PROB_BASE,
-                                        e_mig=_defects.E_MIGRATION, kT=constants.K_T, T_default=constants.T_SUB,
-                                        carbon_id=_defects.CARBON_ID, defect_id=constants.DEFECT_ID)
-                    if world > 1:
-                        ctx.halo_exchange(1)                                          # the ghost copies of the mask nibble
-            row, cet_detected = _ks._metrics_row(last, total_time, nucleation_count, cet_detected, consts, ctx,
-                                                 verbose=verbose and rank == 0, all_gather=all_gather)
+            row, cet_detected = _cadence(ctx, sweep - 1, every, philox_mask, seed, world, total_time, nucleation_count,
+                                         cet_detected, consts, verbose=verbose and rank == 0, all_gather=all_gather)
             rows.append(row)
             if checkpoint_every and (len(rows) % checkpoint_every == 0):
                 checkpoint(ctx, os.path.join(output_dir, "checkpoint"), sweep=sweep, time=total_time,
@@ -245,41 +268,120 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     return f["state"], f["atom_type"], total_time, f["theta"], f["phi"]
 
 
+def gr_partition(n_cases, rank, world, devices, batch=None):
+    """Which cases of a G-R sweep this rank runs, where, and together with which: a list of
+    (device, [case numbers]).  Case q belongs to rank q % world and runs on devices[(q // world) % len(devices)];
+    batch=None runs every case on its own, batch=k the cases of one device in groups of up to k lattices
+    (in case order)."""
+    mine = [q for q in range(n_cases) if q % world == rank]
+    if batch is None:
+        return [(devices[(q // world) % len(devices)], [q]) for q in mine]
+    if int(batch) < 1 or int(batch) > _lib.GROUP_MAX:
+        raise ValueError(f"run_gr_sweep: batch must be 1 to {_lib.GROUP_MAX}, got {batch}")
+    by_dev = {}
+    for q in mine:
+        by_dev.setdefault(devices[(q // world) % len(devices)], []).append(q)
+    return [(d, qs[i:i + int(batch)]) for d, qs in by_dev.items() for i in range(0, len(qs), int(batch))]
+
+
 def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20, defect_fraction=0.0,
-                 output_root="gr_sweep", rank=None, world=None, devices=None, **kw):
+                 output_root="gr_sweep", rank=None, world=None, devices=None, batch=None, **kw):
     """SURVEY §8d config 5: one independent lattice per (T_sub, NU_DEP) grid point — T_sub sets the
     thermal gradient G = (T_MELT - T_sub) / (L dx), NU_DEP the growth velocity R (kmc_simulation.py:
     236-239).  Replicas only: case q runs on rank q % world (torchrun: RANK / WORLD_SIZE / LOCAL_RANK)
     or, in a single process, on device q % len(devices).  Every case writes its own metrics.csv; the
     rank that owns a case appends its final row to outputs/<output_root>/cet_map_rank<r>.csv, and
     merge_cet_map() joins them into cet_map.csv (columns G, R, G_over_R, AspectRatio,
-    EquiaxedFraction, GrainCount, CET_Class, ...)."""
+    EquiaxedFraction, GrainCount, CET_Class, ...).
+    batch=k: the cases of one device advance in groups of up to k lattices, one kernel launch per group
+    and kernel (cetkmc.sweep_run_group) instead of one per lattice; every output file is the same as
+    with batch=None.  Not with `laser`, `checkpoint_every`, `resume_from` or `lattice`."""
     rank = int(os.environ.get("RANK", 0)) if rank is None else rank
     world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
     local = int(os.environ.get("LOCAL_RANK", 0))
     devices = [local] if devices is None else list(devices)
+    if batch is not None:
+        bad = [k for k in ("laser", "checkpoint_every", "resume_from", "lattice") if kw.get(k)]
+        if bad:
+            raise ValueError(f"run_gr_sweep: batch does not take {', '.join(bad)}")
     cases = [(float(t), float(r)) for t in temps for r in nu_deps]
     out_dir = f"outputs/{output_root}"
     os.makedirs(out_dir, exist_ok=True)
+    prefix = [f"{output_root}/T{temp:g}_R{nu_dep:g}" for temp, nu_dep in cases]
+    for device, qs in gr_partition(len(cases), rank, world, devices, batch):
+        if batch is None:
+            q = qs[0]
+            run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=cases[q][0], nu_dep=cases[q][1], impurity_c=impurity_c,
+                               n_seeds=n_seeds, defect_fraction=defect_fraction, output_prefix=prefix[q],
+                               device=device, verbose=False, **kw)
+        else:
+            _run_cases_grouped([(prefix[q],) + cases[q] for q in qs], L=L, n_sweeps=n_sweeps, impurity_c=impurity_c,
+                               n_seeds=n_seeds, defect_fraction=defect_fraction, device=device, **kw)
+    import csv
     rows = []
-    for q, (temp, nu_dep) in enumerate(cases):
-        if q % world != rank:
-            continue
-        prefix = f"{output_root}/T{temp:g}_R{nu_dep:g}"
-        run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=temp, nu_dep=nu_dep, impurity_c=impurity_c, n_seeds=n_seeds,
-                           defect_fraction=defect_fraction, output_prefix=prefix,
-                           device=devices[(q // world) % len(devices)], verbose=False, **kw)
-        import csv
-        with open(f"outputs/{prefix}/metrics.csv") as fh:
+    for q in (q for _d, qs in gr_partition(len(cases), rank, world, devices, batch) for q in qs):
+        temp, nu_dep = cases[q]
+        with open(f"outputs/{prefix[q]}/metrics.csv") as fh:
             last = list(csv.DictReader(fh))[-1]
         G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
         rows.append({"case": q, "T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R, "G_over_R": G / R if R > 0 else np.inf,
                      **{k: last[k] for k in ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize",
                                              "NucleationCount", "CET_Class", "CET_Detected")}})
+    rows.sort(key=lambda r: r["case"])
     _write_rows(rows, os.path.join(out_dir, f"cet_map_rank{rank}.csv"))
     write_plot_cet_tree([(r["case"], f"outputs/{output_root}/T{r['T_sub']:g}_R{r['NU_DEP']:g}/metrics.csv") for r in rows],
                         os.path.join(out_dir, "plot_cet"))
     return rows
+
+
+def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
+                       events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy"):
+    """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
+    lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
+    alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
+    around its host draws).  A case that terminates stops at the row it stops at alone and leaves the group."""
+    if mask_stream not in ("numpy", "philox"):
+        raise ValueError("mask_stream must be 'numpy' or 'philox'")
+    seed = constants.RANDOM_SEED if seed is None else int(seed)
+    every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
+    philox_mask = mask_stream == "philox"
+    runs = []
+    try:
+        for prefix, temp, nu_dep in cases:
+            np.random.seed(seed)
+            os.makedirs(f"outputs/{prefix}", exist_ok=True)
+            ctx = _lib.Context(L=L, device=device)
+            r = dict(ctx=ctx, prefix=prefix, consts=_gr(L, temp, nu_dep), rows=[], total_time=0.0, nucleation_count=0,
+                     cet_detected=False, terminated=False)
+            runs.append(r)
+            ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
+            _upload_initial(ctx, L, n_seeds, temp, impurity_c, None, 0, L)
+            r["sp"], r["tp"] = _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction, thermal_every)
+            r["rng"] = np.random.get_state()
+        sweep = 0
+        active = runs
+        while sweep < n_sweeps and active:
+            n = _stop_at(sweep, every, n_sweeps) - sweep + 1
+            tps = None if active[0]["tp"] is None else [r["tp"] for r in active]     # one thermal_every for all cases
+            results = _lib.sweep_run_group([r["ctx"] for r in active], n, [r["sp"] for r in active], tps)
+            sweep += n
+            for r, res in zip(active, results):
+                if res["overflow"]:
+                    raise RuntimeError("fired-event list overflowed: lower events_per_sweep")
+                r["total_time"] += res["time"]
+                r["nucleation_count"] += res["nucleation_count"]
+                r["terminated"] = bool(res["terminated"]) or res["sweeps_done"] == 0
+                np.random.set_state(r["rng"])
+                row, r["cet_detected"] = _cadence(r["ctx"], sweep - 1, every, philox_mask, seed, 1, r["total_time"],
+                                                  r["nucleation_count"], r["cet_detected"], r["consts"], verbose=False)
+                r["rng"] = np.random.get_state()
+                r["rows"].append(row)
+            active = [r for r in active if not r["terminated"]]
+        for r in runs:
+            _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
+    finally:
+        for r in runs:
+            r["ctx"].close()
 
 
 def write_plot_cet_tree(cases, root):

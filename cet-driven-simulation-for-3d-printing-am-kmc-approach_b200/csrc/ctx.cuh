@@ -68,6 +68,18 @@ struct SweepState {
 static_assert(offsetof(SweepState, n_fired) == 128 && offsetof(SweepState, sum_rate) == 256 && sizeof(SweepState) == 384,
               "SweepState: one 128-byte line per access class");
 
+// Grouped sweeps (cet_sweep_run_group): one launch covers the lattices of a group, and a CTA takes the
+// arguments of its lattice (blockIdx.z, or blockIdx.x for the one-CTA kernels) from a table passed by value
+// in kernel parameter space (32 KB).  CAP is the table's capacity: a launch copies the whole table, so a
+// small group uses the small one.
+constexpr int GROUP_MAX = 64;
+template <class T, int CAP>
+struct GroupArgs {
+    T a[CAP];
+};
+template <class T>
+constexpr bool group_fits() { return sizeof(GroupArgs<T, GROUP_MAX>) <= 32764; }
+
 }  // namespace cet
 
 // Device-memory layout (all arrays cover local planes [0, np) where np = ni + 2*halo and local

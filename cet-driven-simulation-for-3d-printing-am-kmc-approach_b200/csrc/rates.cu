@@ -41,6 +41,7 @@ __global__ void dirty_eval_kernel(const __grid_constant__ RateTileArgs a, const 
                                   unsigned int *queue);
 
 int rates_refresh_list(cet_ctx *c, const int32_t *list, const unsigned int *counter, int64_t nsite_hint);     // rates_refresh.cu
+int rates_refresh_list_group(cet_ctx *const *cs, int n, int64_t nsite_hint, int *blocks_per_sm);
 
 int rate_tables_ensure(cet_ctx *c)
 {
@@ -128,7 +129,7 @@ struct DirtyArgs {
 
 constexpr int DS_STAGE = 2048;     // staged list entries per CTA (256 words = 8192 sites)
 
-__global__ void __launch_bounds__(RB_WARPS * 32) dirty_scan_kernel(const __grid_constant__ DirtyArgs a)
+__device__ __forceinline__ void dirty_scan_body(const DirtyArgs &a)
 {
     __shared__ int s_list[DS_STAGE];                                // staging; spills are appended directly
     __shared__ unsigned int c_list, b_list, s_first_spill;
@@ -175,6 +176,13 @@ __global__ void __launch_bounds__(RB_WARPS * 32) dirty_scan_kernel(const __grid_
     if (threadIdx.x == 0) b_list = n ? atomicAdd(a.n_list, n) : 0u;
     __syncthreads();
     for (unsigned int q = threadIdx.x; q < n; q += RB_WARPS * 32) a.list[b_list + q] = s_list[q];
+}
+__global__ void __launch_bounds__(RB_WARPS * 32) dirty_scan_kernel(const __grid_constant__ DirtyArgs a) { dirty_scan_body(a); }
+// grouped sweeps: grid (CTAs per lattice, 1, lattices)
+template <int CAP>
+__global__ void __launch_bounds__(RB_WARPS * 32) dirty_scan_group_kernel(const __grid_constant__ GroupArgs<DirtyArgs, CAP> g)
+{
+    dirty_scan_body(g.a[blockIdx.z]);
 }
 
 __global__ void __launch_bounds__(RT_THREADS, 5) dirty_eval_kernel(const __grid_constant__ RateTileArgs a, const int32_t *list,
@@ -399,15 +407,21 @@ int rates_rows_compact(cet_ctx *c, int p_lo, int p_hi)
     return 0;
 }
 
+static DirtyArgs dirty_args(const cet_ctx *c, int p_lo, int p_hi, const uint32_t *stamp, int32_t *list, unsigned int *counter)
+{
+    DirtyArgs d;
+    d.stamp = stamp; d.s_lo = (int)(p_lo * c->plane); d.s_hi = (int)(p_hi * c->plane);
+    d.list = list; d.n_list = counter;
+    return d;
+}
+
 // Re-evaluate, on local planes [p_lo, p_hi), the sites whose stamp bit is set — from cvox / pairop.
 int rates_rows_dirty_compact(cet_ctx *c, int p_lo, int p_hi, const uint32_t *stamp, int32_t *list, unsigned int *counter)
 {
     if (p_hi <= p_lo) return 0;
     CompactArgs a;
     if (int rc = compact_args(c, a)) return rc;
-    DirtyArgs d;
-    d.stamp = stamp; d.s_lo = (int)(p_lo * c->plane); d.s_hi = (int)(p_hi * c->plane);
-    d.list = list; d.n_list = counter;
+    const DirtyArgs d = dirty_args(c, p_lo, p_hi, stamp, list, counter);
     const int n_words = ((d.s_hi + 31) >> 5) - (d.s_lo >> 5);
     dirty_scan_kernel<<<(n_words + RB_WARPS * 32 - 1) / (RB_WARPS * 32), RB_WARPS * 32, 0, c->stream>>>(d);
     CET_CUDA(cudaGetLastError());
@@ -420,6 +434,26 @@ int rates_rows_dirty_compact(cet_ctx *c, int p_lo, int p_hi, const uint32_t *sta
     dirty_eval_compact_kernel<<<grid, RT_THREADS, sizeof(CompactSmem), c->stream>>>(a, list, counter, queue);
     CET_CUDA(cudaGetLastError());
     return 0;
+}
+
+// rates_rows_dirty_compact for a group of contexts of one L (grouped sweeps, sweep.cu): one scan launch, then one
+// refresh launch, on the stream of cs[0].  Every context's refresh queue has been cleared by the sweep's reset.
+template <int CAP>
+static int dirty_scan_group(cet_ctx *const *cs, int n, int p_lo, int p_hi)
+{
+    GroupArgs<DirtyArgs, CAP> g;
+    for (int q = 0; q < n; ++q) g.a[q] = dirty_args(cs[q], p_lo, p_hi, cs[q]->stamp, cs[q]->dirty, &cs[q]->sweep->n_dirty);
+    const int n_words = ((g.a[0].s_hi + 31) >> 5) - (g.a[0].s_lo >> 5);
+    dirty_scan_group_kernel<CAP><<<dim3((unsigned)((n_words + RB_WARPS * 32 - 1) / (RB_WARPS * 32)), 1, (unsigned)n), RB_WARPS * 32, 0,
+                                   cs[0]->stream>>>(g);
+    CET_CUDA(cudaGetLastError());
+    return 0;
+}
+int rates_rows_dirty_compact_group(cet_ctx *const *cs, int n, int p_lo, int p_hi, int *refresh_blocks)
+{
+    if (p_hi <= p_lo) return 0;
+    if (int rc = n <= 16 ? dirty_scan_group<16>(cs, n, p_lo, p_hi) : dirty_scan_group<GROUP_MAX>(cs, n, p_lo, p_hi)) return rc;
+    return rates_refresh_list_group(cs, n, (int64_t)(p_hi - p_lo) * cs[0]->plane, refresh_blocks);
 }
 
 // One warp per local plane: plane-segment sums in list order.

@@ -16,6 +16,7 @@
 //           order with the sum in a register (pair_walk.cuh).
 // Same inline arithmetic as every other rate kernel: the result equals a dense rebuild bit for bit (tested).
 #include <algorithm>
+#include <memory>
 #include "ctx.cuh"
 #include "pair_walk.cuh"
 #include "tile_state.cuh"
@@ -108,7 +109,7 @@ __device__ __forceinline__ double rf_pairs(const cet_rate_params &P, const doubl
 }
 
 template <int ROWS>
-__global__ void __launch_bounds__(RF_THREADS, 4) rates_refresh_kernel(const __grid_constant__ RefreshArgs a)
+__device__ __forceinline__ void rates_refresh_body(const RefreshArgs &a)
 {
     constexpr int RF_CHUNK = RF_WARPS * ROWS * 32, RF_ROWS = ROWS;
     extern __shared__ __align__(16) unsigned char refresh_dyn_smem[];
@@ -258,6 +259,14 @@ __global__ void __launch_bounds__(RF_THREADS, 4) rates_refresh_kernel(const __gr
         __syncthreads();                                           // the lists may be overwritten
     }
 }
+template <int ROWS>
+__global__ void __launch_bounds__(RF_THREADS, 4) rates_refresh_kernel(const __grid_constant__ RefreshArgs a) { rates_refresh_body<ROWS>(a); }
+// grouped sweeps: grid (CTAs per lattice, 1, lattices); each lattice's CTAs pop chunks of its own list from its own queue
+template <int ROWS, int CAP>
+__global__ void __launch_bounds__(RF_THREADS, 4) rates_refresh_group_kernel(const __grid_constant__ GroupArgs<RefreshArgs, CAP> g)
+{
+    rates_refresh_body<ROWS>(g.a[blockIdx.z]);
+}
 
 template <int ROWS>
 static int refresh_launch(cet_ctx *c, const RefreshArgs &a, int64_t nsite_hint, int *blocks_per_sm)
@@ -277,10 +286,8 @@ static int refresh_launch(cet_ctx *c, const RefreshArgs &a, int64_t nsite_hint, 
     return 0;
 }
 
-// Re-evaluate the sites listed in `list` (length *counter, produced by dirty_scan_kernel) from cvox / pairop.
-int rates_refresh_list(cet_ctx *c, const int32_t *list, const unsigned int *counter, int64_t nsite_hint)
+static RefreshArgs refresh_args(const cet_ctx *c, const int32_t *list, const unsigned int *counter)
 {
-    if (int rc = rate_tables_ensure(c)) return rc;
     RefreshArgs a;
     memset(&a, 0, sizeof(a));
     a.cvox = c->cvox; a.pairop = c->pairop; a.T = c->T;
@@ -294,12 +301,52 @@ int rates_refresh_list(cet_ctx *c, const int32_t *list, const unsigned int *coun
     a.mLL = (unsigned int)((1ull << 32) / (uint64_t)c->plane) + 1u;
     a.mL = (unsigned int)((1ull << 32) / (uint64_t)c->n1) + 1u;
     for (int o = 0; o < 14; ++o) a.lin[o] = (h_nb_off[o][0] * a.L + h_nb_off[o][1]) * a.L + h_nb_off[o][2];
+    return a;
+}
+
+// Re-evaluate the sites listed in `list` (length *counter, produced by dirty_scan_kernel) from cvox / pairop.
+int rates_refresh_list(cet_ctx *c, const int32_t *list, const unsigned int *counter, int64_t nsite_hint)
+{
+    if (int rc = rate_tables_ensure(c)) return rc;
+    const RefreshArgs a = refresh_args(c, list, counter);
     CET_CUDA(cudaMemsetAsync(a.queue, 0, sizeof(unsigned int), c->stream));
     // stamped sites per CTA and queue entry: 512 (default), 256 / 1024 by debug flag 1048576 / 2097152
     const int v = (c->debug_flags & 1048576) ? 0 : (c->debug_flags & 2097152) ? 2 : 1;
     if (v == 0) return refresh_launch<1>(c, a, nsite_hint, &c->refresh_blocks[0]);
     if (v == 2) return refresh_launch<4>(c, a, nsite_hint, &c->refresh_blocks[2]);
     return refresh_launch<2>(c, a, nsite_hint, &c->refresh_blocks[1]);
+}
+
+// rates_refresh_list for a group of contexts of one L (grouped sweeps): each context's stamped-site list and the
+// queue its CTAs pop chunks from (cleared by the sweep's reset kernel); the list lengths are read on the device.
+// The CTAs resident on the device are shared out evenly; which CTA evaluates a chunk does not change the result.
+template <int CAP>
+static int refresh_group_launch(cet_ctx *const *cs, int n, int64_t nsite_hint, int *blocks_per_sm)
+{
+    constexpr int ROWS = 2, CHUNK = RF_WARPS * ROWS * 32;
+    const size_t smem = sizeof(RefreshSmem<ROWS>);
+    static_assert(group_fits<RefreshArgs>(), "a table of GROUP_MAX entries must fit the kernel parameter space");
+    cet_ctx *c0 = cs[0];
+    if (*blocks_per_sm == 0) {
+        CET_CUDA(cudaFuncSetAttribute(rates_refresh_group_kernel<ROWS, CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int nb = 0;
+        CET_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rates_refresh_group_kernel<ROWS, CAP>, RF_THREADS, smem));
+        CET_REQUIRE(nb >= 1, "rates_refresh_group_kernel does not fit an SM");
+        *blocks_per_sm = nb;
+    }
+    GroupArgs<RefreshArgs, CAP> g;
+    for (int q = 0; q < n; ++q) g.a[q] = refresh_args(cs[q], cs[q]->dirty, &cs[q]->sweep->n_dirty);
+    const int64_t per_ctx = std::max<int64_t>(1, ((int64_t)sm_count(c0) * *blocks_per_sm + n - 1) / n);
+    const int grid = (int)std::min<int64_t>((nsite_hint + CHUNK - 1) / CHUNK, per_ctx);
+    rates_refresh_group_kernel<ROWS, CAP><<<dim3((unsigned)grid, 1, (unsigned)n), RF_THREADS, smem, c0->stream>>>(g);
+    CET_CUDA(cudaGetLastError());
+    return 0;
+}
+// blocks_per_sm: the grouped kernel's occupancy, queried on first use (a group call keeps it for all its sweeps)
+int rates_refresh_list_group(cet_ctx *const *cs, int n, int64_t nsite_hint, int *blocks_per_sm)
+{
+    return n <= 16 ? refresh_group_launch<16>(cs, n, nsite_hint, blocks_per_sm)
+                   : refresh_group_launch<GROUP_MAX>(cs, n, nsite_hint, blocks_per_sm);
 }
 
 }  // namespace cet

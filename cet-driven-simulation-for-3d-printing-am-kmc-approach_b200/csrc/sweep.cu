@@ -30,6 +30,7 @@
 // are rebuilt densely (6 planes per cut face).  Plane sums are combined in a fixed order so the trajectory is independent of the
 // number of slabs.
 #include <algorithm>
+#include <memory>
 #include "ctx.cuh"
 #include "rate_tile.cuh"
 #include "reduce.cuh"
@@ -57,6 +58,11 @@ int rates_rows_compact(cet_ctx *c, int p_lo, int p_hi);
 int comm_sweep_reduce_join(cet_ctx *c);                                           // comm.cu
 int rates_rows_dense(cet_ctx *c, int p_lo, int p_hi);                            // rates_dense.cu
 int rate_tables_ensure(cet_ctx *c);
+int rates_rows_dirty_compact_group(cet_ctx *const *cs, int n, int p_lo, int p_hi, int *refresh_blocks);  // rates.cu
+int rates_rows_dense_group(cet_ctx *const *cs, int n, int *blocks_per_sm);          // rates_dense.cu
+unsigned int *dense_queue(cet_ctx *c);
+int thermal_cet_step_group(cet_ctx *const *cs, const cet_thermal_params *const *tps, int n);   // thermal.cu
+int tile_pairop_T_update_group(cet_ctx *const *cs, int n);                          // sweep_tile.cu
 
 struct Record {          // one fired event
     int32_t src;         // local linear index of the source site
@@ -122,7 +128,9 @@ __device__ __forceinline__ void stream_append(const StreamArgs &a, int *s_list, 
     else a.ss->overflow = 1;
 }
 
-__global__ void __launch_bounds__(ST_THREADS, 6) sweep_stream_kernel(const __grid_constant__ StreamArgs a)
+// The kernel bodies below take their arguments by reference: the solo kernels pass their own parameter, the
+// grouped kernels (cet_sweep_run_group) the table entry of their lattice, so both run the same instructions.
+__device__ __forceinline__ void sweep_stream_body(const StreamArgs &a)
 {
     __shared__ double s_sum[ST_THREADS / 32], s_max[ST_THREADS / 32];
     __shared__ int s_list[ST_STAGE];
@@ -235,6 +243,12 @@ __global__ void __launch_bounds__(ST_THREADS, 6) sweep_stream_kernel(const __gri
         else a.ss->overflow = 1;
     }
 }
+__global__ void __launch_bounds__(ST_THREADS, 6) sweep_stream_kernel(const __grid_constant__ StreamArgs a) { sweep_stream_body(a); }
+template <int CAP>
+__global__ void __launch_bounds__(ST_THREADS, 6) sweep_stream_group_kernel(const __grid_constant__ GroupArgs<StreamArgs, CAP> g)
+{
+    sweep_stream_body(g.a[blockIdx.z]);
+}
 
 // ---- pick: choose the event of every fired site, record it and claim its write set --------------
 struct PickArgs {
@@ -296,7 +310,7 @@ __device__ __forceinline__ void site_events_compact(const PickArgs &a, int s, in
     }
 }
 
-__global__ void __launch_bounds__(128) sweep_pick_kernel(const __grid_constant__ PickArgs a)
+__device__ __forceinline__ void sweep_pick_body(const PickArgs &a)
 {
     const unsigned int n = min(a.ss->n_fired, a.cap_fired);
     const int L = a.g.L;
@@ -363,12 +377,18 @@ __global__ void __launch_bounds__(128) sweep_pick_kernel(const __grid_constant__
         a.records[q] = rec;
     }
 }
+__global__ void __launch_bounds__(128) sweep_pick_kernel(const __grid_constant__ PickArgs a) { sweep_pick_body(a); }
+template <int CAP>
+__global__ void __launch_bounds__(128) sweep_pick_group_kernel(const __grid_constant__ GroupArgs<PickArgs, CAP> g)
+{
+    sweep_pick_body(g.a[blockIdx.z]);
+}
 
 // One warp per evaluated plane: fixed-order sum of the plane's tile partials.  plane_sum is
 // indexed by GLOBAL plane so that every slab count produces the same numbers.
-__global__ void sweep_plane_reduce_kernel(const double *blk_sum, const double *blk_max, int blks_per_plane,
-                                          int n_planes, int first_global, int own_lo, int own_hi,
-                                          double *plane_sum, double *max_out)
+__device__ __forceinline__ void sweep_plane_reduce_body(const double *blk_sum, const double *blk_max, int blks_per_plane,
+                                                        int n_planes, int first_global, int own_lo, int own_hi,
+                                                        double *plane_sum, double *max_out)
 {
     const int pl = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (pl >= n_planes) return;
@@ -386,10 +406,26 @@ __global__ void sweep_plane_reduce_kernel(const double *blk_sum, const double *b
         atomicMax((unsigned long long *)max_out, (unsigned long long)__double_as_longlong(m));   // m >= 0
     }
 }
+__global__ void sweep_plane_reduce_kernel(const double *blk_sum, const double *blk_max, int blks_per_plane,
+                                          int n_planes, int first_global, int own_lo, int own_hi,
+                                          double *plane_sum, double *max_out)
+{
+    sweep_plane_reduce_body(blk_sum, blk_max, blks_per_plane, n_planes, first_global, own_lo, own_hi, plane_sum, max_out);
+}
+
+// What differs between the lattices of a group in the small kernels (reset, plane reduce, finalize).
+struct CloseArgs {
+    SweepState *ss;
+    const double *blk_sum, *blk_max;
+    double *plane_sum;         // [n0] holds the running max
+    uint32_t *stamp;
+    unsigned int *refresh_queue, *dense_queue;
+    double events_per_sweep, p_max;
+};
 
 // Single CTA: total in fixed plane order, tau for the next sweep, time bookkeeping.
-__global__ void sweep_finalize_kernel(SweepState *ss, const double *plane_sum, int L, const double *max_in,
-                                      double events_per_sweep, double p_max)
+__device__ __forceinline__ void sweep_finalize_body(SweepState *ss, const double *plane_sum, int L, const double *max_in,
+                                                    double events_per_sweep, double p_max)
 {
     __shared__ double sm[40];
     const double total = block_sum(plane_sum, L, sm);
@@ -407,6 +443,40 @@ __global__ void sweep_finalize_kernel(SweepState *ss, const double *plane_sum, i
             ss->tau = tau;
         }
     }
+}
+__global__ void sweep_finalize_kernel(SweepState *ss, const double *plane_sum, int L, const double *max_in,
+                                      double events_per_sweep, double p_max)
+{
+    sweep_finalize_body(ss, plane_sum, L, max_in, events_per_sweep, p_max);
+}
+
+// Grouped small kernels.  reset: the stamp bitmap, the plane sums, the list counters and the refresh queue of
+// every lattice (what sweep_once clears with two memsets, sweep_reset_kernel and rates_refresh_list's memset), and
+// the dense rebuild's queue for the next sweep's rebuild (rates_rows_dense clears it before its launch);
+// grid (CTAs per lattice, lattices).
+template <int CAP>
+__global__ void __launch_bounds__(256) sweep_reset_group_kernel(const __grid_constant__ GroupArgs<CloseArgs, CAP> g, int stamp_words, int n0)
+{
+    const CloseArgs &a = g.a[blockIdx.y];
+    for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < stamp_words; q += gridDim.x * blockDim.x) a.stamp[q] = 0u;
+    if (blockIdx.x == 0) {
+        for (int q = threadIdx.x; q <= n0; q += blockDim.x) a.plane_sum[q] = 0.0;
+        if (threadIdx.x == 0) { a.ss->n_fired = 0; a.ss->n_dirty = 0; a.ss->n_dirty_emp = 0; *a.refresh_queue = 0u; *a.dense_queue = 0u; }
+    }
+}
+// grid (plane blocks, lattices); single-slab lattices: every evaluated plane is owned
+template <int CAP>
+__global__ void sweep_plane_reduce_group_kernel(const __grid_constant__ GroupArgs<CloseArgs, CAP> g, int blks_per_plane, int n_planes)
+{
+    const CloseArgs &a = g.a[blockIdx.y];
+    sweep_plane_reduce_body(a.blk_sum, a.blk_max, blks_per_plane, n_planes, 0, 0, n_planes, a.plane_sum, a.plane_sum + n_planes);
+}
+// one CTA per lattice
+template <int CAP>
+__global__ void sweep_finalize_group_kernel(const __grid_constant__ GroupArgs<CloseArgs, CAP> g, int L)
+{
+    const CloseArgs &a = g.a[blockIdx.x];
+    sweep_finalize_body(a.ss, a.plane_sum, L, a.plane_sum + L, a.events_per_sweep, a.p_max);
 }
 
 // ---- apply ---------------------------------------------------------------------------------------
@@ -500,7 +570,7 @@ __device__ __forceinline__ void site_changed(const ApplyArgs &a, int site, int, 
     }
 }
 
-__global__ void __launch_bounds__(128) sweep_apply_kernel(const __grid_constant__ ApplyArgs a)
+__device__ __forceinline__ void sweep_apply_body(const ApplyArgs &a)
 {
     const unsigned int n = min(a.ss->n_fired, a.cap_fired);
     const int LL = a.L * a.L;
@@ -584,6 +654,12 @@ __global__ void __launch_bounds__(128) sweep_apply_kernel(const __grid_constant_
         if (cta_cnt[1]) atomicAdd(&a.ss->n_applied, (unsigned long long)cta_cnt[1]);
         if (cta_cnt[2]) atomicAdd(&a.ss->n_nuc, (unsigned long long)cta_cnt[2]);
     }
+}
+__global__ void __launch_bounds__(128) sweep_apply_kernel(const __grid_constant__ ApplyArgs a) { sweep_apply_body(a); }
+template <int CAP>
+__global__ void __launch_bounds__(128) sweep_apply_group_kernel(const __grid_constant__ GroupArgs<ApplyArgs, CAP> g)
+{
+    sweep_apply_body(g.a[blockIdx.z]);
 }
 
 // Receiver side of the delta exchange: the neighbour's changed sites are written into the ghost planes
@@ -726,15 +802,9 @@ static int refresh_tiled(cet_ctx *c, const SlabRanges &R)
 // way, so both variants run the same trajectory bit for bit.
 // count == false is the priming pass of a fresh clock: tau is still 0, nothing can fire, and the pass
 // only measures the totals that give the first real sweep its interval.
-static int sweep_once(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_params *tp, const SlabRanges &R, bool tiled,
-                      bool count)
+// The start of a sweep: the thermal step when one is due, and the dense rebuild when the resident rates are stale.
+static int sweep_prepare(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_params *tp, const SlabRanges &R, bool tiled)
 {
-    const int n_eval = R.eval_hi - R.eval_lo;
-    const int i_off = (int)(c->i_begin - c->halo);
-    const int top_plane = (int)(c->n0 - 1 - i_off);
-    const int tpp = (int)((c->plane + ST_TILE - 1) / ST_TILE);
-    double *max_slot = c->plane_sum + c->n0;      // plane_sum[n0] holds the running max
-    ProfScope step_scope(c, PROF_STEP);
     if (sp->thermal_every > 0 && c->sweep_index % sp->thermal_every == 0 && c->last_thermal_index != c->sweep_index) {
         if (int rc = thermal_cet_step(c, tp, &c->sweep->terminated)) return rc;      // clears sweep_rates_valid
         if (c->world > 1) if (int rc = comm_halo_exchange(c, 4)) return rc;
@@ -758,18 +828,67 @@ static int sweep_once(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_
         }
         c->sweep_rates_valid = true;
     }
+    return 0;
+}
+
+// Kernel arguments of one sweep of context c.
+static StreamArgs stream_args(const cet_ctx *c, const cet_sweep_params *sp, const SlabRanges &R)
+{
+    const int i_off = (int)(c->i_begin - c->halo);
+    const int top_plane = (int)(c->n0 - 1 - i_off);
+    StreamArgs a;
+    a.site_rate = c->site_rate; a.dep_rate = c->dep_rate; a.ss = c->sweep;
+    a.fired = c->fired; a.cap_fired = (unsigned int)c->cap_fired;
+    a.blk_sum = c->blk_sum; a.blk_max = c->blk_max;
+    a.p_lo = R.eval_lo;
+    a.top_plane = (top_plane >= R.eval_lo && top_plane < R.eval_hi) ? top_plane : -1;
+    a.plane_sites = (int)c->plane; a.tiles_per_plane = (int)((c->plane + ST_TILE - 1) / ST_TILE); a.i_off = i_off;
+    a.seed = sp->seed; a.sweep = (uint32_t)c->sweep_index;
+    return a;
+}
+static PickArgs pick_args(const cet_ctx *c, const cet_sweep_params *sp, bool tiled)
+{
+    PickArgs a;
+    a.g = c->lat(); a.theta = c->theta; a.phi = c->phi; a.site_rate = c->site_rate; a.dep_rate = c->dep_rate;
+    a.P = c->rp; a.ss = c->sweep; a.fired = c->fired; a.cap_fired = (unsigned int)c->cap_fired;
+    a.records = (Record *)c->records; a.claim = c->claim;
+    a.seed = sp->seed; a.sweep = (uint32_t)c->sweep_index;
+    a.cvox = tiled ? c->cvox : nullptr; a.pairop = c->pairop; a.tab = c->rate_tab;
+    return a;
+}
+static ApplyArgs apply_args_of(const cet_ctx *c, const cet_sweep_params *sp, const SlabRanges &R, bool tiled, bool count)
+{
+    ApplyArgs b;
+    b.vox = c->vox; b.theta = c->theta; b.phi = c->phi; b.v = c->v;
+    b.ss = c->sweep; b.records = (const Record *)c->records; b.cap_fired = (unsigned int)c->cap_fired;
+    b.claim = c->claim; b.stamp = c->stamp; b.nst = (unsigned long long *)c->nst;
+    b.P = c->rp; b.L = (int)c->n1; b.n0 = (int)c->n0; b.i_off = (int)(c->i_begin - c->halo); b.np = (int)c->np;
+    b.c_lo = R.claim_lo; b.c_hi = R.claim_hi; b.own_lo = R.own_lo; b.own_hi = R.own_hi;
+    b.seed = sp->seed; b.sweep = (uint32_t)c->sweep_index;
+    b.defect_fraction = sp->defect_fraction;
+    b.cvox = tiled ? c->cvox : nullptr; b.pairop = c->pairop; b.T = c->T; b.tlut = tile_code_lut(c->rp);
+    const bool deltas = tiled && c->world > 1 && count;
+    b.delta_lo = (deltas && c->rank > 0) ? (unsigned char *)c->delta_send[0] : nullptr;
+    b.delta_hi = (deltas && c->rank < c->world - 1) ? (unsigned char *)c->delta_send[1] : nullptr;
+    b.delta_cap = (unsigned int)c->delta_cap;
+    b.probe = (c->debug_flags >> 6) & 3;
+    return b;
+}
+
+static int sweep_once(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_params *tp, const SlabRanges &R, bool tiled,
+                      bool count)
+{
+    const int n_eval = R.eval_hi - R.eval_lo;
+    const int i_off = (int)(c->i_begin - c->halo);
+    const int tpp = (int)((c->plane + ST_TILE - 1) / ST_TILE);
+    double *max_slot = c->plane_sum + c->n0;      // plane_sum[n0] holds the running max
+    ProfScope step_scope(c, PROF_STEP);
+    if (int rc = sweep_prepare(c, sp, tp, R, tiled)) return rc;
     CET_CUDA(cudaMemsetAsync(c->stamp, 0, (size_t)c->nloc / 8 + 8, c->stream));      // stamp bitmap of this sweep
     sweep_reset_kernel<<<1, 1, 0, c->stream>>>(c->sweep, max_slot);
     CET_CUDA(cudaMemsetAsync(c->plane_sum, 0, (size_t)c->n0 * sizeof(double), c->stream));
     {
-        StreamArgs a;
-        a.site_rate = c->site_rate; a.dep_rate = c->dep_rate; a.ss = c->sweep;
-        a.fired = c->fired; a.cap_fired = (unsigned int)c->cap_fired;
-        a.blk_sum = c->blk_sum; a.blk_max = c->blk_max;
-        a.p_lo = R.eval_lo;
-        a.top_plane = (top_plane >= R.eval_lo && top_plane < R.eval_hi) ? top_plane : -1;
-        a.plane_sites = (int)c->plane; a.tiles_per_plane = tpp; a.i_off = i_off;
-        a.seed = sp->seed; a.sweep = (uint32_t)c->sweep_index;
+        const StreamArgs a = stream_args(c, sp, R);
         ProfScope ps(c, PROF_DECIDE);
         sweep_stream_kernel<<<dim3((unsigned)tpp, (unsigned)n_eval), ST_THREADS, 0, c->stream>>>(a);
     }
@@ -784,31 +903,13 @@ static int sweep_once(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_
     const int sparse_grid = sm_count(c) * 32;
     ApplyArgs apply_args;
     {
-        PickArgs a;
-        a.g = c->lat(); a.theta = c->theta; a.phi = c->phi; a.site_rate = c->site_rate; a.dep_rate = c->dep_rate;
-        a.P = c->rp; a.ss = c->sweep; a.fired = c->fired; a.cap_fired = (unsigned int)c->cap_fired;
-        a.records = (Record *)c->records; a.claim = c->claim;
-        a.seed = sp->seed; a.sweep = (uint32_t)c->sweep_index;
-        a.cvox = tiled ? c->cvox : nullptr; a.pairop = c->pairop; a.tab = c->rate_tab;
+        const PickArgs a = pick_args(c, sp, tiled);
         ProfScope ps(c, PROF_PICK);
         sweep_pick_kernel<<<sparse_grid, 128, 0, c->stream>>>(a);
     }
     CET_CUDA(cudaGetLastError());
     {
-        ApplyArgs b;
-        b.vox = c->vox; b.theta = c->theta; b.phi = c->phi; b.v = c->v;
-        b.ss = c->sweep; b.records = (const Record *)c->records; b.cap_fired = (unsigned int)c->cap_fired;
-        b.claim = c->claim; b.stamp = c->stamp; b.nst = (unsigned long long *)c->nst;
-        b.P = c->rp; b.L = (int)c->n1; b.n0 = (int)c->n0; b.i_off = i_off; b.np = (int)c->np;
-        b.c_lo = R.claim_lo; b.c_hi = R.claim_hi; b.own_lo = R.own_lo; b.own_hi = R.own_hi;
-        b.seed = sp->seed; b.sweep = (uint32_t)c->sweep_index;
-        b.defect_fraction = sp->defect_fraction;
-        b.cvox = tiled ? c->cvox : nullptr; b.pairop = c->pairop; b.T = c->T; b.tlut = tile_code_lut(c->rp);
-        const bool deltas = tiled && c->world > 1 && count;
-        b.delta_lo = (deltas && c->rank > 0) ? (unsigned char *)c->delta_send[0] : nullptr;
-        b.delta_hi = (deltas && c->rank < c->world - 1) ? (unsigned char *)c->delta_send[1] : nullptr;
-        b.delta_cap = (unsigned int)c->delta_cap;
-        b.probe = (c->debug_flags >> 6) & 3;
+        const ApplyArgs b = apply_args_of(c, sp, R, tiled, count);
         if (b.delta_lo) CET_CUDA(cudaMemsetAsync(b.delta_lo, 0, DELTA_HEADER, c->stream));
         if (b.delta_hi) CET_CUDA(cudaMemsetAsync(b.delta_hi, 0, DELTA_HEADER, c->stream));
         apply_args = b;
@@ -880,6 +981,26 @@ static int sweep_once(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_
     return 0;
 }
 
+// The result block of a call from the sweep state before and after it.
+static int sweep_finish(cet_ctx *c, const SweepState &before, const SweepState &after, int64_t n_sweeps, cet_sweep_result *res)
+{
+    if (after.dirty_overflow) {      // refresh list overflowed: the resident rates are stale
+        c->sweep_rates_valid = false;
+        CET_CUDA(cudaMemsetAsync(&c->sweep->dirty_overflow, 0, sizeof(unsigned int), c->stream));
+    }
+    res->sweeps_done = n_sweeps;
+    res->events_fired = (int64_t)(after.n_fired_total - before.n_fired_total);
+    res->events_applied = (int64_t)(after.n_applied - before.n_applied);
+    res->nucleation_count = (int64_t)(after.n_nuc - before.n_nuc);
+    res->sweep_index = c->sweep_index;
+    res->time = after.time - before.time;
+    res->last_total_rate = after.sum_rate; res->last_max_rate = after.max_rate; res->last_tau = after.tau;
+    res->sites_refreshed = (int64_t)(after.n_refreshed_total - before.n_refreshed_total);
+    res->terminated = after.terminated;
+    res->overflow = (int32_t)(after.overflow | (after.dirty_overflow << 1));
+    return 0;
+}
+
 }  // namespace cet
 
 extern "C" int cet_sweep_run(cet_ctx *c, int64_t n_sweeps, const cet_sweep_params *sp,
@@ -931,19 +1052,216 @@ extern "C" int cet_sweep_run(cet_ctx *c, int64_t n_sweeps, const cet_sweep_param
     SweepState after;
     CET_CUDA(cudaMemcpyAsync(&after, c->sweep, sizeof(after), cudaMemcpyDeviceToHost, c->stream));
     CET_CUDA(cudaStreamSynchronize(c->stream));
-    if (after.dirty_overflow) {      // refresh list overflowed: the resident rates are stale
-        c->sweep_rates_valid = false;
-        CET_CUDA(cudaMemsetAsync(&c->sweep->dirty_overflow, 0, sizeof(unsigned int), c->stream));
+    return sweep_finish(c, before, after, n_sweeps, res);
+}
+
+// ---- grouped sweeps -------------------------------------------------------------------------------
+// A group of independent whole-lattice contexts of one L advances with one launch per kernel for all of them.
+// Per sweep: the thermal stencil and tile_pairop_T of the contexts whose step is due, the dense rebuild of the
+// contexts whose rates are stale, then reset, stream, plane reduce, pick, apply, dirty scan, refresh and finalize,
+// each one grouped launch whose CTAs find their lattice's arguments in the launch's table (the stencil: one launch
+// per variant in use, with and without the nan_to_num pass).  On L that a tensor map cannot describe (tile_tma_ok)
+// the dense rebuild is the compact gather kernel, issued per context.  Every lattice runs the solo kernel bodies
+// on its own data, so it ends bit for bit where cet_sweep_run would leave it.
+namespace cet {
+
+struct GroupMember {
+    cet_ctx *c;
+    const cet_sweep_params *sp;
+    const cet_thermal_params *tp;
+};
+
+template <int CAP>
+struct GroupTables {
+    GroupArgs<CloseArgs, CAP> close;
+    GroupArgs<StreamArgs, CAP> stream;
+    GroupArgs<PickArgs, CAP> pick;
+    GroupArgs<ApplyArgs, CAP> apply;
+};
+static_assert(group_fits<StreamArgs>() && group_fits<PickArgs>() && group_fits<ApplyArgs>() && group_fits<CloseArgs>(),
+              "a table of GROUP_MAX entries must fit the kernel parameter space");
+
+// occupancy of the persistent grouped kernels, queried on their first launch in a call
+struct GroupBlocks {
+    int refresh = 0, dense = 0;
+};
+
+// sweep_prepare for a group: the due thermal steps, then the rebuild of every context whose rates are stale
+static int sweep_group_prepare(const std::vector<GroupMember> &m, const SlabRanges &R, GroupBlocks &blocks)
+{
+    std::vector<cet_ctx *> due, stale;
+    std::vector<const cet_thermal_params *> due_tp;
+    for (const GroupMember &g : m) {
+        cet_ctx *c = g.c;
+        if (g.sp->thermal_every > 0 && c->sweep_index % g.sp->thermal_every == 0 && c->last_thermal_index != c->sweep_index) {
+            due.push_back(c);
+            due_tp.push_back(g.tp);
+        }
     }
-    res->sweeps_done = n_sweeps;
-    res->events_fired = (int64_t)(after.n_fired_total - before.n_fired_total);
-    res->events_applied = (int64_t)(after.n_applied - before.n_applied);
-    res->nucleation_count = (int64_t)(after.n_nuc - before.n_nuc);
-    res->sweep_index = c->sweep_index;
-    res->time = after.time - before.time;
-    res->last_total_rate = after.sum_rate; res->last_max_rate = after.max_rate; res->last_tau = after.tau;
-    res->sites_refreshed = (int64_t)(after.n_refreshed_total - before.n_refreshed_total);
-    res->terminated = after.terminated;
-    res->overflow = (int32_t)(after.overflow | (after.dirty_overflow << 1));
+    if (!due.empty()) {
+        if (int rc = thermal_cet_step_group(due.data(), due_tp.data(), (int)due.size())) return rc;   // clears sweep_rates_valid
+        if (int rc = tile_pairop_T_update_group(due.data(), (int)due.size())) return rc;
+        for (cet_ctx *c : due) c->last_thermal_index = c->sweep_index;
+    }
+    for (const GroupMember &g : m)
+        if (!g.c->sweep_rates_valid) stale.push_back(g.c);
+    if (stale.empty()) return 0;
+    {
+        ProfScope ps(m[0].c, PROF_RATES);
+        if (tile_tma_ok(m[0].c)) {
+            if (int rc = rates_rows_dense_group(stale.data(), (int)stale.size(), &blocks.dense)) return rc;
+        } else {
+            for (cet_ctx *c : stale)
+                if (int rc = rates_rows_compact(c, R.eval_lo, R.eval_hi)) return rc;
+        }
+    }
+    for (cet_ctx *c : stale) c->sweep_rates_valid = true;
+    return 0;
+}
+
+template <int CAP>
+static int sweep_group_once(const std::vector<GroupMember> &m, GroupTables<CAP> &t, GroupBlocks &blocks, bool count)
+{
+    const int n = (int)m.size();
+    cet_ctx *c0 = m[0].c;
+    cudaStream_t st = c0->stream;
+    const SlabRanges R = slab_ranges(c0);             // single-slab contexts of one L: the same for all
+    const int n_eval = R.eval_hi - R.eval_lo;
+    const int tpp = (int)((c0->plane + ST_TILE - 1) / ST_TILE);
+    ProfScope step_scope(c0, PROF_STEP);
+    if (int rc = sweep_group_prepare(m, R, blocks)) return rc;
+    for (int q = 0; q < n; ++q) {
+        cet_ctx *c = m[q].c;
+        CloseArgs &a = t.close.a[q];
+        a.ss = c->sweep; a.blk_sum = c->blk_sum; a.blk_max = c->blk_max; a.plane_sum = c->plane_sum; a.stamp = c->stamp;
+        a.refresh_queue = (unsigned int *)(c->rate_tab + RT_TABLE_DOUBLES) + 3;
+        a.dense_queue = dense_queue(c);
+        a.events_per_sweep = m[q].sp->events_per_sweep; a.p_max = m[q].sp->p_max;
+        t.stream.a[q] = stream_args(c, m[q].sp, R);
+        t.pick.a[q] = pick_args(c, m[q].sp, true);
+        t.apply.a[q] = apply_args_of(c, m[q].sp, R, true, count);
+    }
+    const int stamp_words = (int)(((size_t)c0->nloc / 8 + 8 + 3) / 4);
+    sweep_reset_group_kernel<CAP><<<dim3((unsigned)std::min((stamp_words + 255) / 256, 64), (unsigned)n), 256, 0, st>>>(
+        t.close, stamp_words, (int)c0->n0);
+    CET_CUDA(cudaGetLastError());
+    {
+        ProfScope ps(c0, PROF_DECIDE);
+        sweep_stream_group_kernel<CAP><<<dim3((unsigned)tpp, (unsigned)n_eval, (unsigned)n), ST_THREADS, 0, st>>>(t.stream);
+    }
+    CET_CUDA(cudaGetLastError());
+    sweep_plane_reduce_group_kernel<CAP><<<dim3((unsigned)((n_eval + 3) / 4), (unsigned)n), 128, 0, st>>>(t.close, tpp, n_eval);
+    CET_CUDA(cudaGetLastError());
+    // pick / apply stride over each lattice's fired list; the split of a list over CTAs does not change the outcome
+    // (claims are resolved by atomicMax of fixed keys, counters by integer atomics)
+    const unsigned sparse_x = (unsigned)std::max(1, (sm_count(c0) * 32 + n - 1) / n);
+    {
+        ProfScope ps(c0, PROF_PICK);
+        sweep_pick_group_kernel<CAP><<<dim3(sparse_x, 1, (unsigned)n), 128, 0, st>>>(t.pick);
+    }
+    CET_CUDA(cudaGetLastError());
+    {
+        ProfScope ps(c0, PROF_APPLY);
+        sweep_apply_group_kernel<CAP><<<dim3(sparse_x, 1, (unsigned)n), 128, 0, st>>>(t.apply);
+    }
+    CET_CUDA(cudaGetLastError());
+    {
+        ProfScope ps(c0, PROF_REFRESH);
+        std::vector<cet_ctx *> cs(n);
+        for (int q = 0; q < n; ++q) cs[q] = m[q].c;
+        if (int rc = rates_rows_dirty_compact_group(cs.data(), n, R.eval_lo, R.eval_hi, &blocks.refresh)) return rc;
+    }
+    sweep_finalize_group_kernel<CAP><<<n, 256, 0, st>>>(t.close, (int)c0->n0);
+    CET_CUDA(cudaGetLastError());
+    if (count)
+        for (const GroupMember &g : m) g.c->sweep_index++;
+    return 0;
+}
+
+template <int CAP>
+static int sweep_group_run(const std::vector<GroupMember> &all, const std::vector<GroupMember> &priming, int64_t n_sweeps)
+{
+    std::unique_ptr<GroupTables<CAP>> t(new GroupTables<CAP>());
+    GroupBlocks blocks;
+    if (!priming.empty())
+        if (int rc = sweep_group_once<CAP>(priming, *t, blocks, false)) return rc;
+    for (int64_t s = 0; s < n_sweeps; ++s)
+        if (int rc = sweep_group_once<CAP>(all, *t, blocks, true)) return rc;
+    return 0;
+}
+
+// The group's work runs on the first context's stream: every context's stream is pointed at it for the call
+// (so that the per-context compact rebuild of non-TMA L launches there too) and restored after it.  The call synchronises every context before and after, so no events are needed to order the work.
+struct StreamSwap {
+    std::vector<cet_ctx *> cs;
+    std::vector<cudaStream_t> own;
+    StreamSwap(cet_ctx *const *ctxs, int n) : cs(ctxs, ctxs + n)
+    {
+        for (cet_ctx *c : cs) { own.push_back(c->stream); c->stream = cs[0]->stream; }
+    }
+    ~StreamSwap() { for (size_t q = 0; q < cs.size(); ++q) cs[q]->stream = own[q]; }
+};
+
+}  // namespace cet
+
+extern "C" int cet_sweep_run_group(cet_ctx *const *ctxs, int32_t n_ctx, int64_t n_sweeps, const cet_sweep_params *sp,
+                                   const cet_thermal_params *tp, cet_sweep_result *res)
+{
+    CET_REQUIRE(ctxs && sp && res, "cet_sweep_run_group: NULL argument");
+    CET_REQUIRE(n_ctx >= 1 && n_ctx <= GROUP_MAX, "cet_sweep_run_group: need 1 <= n_ctx <= %d, got %d", GROUP_MAX, (int)n_ctx);
+    CET_REQUIRE(n_sweeps >= 0, "cet_sweep_run_group: n_sweeps < 0");
+    for (int q = 0; q < n_ctx; ++q) {
+        const cet_ctx *c = ctxs[q];
+        CET_REQUIRE(c, "cet_sweep_run_group: context %d is NULL", q);
+        for (int r = 0; r < q; ++r) CET_REQUIRE(ctxs[r] != c, "cet_sweep_run_group: context %d repeats context %d", q, r);
+        CET_REQUIRE(c->device == ctxs[0]->device, "cet_sweep_run_group: context %d is on another device", q);
+        CET_REQUIRE(c->world == 1 && c->halo == 0 && c->i_begin == 0 && c->i_end == c->n0,
+                    "cet_sweep_run_group: context %d is a slab; groups take whole-lattice contexts", q);
+        CET_REQUIRE(c->cubic && c->have_rp, "cet_sweep_run_group: context %d needs a cubic lattice with rate params", q);
+        CET_REQUIRE(c->n1 == ctxs[0]->n1, "cet_sweep_run_group: context %d has L = %lld, context 0 L = %lld", q,
+                    (long long)c->n1, (long long)ctxs[0]->n1);
+        CET_REQUIRE(c->debug_flags == 0, "cet_sweep_run_group: context %d has debug flags set", q);
+        CET_REQUIRE(c->nloc < (1ll << 31), "cet_sweep_run_group: the lattice must have fewer than 2^31 sites");
+        CET_REQUIRE(sp[q].p_max > 0.0 && sp[q].p_max < 1.0 && sp[q].events_per_sweep > 0.0,
+                    "cet_sweep_run_group: context %d: need 0 < p_max < 1 and events_per_sweep > 0", q);
+        CET_REQUIRE(sp[q].thermal_every <= 0 || tp != nullptr, "cet_sweep_run_group: context %d: thermal_every needs thermal params", q);
+    }
+    cet::DeviceGuard dg(ctxs[0]->device);
+    // the tile path's state and its condition (no empty site carries an orientation), checked on every context
+    // before anything else is allocated or launched: a lattice that fails it needs the gather kernels, which are not
+    // grouped.  The check derives the compact tile state (cvox / pairop) of the contexts it examines; nothing a
+    // caller can read changes.
+    for (int q = 0; q < n_ctx; ++q) {
+        cet_ctx *c = ctxs[q];
+        if (int rc = tile_state_ensure(c)) return rc;
+        CET_REQUIRE(c->emp_canonical, "cet_sweep_run_group: context %d has empty sites with an orientation (gather path)", q);
+    }
+    for (int q = 0; q < n_ctx; ++q)
+        if (int rc = sweep_alloc(ctxs[q])) return rc;
+    std::vector<SweepState> before(n_ctx), after(n_ctx);
+    std::vector<GroupMember> all, priming;
+    for (int q = 0; q < n_ctx; ++q) {
+        cet_ctx *c = ctxs[q];
+        if (int rc = rate_tables_ensure(c)) return rc;
+        c->nst_valid = false;
+        CET_CUDA(cudaMemsetAsync(dense_queue(c), 0, sizeof(unsigned int), c->stream));    // the grouped rebuild's queue
+        CET_CUDA(cudaMemcpyAsync(&before[q], c->sweep, sizeof(SweepState), cudaMemcpyDeviceToHost, c->stream));
+        CET_CUDA(cudaStreamSynchronize(c->stream));
+        const GroupMember g{c, &sp[q], tp ? &tp[q] : nullptr};
+        all.push_back(g);
+        if (n_sweeps > 0 && before[q].tau == 0.0 && !before[q].terminated) priming.push_back(g);
+    }
+    {
+        StreamSwap swap(ctxs, n_ctx);
+        const int rc = n_ctx <= 16 ? sweep_group_run<16>(all, priming, n_sweeps) : sweep_group_run<GROUP_MAX>(all, priming, n_sweeps);
+        if (rc) return rc;
+        for (int q = 0; q < n_ctx; ++q) {
+            ctxs[q]->rates_valid = false;
+            CET_CUDA(cudaMemcpyAsync(&after[q], ctxs[q]->sweep, sizeof(SweepState), cudaMemcpyDeviceToHost, ctxs[q]->stream));
+        }
+        CET_CUDA(cudaStreamSynchronize(ctxs[0]->stream));
+    }
+    for (int q = 0; q < n_ctx; ++q)
+        if (int rc = sweep_finish(ctxs[q], before[q], after[q], n_sweeps, &res[q])) return rc;
     return 0;
 }

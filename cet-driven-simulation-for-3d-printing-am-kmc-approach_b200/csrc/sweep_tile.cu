@@ -398,11 +398,28 @@ __global__ void tile_state_build_kernel(const uint8_t *__restrict__ vox, const V
     }
 }
 // after a thermal step: the temperature half of pairop
-__global__ void tile_pairop_T_kernel(const uint8_t *__restrict__ cvox, const double *__restrict__ T, double *pairop, int64_t s_lo,
-                                     int64_t s_hi)
+__device__ __forceinline__ void tile_pairop_T_body(const uint8_t *__restrict__ cvox, const double *__restrict__ T, double *pairop,
+                                                   int64_t s_lo, int64_t s_hi)
 {
     for (int64_t s = s_lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < s_hi; s += (int64_t)gridDim.x * blockDim.x)
         if ((cvox[s] & 15u) == TC_EMPTY) pairop[s] = T[s];
+}
+__global__ void tile_pairop_T_kernel(const uint8_t *__restrict__ cvox, const double *__restrict__ T, double *pairop, int64_t s_lo,
+                                     int64_t s_hi)
+{
+    tile_pairop_T_body(cvox, T, pairop, s_lo, s_hi);
+}
+// grouped sweeps: grid (CTAs per lattice, lattices), whole-lattice contexts of one size
+struct PairopTArgs {
+    const uint8_t *cvox;
+    const double *T;
+    double *pairop;
+};
+template <int CAP>
+__global__ void tile_pairop_T_group_kernel(const __grid_constant__ GroupArgs<PairopTArgs, CAP> g, int64_t n_sites)
+{
+    const PairopTArgs &a = g.a[blockIdx.y];
+    tile_pairop_T_body(a.cvox, a.T, a.pairop, 0, n_sites);
 }
 // set the stamp bits of local sites [s_lo, s_hi)
 __global__ void stamp_fill_kernel(uint32_t *stamp, int64_t s_lo, int64_t s_hi)
@@ -490,6 +507,24 @@ int tile_pairop_T_update(cet_ctx *c)
     tile_pairop_T_kernel<<<grid, 256, 0, c->stream>>>(c->cvox, c->T, c->pairop, s_lo, s_hi);
     CET_CUDA(cudaGetLastError());
     return 0;
+}
+
+template <int CAP>
+static int tile_pairop_T_group_launch(cet_ctx *const *cs, int n)
+{
+    GroupArgs<PairopTArgs, CAP> g;
+    for (int q = 0; q < n; ++q) g.a[q] = PairopTArgs{cs[q]->cvox, cs[q]->T, cs[q]->pairop};
+    const int64_t n_sites = cs[0]->nloc;
+    const int per = (int)std::max<int64_t>(1, std::min<int64_t>((n_sites + 255) / 256, ((int64_t)sm_count(cs[0]) * 16 + n - 1) / n));
+    tile_pairop_T_group_kernel<CAP><<<dim3((unsigned)per, (unsigned)n), 256, 0, cs[0]->stream>>>(g, n_sites);
+    CET_CUDA(cudaGetLastError());
+    return 0;
+}
+// tile_pairop_T_update for a group of whole-lattice contexts of one L (cet_sweep_run_group), on the stream of cs[0]
+int tile_pairop_T_update_group(cet_ctx *const *cs, int n)
+{
+    if (n <= 0) return 0;
+    return n <= 16 ? tile_pairop_T_group_launch<16>(cs, n) : tile_pairop_T_group_launch<GROUP_MAX>(cs, n);
 }
 
 int stamp_fill(cet_ctx *c, int p_lo, int p_hi)

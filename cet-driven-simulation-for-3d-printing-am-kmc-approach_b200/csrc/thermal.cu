@@ -49,12 +49,14 @@ constexpr int TH_TK = 128;   // threads along k
 constexpr int TH_TJ = 4;     // rows per CTA
 constexpr int TH_PLANES = 8; // planes marched per CTA
 
+// The kernel bodies take their arguments by reference and the plane block `zb` (blockIdx.z of a solo launch): the
+// grouped launches of cet_sweep_run_group run them for the table entry of their lattice.
 template <bool FULL>
-__global__ void __launch_bounds__(TH_TK *TH_TJ) thermal_kernel(ThermalArgs a)
+__device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb)
 {
     const int k = blockIdx.x * TH_TK + threadIdx.x;
     const int j = blockIdx.y * TH_TJ + threadIdx.y;
-    const int p0 = a.p_lo + blockIdx.z * TH_PLANES;
+    const int p0 = a.p_lo + zb * TH_PLANES;
     if (k >= a.n2 || j >= a.n1) return;
     const int64_t plane = (int64_t)a.n1 * a.n2;
     const int jm = j > 0 ? j - 1 : 0, jp = j < a.n1 - 1 ? j + 1 : a.n1 - 1;
@@ -104,6 +106,8 @@ __global__ void __launch_bounds__(TH_TK *TH_TJ) thermal_kernel(ThermalArgs a)
         centre = above;
     }
 }
+template <bool FULL>
+__global__ void __launch_bounds__(TH_TK *TH_TJ) thermal_kernel(ThermalArgs a) { thermal_body<FULL>(a, blockIdx.z); }
 
 // Fast path (n2 a multiple of V = 2 or 4): V consecutive k per thread with 16-byte loads/stores,
 // the k-neighbours exchanged by warp shuffles, the i-neighbours kept in a register queue while
@@ -131,12 +135,12 @@ struct RowVec {
 };
 
 template <bool FULL, bool NANFIX, int V>
-__global__ void __launch_bounds__(32 * TH2_TJ) thermal_kernel_v2(const ThermalArgs a)
+__device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb)
 {
     const int lane = threadIdx.x;
     const int k0 = (blockIdx.x * 32 + lane) * V;
     const int j = blockIdx.y * TH2_TJ + threadIdx.y;
-    const int p0 = a.p_lo + blockIdx.z * TH2_PLANES;
+    const int p0 = a.p_lo + zb * TH2_PLANES;
     if (j >= a.n1) return;                                   // whole warp (threadIdx.y is per warp)
     const bool in = k0 < a.n2;                               // n2 % V == 0: the whole vector is inside
     const int64_t plane = (int64_t)a.n1 * a.n2;
@@ -210,6 +214,18 @@ __global__ void __launch_bounds__(32 * TH2_TJ) thermal_kernel_v2(const ThermalAr
         pc += plane; pm += plane; pp += plane; po += plane;
     }
 }
+template <bool FULL, bool NANFIX, int V>
+__global__ void __launch_bounds__(32 * TH2_TJ) thermal_kernel_v2(const ThermalArgs a) { thermal_v2_body<FULL, NANFIX, V>(a, blockIdx.z); }
+
+// Grouped update_temperature_cet (cet_sweep_run_group): blockIdx.z = lattice * nzb + plane block.  V = 0: the
+// scalar kernel (odd n2).
+template <bool NANFIX, int V, int CAP>
+__global__ void __launch_bounds__(V ? 32 * TH2_TJ : TH_TK * TH_TJ) thermal_group_kernel(const __grid_constant__ GroupArgs<ThermalArgs, CAP> g, int nzb)
+{
+    const ThermalArgs &a = g.a[blockIdx.z / nzb];
+    if constexpr (V == 0) thermal_body<false>(a, blockIdx.z % nzb);
+    else thermal_v2_body<false, NANFIX, V>(a, blockIdx.z % nzb);
+}
 
 __global__ void fill_gradient_kernel(double *T, int64_t plane, int np, int i_off, int n0, double t0, double g)
 {
@@ -232,14 +248,27 @@ static void thermal_range(const cet_ctx *c, int *p_lo, int *p_hi)
     *p_lo = lo; *p_hi = hi;
 }
 
-template <bool FULL>
-static int launch_thermal(cet_ctx *c, ThermalArgs &a)
+static void thermal_geometry(const cet_ctx *c, ThermalArgs &a)
 {
     a.Tin = c->T; a.Tout = c->T2;
     a.n0 = (int)c->n0; a.n1 = (int)c->n1; a.n2 = (int)c->n2;
     a.i_off = (int)(c->i_begin - c->halo);
     a.np = (int)c->np;
     thermal_range(c, &a.p_lo, &a.p_hi);
+}
+// the host side of a finished step: T2 becomes T, and what the new temperatures invalidate
+static void thermal_done(cet_ctx *c, const ThermalArgs &a, bool full)
+{
+    double *t = c->T; c->T = c->T2; c->T2 = t;
+    if (a.nan_to_num) c->T_finite = true;   // a pass skipped by the stop flag cannot be the first of a run
+    if (full) c->T_finite = false;          // the laser source term is caller data
+    c->rates_valid = false; c->sweep_rates_valid = false;
+}
+
+template <bool FULL>
+static int launch_thermal(cet_ctx *c, ThermalArgs &a)
+{
+    thermal_geometry(c, a);
     if (a.p_hi <= a.p_lo) return 0;
     // np.nan_to_num is the identity on a finite field, and a finite field stays finite under the
     // clipped update: once a fixing pass has run (or the field is known finite) skip the checks.
@@ -273,22 +302,89 @@ static int launch_thermal(cet_ctx *c, ThermalArgs &a)
     if (a.p_hi < c->np)
         CET_CUDA(cudaMemcpyAsync(c->T2 + (int64_t)a.p_hi * plane, c->T + (int64_t)a.p_hi * plane,
                                  (size_t)(c->np - a.p_hi) * plane * 8, cudaMemcpyDeviceToDevice, c->stream));
-    double *t = c->T; c->T = c->T2; c->T2 = t;
-    if (a.nan_to_num) c->T_finite = true;   // a pass skipped by the stop flag cannot be the first of a run
-    if (FULL) c->T_finite = false;          // the laser source term is caller data
-    c->rates_valid = false; c->sweep_rates_valid = false;
+    thermal_done(c, a, FULL);
     return 0;
 }
 
-// Used by the KMC drivers (kmc_exact.cu, sweep.cu): one update_temperature_cet on the ctx stream.
-int thermal_cet_step(cet_ctx *c, const cet_thermal_params *p, const int32_t *stop_flag)
+static ThermalArgs cet_step_args(const cet_thermal_params *p, const int32_t *stop_flag)
 {
     ThermalArgs a;
     memset(&a, 0, sizeof(a));
     a.dt_alpha = p->dt_alpha; a.inv_dx2 = p->inv_dx2; a.lo = p->lo; a.hi = p->hi;
     a.nan_value = p->nan_value; a.nan_to_num = p->nan_to_num;
     a.stop = stop_flag;
+    return a;
+}
+
+// Used by the KMC drivers (kmc_exact.cu, sweep.cu): one update_temperature_cet on the ctx stream.
+int thermal_cet_step(cet_ctx *c, const cet_thermal_params *p, const int32_t *stop_flag)
+{
+    ThermalArgs a = cet_step_args(p, stop_flag);
     return launch_thermal<false>(c, a);
+}
+
+template <bool NANFIX, int V, int CAP>
+static int thermal_group_launch(cet_ctx *const *cs, const ThermalArgs *args, int n)
+{
+    GroupArgs<ThermalArgs, CAP> g;
+    for (int q = 0; q < n; ++q) g.a[q] = args[q];
+    const cet_ctx *c = cs[0];
+    const int planes = args[0].p_hi - args[0].p_lo;
+    dim3 block, grid;
+    int nzb;
+    if (V) {
+        nzb = (planes + TH2_PLANES - 1) / TH2_PLANES;
+        block = dim3(32, TH2_TJ);
+        grid = dim3((unsigned)((c->n2 / V + 31) / 32), (unsigned)((c->n1 + TH2_TJ - 1) / TH2_TJ), (unsigned)(nzb * n));
+    } else {
+        nzb = (planes + TH_PLANES - 1) / TH_PLANES;
+        block = dim3(TH_TK, TH_TJ);
+        grid = dim3((unsigned)((c->n2 + TH_TK - 1) / TH_TK), (unsigned)((c->n1 + TH_TJ - 1) / TH_TJ), (unsigned)(nzb * n));
+    }
+    thermal_group_kernel<NANFIX, V, CAP><<<grid, block, 0, c->stream>>>(g, nzb);
+    CET_CUDA(cudaGetLastError());
+    return 0;
+}
+template <bool NANFIX, int V>
+static int thermal_group_launch(cet_ctx *const *cs, const ThermalArgs *args, int n)
+{
+    return n <= 16 ? thermal_group_launch<NANFIX, V, 16>(cs, args, n) : thermal_group_launch<NANFIX, V, GROUP_MAX>(cs, args, n);
+}
+
+// thermal_cet_step for a group of whole-lattice contexts of one L (cet_sweep_run_group), on the stream of cs[0]: one
+// launch per kernel variant in use — the contexts whose T is not yet known to be finite take the nan_to_num pass.
+int thermal_cet_step_group(cet_ctx *const *cs, const cet_thermal_params *const *tps, int n)
+{
+    if (n <= 0) return 0;
+    ThermalArgs fix[GROUP_MAX], plain[GROUP_MAX];
+    cet_ctx *fix_c[GROUP_MAX], *plain_c[GROUP_MAX];
+    int n_fix = 0, n_plain = 0;
+    for (int q = 0; q < n; ++q) {
+        cet_ctx *c = cs[q];
+        ThermalArgs a = cet_step_args(tps[q], &c->sweep->terminated);
+        thermal_geometry(c, a);
+        CET_REQUIRE(a.p_lo == 0 && a.p_hi == (int)c->np, "thermal_cet_step_group: whole-lattice contexts only");
+        if (a.nan_to_num && !c->T_finite) { fix_c[n_fix] = c; fix[n_fix++] = a; }
+        else { plain_c[n_plain] = c; plain[n_plain++] = a; }
+    }
+    const int V = cs[0]->n2 % 4 == 0 ? 4 : cs[0]->n2 % 2 == 0 ? 2 : 0;
+    {
+        ProfScope ps(cs[0], PROF_THERMAL);
+        for (int f = 0; f < 2; ++f) {
+            cet_ctx *const *gc = f ? fix_c : plain_c;
+            const ThermalArgs *ga = f ? fix : plain;
+            const int m = f ? n_fix : n_plain;
+            if (m == 0) continue;
+            int rc;
+            if (V == 4) rc = f ? thermal_group_launch<true, 4>(gc, ga, m) : thermal_group_launch<false, 4>(gc, ga, m);
+            else if (V == 2) rc = f ? thermal_group_launch<true, 2>(gc, ga, m) : thermal_group_launch<false, 2>(gc, ga, m);
+            else rc = thermal_group_launch<false, 0>(gc, ga, m);      // the scalar kernel applies nan_to_num per value
+            if (rc) return rc;
+        }
+    }
+    for (int q = 0; q < n_fix; ++q) thermal_done(fix_c[q], fix[q], false);
+    for (int q = 0; q < n_plain; ++q) thermal_done(plain_c[q], plain[q], false);
+    return 0;
 }
 
 }  // namespace cet

@@ -168,6 +168,18 @@ int cet_kmc_run(cet_ctx *ctx, int64_t step0, int64_t n_steps, double defect_frac
  * rate, so that every counted sweep is a real one. */
 int cet_sweep_run(cet_ctx *ctx, int64_t n_sweeps, const cet_sweep_params *sp,
                   const cet_thermal_params *tp, cet_sweep_result *res);
+/* Advance n_ctx independent lattices by n_sweeps sweeps each, with one launch per kernel for the whole group.
+ * sp, tp, res are arrays of n_ctx (tp may be NULL when no sp[q].thermal_every > 0).  Every context ends exactly
+ * as cet_sweep_run(ctxs[q], n_sweeps, &sp[q], &tp[q], &res[q]) would leave it, bit for bit, whatever else is in
+ * the group and in whatever order.  The contexts must be distinct whole-lattice contexts (no slabs) of one L on
+ * one device, with rate params, no debug flags and no empty site carrying an orientation; 1 <= n_ctx <= 64.
+ * Everything is checked before any sweep buffer is allocated or any sweep runs (the check of the last condition
+ * derives each examined context's compact tile state, which no caller can read).  The work is ordered on the
+ * stream of ctxs[0]; the call returns when it is done.  The thermal step, tile_pairop_T and the dense rate rebuild
+ * are grouped too, except the rebuild on L that a tensor map cannot describe (L % 16 != 0 or L < 64), which runs
+ * per context.  When profiling is enabled on ctxs[0], the spans of the grouped kernels are recorded there. */
+int cet_sweep_run_group(cet_ctx *const *ctxs, int32_t n_ctx, int64_t n_sweeps, const cet_sweep_params *sp,
+                        const cet_thermal_params *tp, cet_sweep_result *res);
 int cet_sweep_reset(cet_ctx *ctx); /* zero the sweep counter, clock, tau and event counters */
 /* Checkpoint / resume of the sweep clock: running sweep counter (the Philox key of the next sweep),
  * the interval tau the next sweep will use, the accumulated time. */

@@ -2,7 +2,10 @@
 GPUs of one box, producing cet_map.csv and the tree the reference's plot_cet.py reads.
 
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29541 \
-        scripts/run_gr_sweep.py [--L 64] [--sweeps 400] [--out gr_sweep]
+        scripts/run_gr_sweep.py [--L 64] [--sweeps 400] [--out gr_sweep] [--batch 16]
+
+--batch k: the cases of a GPU advance in groups of up to k lattices (one kernel launch per group and kernel);
+the outputs are the same as without it.
 """
 import argparse
 import json
@@ -22,13 +25,14 @@ def main():
     ap.add_argument("--L", type=int, default=64)
     ap.add_argument("--sweeps", type=int, default=401)
     ap.add_argument("--out", default="gr_sweep")
+    ap.add_argument("--batch", type=int, default=None)
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     temps = [2600.0, 2800.0, 3000.0, 3200.0]                      # T_sub -> G = (T_MELT - T_sub) / (L dx)
     nu_deps = [1e12, 5e12, 2e13, 1e14]                            # NU_DEP -> R
     t0 = time.perf_counter()
     rows = campaign.run_gr_sweep(temps, nu_deps, L=args.L, n_sweeps=args.sweeps, n_seeds=20, defect_fraction=3e-3,
-                                 impurity_c=0.1, output_root=args.out, metrics_every=100)
+                                 impurity_c=0.1, output_root=args.out, metrics_every=100, batch=args.batch)
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -39,7 +43,7 @@ def main():
         merged = campaign.merge_cet_map(args.out)
         wall = time.perf_counter() - t0
         sites = len(temps) * len(nu_deps) * args.L ** 3 * args.sweeps
-        print(json.dumps({"cases": len(merged), "world": world, "L": args.L, "sweeps": args.sweeps, "wall_s": wall,
+        print(json.dumps({"cases": len(merged), "world": world, "L": args.L, "sweeps": args.sweeps, "batch": args.batch, "wall_s": wall,
                           "rank0_s": dt, "site_updates_per_s": sites / wall,
                           "classes": sorted(set(r["CET_Class"] for r in merged))}))
         for r in merged:

@@ -63,6 +63,19 @@ class SweepResult(C.Structure):                     # cet_sweep_result
                 ("terminated", C.c_int32), ("overflow", C.c_int32), ("sites_refreshed", C.c_int64)]
 
 
+class MetricsParams(C.Structure):                   # cet_metrics_params
+    _fields_ = [("theta_threshold", C.c_double), ("ar_threshold", C.c_double), ("pct_pos", C.c_int64 * 4),
+                ("refresh", C.c_int32), ("carbon_id", C.c_int32), ("epoch", C.c_uint32), ("pad_", C.c_int32),
+                ("seed", C.c_uint64), ("prob_base", C.c_double), ("e_mig", C.c_double), ("kT", C.c_double),
+                ("T_default", C.c_double)]
+
+
+class MetricsResult(C.Structure):                   # cet_metrics_result
+    _fields_ = [("counts", C.c_int64 * 16), ("n_carbon", C.c_int64), ("n_defects", C.c_int64),
+                ("n_grains", C.c_int64), ("size_sum", C.c_int64), ("n_equiaxed", C.c_int64),
+                ("pct_index", C.c_int64 * 4), ("ar_sum", C.c_double)]
+
+
 _lib = None
 _lock = threading.Lock()
 
@@ -115,6 +128,9 @@ SIGNATURES = {
     "cet_grains_stats": [_VP, _I64, _VP, _VP, _VP, _VP],
     "cet_grains_download_labels": [_VP, _VP],
     "cet_grains_download_planes": [_VP, _I64, _I64, _VP],
+    "cet_counts_group": [C.POINTER(_VP), _I32, C.POINTER(_I64)],
+    "cet_metrics_group": [C.POINTER(_VP), _I32, C.POINTER(MetricsParams), C.POINTER(_VP), C.POINTER(_I64),
+                          C.POINTER(MetricsResult)],
     "cet_debug_nst_mismatches": [_VP, C.POINTER(_I64)],
     "cet_debug_flags": [_VP, C.c_int],
     "cet_profile_enable": [_VP, C.c_int],
@@ -525,6 +541,57 @@ def sweep_run_group(ctxs, n_sweeps, sps, tps=None):
     res = (SweepResult * n)()
     check(lib().cet_sweep_run_group(handles, n, int(n_sweeps), sp_arr, tp_arr, res), "cet_sweep_run_group")
     return [{f: getattr(r, f) for f, _ in SweepResult._fields_ if f != "pad_"} for r in res]
+
+
+def _group_handles(fn, ctxs):
+    if any(not isinstance(c, Context) for c in ctxs):
+        raise TypeError(f"{fn}: ctxs must be Context objects")
+    return (C.c_void_p * len(ctxs))(*[c._h.value for c in ctxs])
+
+
+def counts_group(ctxs):
+    """Context.counts() of every context of `ctxs` (whole-lattice Contexts of one L on one device) with one launch
+    and one synchronisation: an (n, 16) int64 array."""
+    ctxs = list(ctxs)
+    handles = _group_handles("counts_group", ctxs)
+    out = np.zeros((len(ctxs), 16), np.int64)
+    check(lib().cet_counts_group(handles, len(ctxs), out.ctypes.data_as(C.POINTER(C.c_int64))), "cet_counts_group")
+    return out
+
+
+def metrics_group(ctxs, params, draws=None):
+    """The metrics cadence of a group of whole-lattice Contexts of one L on one device, each kernel one launch for
+    the group: per context the optional defect-mask refresh (params[q].refresh; draws[q] the NumPy stream's draws,
+    or None for the Philox stream), the state histogram, the grain labelling (Context.grains() reports it
+    afterwards) and the reductions of a metrics row.  params: one MetricsParams per context; draws: None or a list
+    with one entry per context.  Returns one dict per context with the fields of MetricsResult (counts and
+    pct_index as int64 arrays)."""
+    ctxs, params = list(ctxs), list(params)
+    n = len(ctxs)
+    if len(params) != n:
+        raise ValueError(f"metrics_group: {len(params)} params for {n} contexts")
+    if any(not isinstance(p, MetricsParams) for p in params):
+        raise TypeError("metrics_group: params must be MetricsParams")
+    if draws is not None:
+        draws = list(draws)
+        if len(draws) != n:
+            raise ValueError(f"metrics_group: {len(draws)} draw arrays for {n} contexts")
+        draws = [None if d is None else np.ascontiguousarray(d, dtype=np.float64) for d in draws]
+    handles = _group_handles("metrics_group", ctxs)
+    mp = (MetricsParams * n)(*params)
+    res = (MetricsResult * n)()
+    d_ptr = n_draws = None
+    if draws is not None:
+        d_ptr = (C.c_void_p * n)(*[None if d is None else d.ctypes.data for d in draws])
+        n_draws = (C.c_int64 * n)(*[0 if d is None else d.size for d in draws])
+    check(lib().cet_metrics_group(handles, n, mp, d_ptr, n_draws, res), "cet_metrics_group")
+    out = []
+    for r in res:
+        d = {f: getattr(r, f) for f, _ in MetricsResult._fields_}
+        d["counts"] = np.array(list(r.counts), np.int64)
+        d["pct_index"] = np.array(list(r.pct_index), np.int64)
+        out.append(d)
+    return out
 
 
 def comm_unique_id() -> bytes:

@@ -159,6 +159,36 @@ def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_
                             all_gather=all_gather)
 
 
+def _cadence_group(runs, last, every, philox_mask, seed):
+    """_cadence for every case of a group at once (cetkmc.metrics_group, one launch per kernel for the group): the
+    defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  With NumPy's
+    stream each case draws its mask from its own saved position (r["rng"]), in group order, as refresh_resident
+    draws it."""
+    ctxs = [r["ctx"] for r in runs]
+    refresh = last % every == 0
+    draws = None
+    if refresh and not philox_mask:
+        draws = []
+        for r, n_c in zip(runs, _lib.counts_group(ctxs)[:, _defects.CARBON_ID]):
+            np.random.set_state(r["rng"])
+            draws.append(np.random.random(int(n_c)) if n_c > 0 else np.zeros(0))      # defects.py:9,18
+            r["rng"] = np.random.get_state()
+    n_sites = int(np.prod(ctxs[0].owned_shape))
+    params = []
+    for _r in runs:
+        p = _lib.MetricsParams()
+        p.theta_threshold, p.ar_threshold = 0.5, constants.CET_AR_THRESHOLD
+        p.pct_pos[:] = _metrics.percentile_positions(n_sites)
+        p.refresh, p.carbon_id, p.epoch, p.seed = int(refresh), _defects.CARBON_ID, last // every, seed
+        p.prob_base, p.e_mig, p.kT, p.T_default = constants.DEFECT_PROB_BASE, _defects.E_MIGRATION, constants.K_T, constants.T_SUB
+        params.append(p)
+    for r, res in zip(runs, _lib.metrics_group(ctxs, params, draws)):
+        m = _metrics.metrics_from_summary(res, n_sites, voxel_size=constants.VOXEL_SIZE)
+        row, r["cet_detected"] = _ks._row_from_metrics(last, r["total_time"], r["nucleation_count"], r["cet_detected"],
+                                                       r["consts"], res["counts"], m, n_sites, verbose=False)
+        r["rows"].append(row)
+
+
 def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_seeds=5, impurity_c=0.0,
                        output_prefix="cet_sublattice", metrics_every=None, events_per_sweep=None, p_max=0.1,
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
@@ -339,7 +369,8 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
-    around its host draws).  A case that terminates stops at the row it stops at alone and leaves the group."""
+    around its host draws).  The metrics cadence of the group is one cetkmc.metrics_group call per row
+    (_cadence_group).  A case that terminates stops at the row it stops at alone and leaves the group."""
     if mask_stream not in ("numpy", "philox"):
         raise ValueError("mask_stream must be 'numpy' or 'philox'")
     seed = constants.RANDOM_SEED if seed is None else int(seed)
@@ -371,11 +402,7 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
                 r["total_time"] += res["time"]
                 r["nucleation_count"] += res["nucleation_count"]
                 r["terminated"] = bool(res["terminated"]) or res["sweeps_done"] == 0
-                np.random.set_state(r["rng"])
-                row, r["cet_detected"] = _cadence(r["ctx"], sweep - 1, every, philox_mask, seed, 1, r["total_time"],
-                                                  r["nucleation_count"], r["cet_detected"], r["consts"], verbose=False)
-                r["rng"] = np.random.get_state()
-                r["rows"].append(row)
+            _cadence_group(active, sweep - 1, every, philox_mask, seed)
             active = [r for r in active if not r["terminated"]]
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")

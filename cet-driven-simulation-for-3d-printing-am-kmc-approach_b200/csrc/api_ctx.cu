@@ -2,7 +2,7 @@
 // life cycle, and conversion between the reference's host layouts (int64 / float64 arrays,
 // lattice_init.py:23-32) and the packed HBM layout (1 byte per voxel + float64 fields).
 #include <stdarg.h>
-#include "ctx.cuh"
+#include "cadence.cuh"
 #include "rate_tile.cuh"
 
 namespace cet {
@@ -57,14 +57,7 @@ __global__ void unpack_kernel(const uint8_t *__restrict__ vox, int64_t *state, i
 
 __global__ void counts_kernel(const uint8_t *__restrict__ vox, int64_t n, unsigned long long *out)
 {
-    __shared__ unsigned int h[16];
-    if (threadIdx.x < 16) h[threadIdx.x] = 0;
-    __syncthreads();
-    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n;
-         q += (int64_t)gridDim.x * blockDim.x)
-        atomicAdd(&h[vox[q] & 0x0F], 1u);
-    __syncthreads();
-    if (threadIdx.x < 16 && h[threadIdx.x]) atomicAdd(&out[threadIdx.x], (unsigned long long)h[threadIdx.x]);
+    counts_body(vox, n, out);
 }
 
 __global__ void orient_kernel(const double *__restrict__ theta, const double *__restrict__ phi, Vec4 *v, int64_t n)
@@ -261,7 +254,7 @@ int cet_destroy(cet_ctx *c)
                     c->row_occ, c->row_emp, c->row_dep, c->row_depcnt, c->seg, c->total, c->q_top,
                     c->stage, c->kmc, c->d_py, c->d_np, c->d_sp, c->d_log, c->sweep, c->claim,
                     c->records, c->blk_sum, c->blk_max, c->plane_sum, c->stamp, c->dirty, c->fired,
-                    c->grain_label, c->grain_gid, c->rate_tab, c->cvox, c->pairop, c->tile_flag,
+                    c->grain_label, c->grain_gid, c->grain_st, c->group_tab, c->rate_tab, c->cvox, c->pairop, c->tile_flag,
                     c->delta_send[0], c->delta_send[1], c->delta_recv[0], c->delta_recv[1]};
     for (void *p : ptrs)
         if (p) cudaFree(p);
@@ -269,6 +262,7 @@ int cet_destroy(cet_ctx *c)
     for (auto e : c->prof_pool) cudaEventDestroy(e);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
+    if (c->ev_group) cudaEventDestroy(c->ev_group);
     if (c->ev_reduce_ready) cudaEventDestroy(c->ev_reduce_ready);
     if (c->ev_reduce_done) cudaEventDestroy(c->ev_reduce_done);
     if (c->stream2) cudaStreamDestroy(c->stream2);

@@ -171,6 +171,11 @@ struct cet_ctx {
     int *grain_label = nullptr, *grain_gid = nullptr;
     int64_t n_grains = 0;
     int grain_p_lo = 0, grain_p_hi = 0;   // local planes the last labelling covered
+    // grouped metrics cadence (metrics_group.cu), grow-only
+    void *grain_st = nullptr;         // per-grain statistics in site order of the roots + pairwise leaf sums of the aspect ratios
+    size_t cap_grain_st = 0;
+    void *group_tab = nullptr;        // result table of the groups this context leads (GROUP_MAX entries)
+    cudaEvent_t ev_group = nullptr;   // orders this context's stream before the work of a group led by another context
 
     // per-kernel-kind device timing (cet_profile_*): event pairs recorded around the dominant
     // kernels on the context stream, resolved when the totals are read

@@ -12,100 +12,22 @@
 //                  comes from a two-level ordered count: per-tile counts, a scan of the tile counts,
 //                  in-tile ranks by ballot);
 //   draws == NULL  Philox4x32-10 keyed by (seed, epoch, global site): the large-lattice path.
-#include "ctx.cuh"
-#include "reduce.cuh"
+#include "cadence.cuh"
 
 namespace cet {
 
-constexpr int DF_THREADS = 256, DF_PER_THREAD = 4, DF_TILE = DF_THREADS * DF_PER_THREAD;
-
-__device__ __forceinline__ void philox_round10(uint32_t c[4], uint32_t k0, uint32_t k1)
-{
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-        const uint32_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
-        c[0] = n0; c[1] = lo1; c[2] = n2; c[3] = lo0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-}
-
-struct DefectArgs {
-    uint8_t *vox;              // owned planes
-    const double *T;
-    int64_t n;                 // owned sites
-    int64_t g_off;             // global linear index of the first owned site
-    const double *draws;
-    uint64_t seed;
-    uint32_t epoch;
-    int carbon_id, defect_id, apply_to_state;
-    double base, e_mig, kT, T_default;
-    unsigned int *tile_count;      // [n_tiles + 1]: counts, then exclusive offsets
-    unsigned long long *totals;    // [0] carbon sites, [1] defects set
-};
-
-// pass 1: carbon sites per tile
 __global__ void __launch_bounds__(DF_THREADS) defects_count_kernel(const DefectArgs a)
 {
-    __shared__ int sm[DF_THREADS / 32];
-    const int64_t base = (int64_t)blockIdx.x * DF_TILE;
-    int c = 0;
-#pragma unroll
-    for (int e = 0; e < DF_PER_THREAD; ++e) {
-        const int64_t s = base + e * DF_THREADS + threadIdx.x;
-        if (s < a.n && (a.vox[s] & 15) == a.carbon_id) ++c;
-    }
-    c = warp_sum_i(c);
-    if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = c;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int t = 0;
-        for (int w = 0; w < DF_THREADS / 32; ++w) t += sm[w];
-        a.tile_count[blockIdx.x] = (unsigned)t;
-    }
+    defects_count_body(a);
 }
 
-// pass 2: exclusive scan of the tile counts (one CTA, sequential over 1024-entry strips)
 __global__ void __launch_bounds__(1024) defects_scan_kernel(unsigned int *tile_count, int n_tiles, unsigned long long *totals)
 {
-    __shared__ unsigned int sm[33];
-    __shared__ unsigned long long run;
-    if (threadIdx.x == 0) run = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int t0 = 0; t0 < n_tiles; t0 += 1024) {
-        const int q = t0 + threadIdx.x;
-        const unsigned v = q < n_tiles ? tile_count[q] : 0u;
-        unsigned inc = v;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const unsigned t = __shfl_up_sync(0xffffffffu, inc, d);
-            if (lane >= d) inc += t;
-        }
-        if (lane == 31) sm[w] = inc;
-        __syncthreads();
-        if (w == 0) {
-            unsigned x = sm[lane], xi = x;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const unsigned t = __shfl_up_sync(0xffffffffu, xi, d);
-                if (lane >= d) xi += t;
-            }
-            sm[lane] = xi - x;
-            if (lane == 31) sm[32] = xi;
-        }
-        __syncthreads();
-        const unsigned long long r0 = run;
-        if (q < n_tiles) tile_count[q] = (unsigned)(r0 + sm[w] + inc - v);      // < 2^32: fewer than 2^31 sites per context
-        __syncthreads();
-        if (threadIdx.x == 0) run = r0 + sm[32];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) totals[0] = run;
+    tile_scan_body(tile_count, n_tiles, totals);
 }
 
-// pass 3: rewrite the mask nibble of every site
+// pass 3.  The body of defects_assign_body (cadence.cuh), kept here as the kernel's own code: called through the
+// shared body, this kernel is allocated one register fewer.
 __global__ void __launch_bounds__(DF_THREADS) defects_assign_kernel(const DefectArgs a)
 {
     __shared__ int sm[DF_THREADS / 32];

@@ -13,90 +13,26 @@
 // misorientation < t  <=>  arccos(clamp(v1.v2)) < t  <=>  clamp(v1.v2) > cos t, evaluated on the
 // resident unit vectors (kmc_event_rates.py:11-23).
 #include <algorithm>
-#include "ctx.cuh"
-#include "reduce.cuh"
+#include "cadence.cuh"
 
 namespace cet {
 
-__device__ __forceinline__ int uf_find(int *label, int x)
-{
-    int p = label[x];
-    while (p != x) {                      // path halving
-        const int gp = label[p];
-        if (gp != p) label[x] = gp;
-        x = p; p = gp;
-    }
-    return x;
-}
-__device__ __forceinline__ void uf_union(int *label, int a, int b)
-{
-    while (true) {
-        a = uf_find(label, a); b = uf_find(label, b);
-        if (a == b) return;
-        if (a > b) { const int t = a; a = b; b = t; }          // a < b: hook b under a
-        const int old = atomicMin(&label[b], a);
-        if (old == b) return;
-        b = old;                                                // someone re-hooked b meanwhile: retry from there
-    }
-}
-
 __global__ void grains_init_kernel(const uint8_t *__restrict__ vox, int *label, int64_t lo, int64_t hi)
 {
-    for (int64_t s = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < hi; s += (int64_t)gridDim.x * blockDim.x)
-        label[s] = (vox[s] & 0x0F) != 0 ? (int)s : -1;
+    grains_init_body(vox, label, lo, hi);
 }
 
-// offsets 0,1,4,5,8,10,12 are one of each +/- pair of the neighbour table
-// theta == nullptr: edge iff clamp(v1.v2) > thr (thr = cos of the misorientation threshold);
-// theta != nullptr: the |theta1 - theta2| < thr criterion of utils.py:49-50 (orientation_phi=None).
 __global__ void grains_union_kernel(const uint8_t *__restrict__ vox, const Vec4 *__restrict__ v, const double *__restrict__ theta,
                                     int *label, int L, int p_lo, int p_hi, double thr)
 {
-    const int LL = L * L;
-    const int64_t lo = (int64_t)p_lo * LL, hi = (int64_t)p_hi * LL;
-    for (int64_t s = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < hi; s += (int64_t)gridDim.x * blockDim.x) {
-        if ((vox[s] & 0x0F) == 0) continue;
-        const int p = (int)(s / LL), j = (int)((s / L) % L), k = (int)(s % L);
-        Vec4 a = Vec4{0.0, 0.0, 0.0, 0.0};
-        double ta = 0.0;
-        if (theta) ta = theta[s]; else a = v[s];
-        const int pos[7] = {0, 1, 4, 5, 8, 10, 12};
-#pragma unroll
-        for (int q = 0; q < 7; ++q) {
-            const int o = pos[q];
-            const int pi = p + CET_NB_DI(o), nj = j + CET_NB_DJ(o), nk = k + CET_NB_DK(o);
-            if (pi < p_lo || pi >= p_hi || nj < 0 || nj >= L || nk < 0 || nk >= L) continue;
-            const int64_t t = s + ((int64_t)CET_NB_DI(o) * L + CET_NB_DJ(o)) * L + CET_NB_DK(o);
-            if ((vox[t] & 0x0F) == 0) continue;
-            bool edge;
-            if (theta) {
-                edge = fabs(ta - theta[t]) < thr;
-            } else {
-                const Vec4 b = v[t];
-                double dot = a.x * b.x + a.y * b.y + a.z * b.z;
-                dot = pymax(pymin(dot, 1.0), -1.0);
-                edge = dot > thr;
-            }
-            if (edge) uf_union(label, (int)s, (int)t);
-        }
-    }
+    grains_union_body(vox, v, theta, label, L, p_lo, p_hi, thr);
 }
 
 // label[s] := root of s; roots counted and given dense ids in order of arrival (the host orders
 // the grains by root index afterwards)
-struct GrainStat { int root, size, lo[3], hi[3]; };
-
 __global__ void grains_flatten_kernel(int *label, int *gid, int64_t lo, int64_t hi, unsigned int *n_roots)
 {
-    for (int64_t s = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < hi; s += (int64_t)gridDim.x * blockDim.x) {
-        int r = label[s];
-        if (r < 0) continue;
-        // read-only walk (no path halving here: a halving store by another thread could overwrite
-        // the final label of a site its owner has already flattened); owners only shorten chains
-        for (int x = (int)s; r != x;) { x = r; r = label[x]; }
-        if (r == (int)s) gid[s] = (int)atomicAdd(n_roots, 1u);
-        else label[s] = r;       // a root's own entry never changes, so concurrent walks stay valid
-    }
+    grains_flatten_body<true>(label, gid, lo, hi, n_roots);
 }
 
 __global__ void grains_stats_init_kernel(const int *__restrict__ label, const int *__restrict__ gid, int64_t lo,
@@ -104,39 +40,14 @@ __global__ void grains_stats_init_kernel(const int *__restrict__ label, const in
 {
     for (int64_t s = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < hi; s += (int64_t)gridDim.x * blockDim.x) {
         if (label[s] != (int)s) continue;
-        GrainStat g;
-        g.root = (int)s; g.size = 0;
-        g.lo[0] = g.lo[1] = g.lo[2] = 0x7fffffff;
-        g.hi[0] = g.hi[1] = g.hi[2] = -1;
-        st[gid[s]] = g;
+        grain_stat_init(st + gid[s], (int)s);
     }
 }
 
-// One atomic set per (warp, grain): lanes holding voxels of the same grain elect a leader.
 __global__ void grains_stats_kernel(const int *__restrict__ label, const int *__restrict__ gid, int64_t lo, int64_t hi,
                                     GrainStat *st, int L, int i_off)
 {
-    const int LL = L * L;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    const int lane = threadIdx.x & 31;
-    for (int64_t s0 = lo + (int64_t)blockIdx.x * blockDim.x; s0 < hi; s0 += stride) {
-        const int64_t s = s0 + threadIdx.x;
-        const int r = s < hi ? label[s] : -1;
-        const unsigned live = __ballot_sync(0xffffffffu, r >= 0);
-        if (r < 0) continue;
-        const unsigned peers = __match_any_sync(live, r);
-        const int c0 = i_off + (int)(s / LL), c1 = (int)((s / L) % L), c2 = (int)(s % L);
-        const int mn0 = __reduce_min_sync(peers, c0), mx0 = __reduce_max_sync(peers, c0);
-        const int mn1 = __reduce_min_sync(peers, c1), mx1 = __reduce_max_sync(peers, c1);
-        const int mn2 = __reduce_min_sync(peers, c2), mx2 = __reduce_max_sync(peers, c2);
-        if (lane == __ffs(peers) - 1) {
-            GrainStat *g = st + gid[r];
-            atomicAdd(&g->size, __popc(peers));
-            atomicMin(&g->lo[0], mn0); atomicMax(&g->hi[0], mx0);
-            atomicMin(&g->lo[1], mn1); atomicMax(&g->hi[1], mx1);
-            atomicMin(&g->lo[2], mn2); atomicMax(&g->hi[2], mx2);
-        }
-    }
+    grains_stats_body(label, gid, lo, hi, st, L, i_off);
 }
 
 }  // namespace cet

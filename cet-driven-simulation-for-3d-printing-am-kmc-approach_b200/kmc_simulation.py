@@ -60,7 +60,6 @@ def _replay(stream_state_setter, state, draw, n):
 def _metrics_row(step, total_time, nucleation_count, cet_detected, consts, ctx, verbose=True, all_gather=None):
     """kmc_simulation.py:341-378 — one metrics.csv row, from the lattice resident in `ctx`; with
     `all_gather` (a lattice split into z-slabs, one context per rank) from all slabs, identical on every rank."""
-    G, R, R_phys, G_over_R_phys = consts
     counts = ctx.counts()
     if all_gather is None:
         n_sites = int(np.prod(ctx.owned_shape))
@@ -70,6 +69,13 @@ def _metrics_row(step, total_time, nucleation_count, cet_detected, consts, ctx, 
         n_sites = int(ctx.n0 * ctx.owned_shape[1] * ctx.owned_shape[2])
         grains = _gpu_metrics.grains_distributed(ctx, all_gather, 0.5)
     m = _gpu_metrics.metrics_from_grains(grains, n_sites, voxel_size=constants.VOXEL_SIZE)
+    return _row_from_metrics(step, total_time, nucleation_count, cet_detected, consts, counts, m, n_sites, verbose)
+
+
+def _row_from_metrics(step, total_time, nucleation_count, cet_detected, consts, counts, m, n_sites, verbose):
+    """The metrics.csv row of _metrics_row from the state histogram `counts`, the grain metrics `m`
+    (metrics_from_grains or metrics_from_summary; updated in place) and the number of sites."""
+    G, R, R_phys, G_over_R_phys = consts
     n_w, n_re, n_c = int(counts[1]), int(counts[2]), int(counts[3])
     defect_voxels = int(counts[constants.DEFECT_ID])
     m["Defect_voxel_count"] = defect_voxels

@@ -21,6 +21,19 @@ from . import _lib
 from ._config import constants as K
 
 
+def _percentile_position(n, q):
+    """(pos, lo, hi) of np.percentile's linear method over n values: pos = q/100 * (n - 1), its floor and ceil."""
+    pos = (q / 100.0) * (n - 1)
+    return pos, int(np.floor(pos)), int(np.ceil(pos))
+
+
+def _interpolate(values, pos, lo, i_lo, i_hi):
+    a = float(values[i_lo])
+    b = float(values[i_hi])
+    t = pos - lo
+    return a + (b - a) * t if t < 0.5 else b - (b - a) * (1 - t)
+
+
 def _percentile_of_counts(values, counts, q):
     """np.percentile(np.repeat(values, counts), q) (method 'linear') without materialising the
     repeat; values ascending."""
@@ -28,12 +41,21 @@ def _percentile_of_counts(values, counts, q):
     if n == 0:
         return 0.0
     cum = np.cumsum(counts)
-    pos = (q / 100.0) * (n - 1)
-    lo, hi = int(np.floor(pos)), int(np.ceil(pos))
-    a = float(values[np.searchsorted(cum, lo, side="right")])
-    b = float(values[np.searchsorted(cum, hi, side="right")])
-    t = pos - lo
-    return a + (b - a) * t if t < 0.5 else b - (b - a) * (1 - t)
+    pos, lo, hi = _percentile_position(n, q)
+    return _interpolate(values, pos, lo, np.searchsorted(cum, lo, side="right"), np.searchsorted(cum, hi, side="right"))
+
+
+PERCENTILES = (50.0, 90.0)          # Grain_d50_um, Grain_d90_um
+
+
+def percentile_positions(n_sites):
+    """The lo and hi positions of each of PERCENTILES over n_sites values, in that order: what
+    cet_metrics_params.pct_pos takes (metrics_from_summary reads the indices the device returns for them)."""
+    out = []
+    for q in PERCENTILES:
+        _pos, lo, hi = _percentile_position(n_sites, q)
+        out += [lo, hi]
+    return out
 
 
 def grain_aspect_ratios(g):
@@ -49,13 +71,7 @@ def metrics_from_grains(g, n_sites, defects=None, voxel_size=None, rng_seed=None
     voxel_size = K.VOXEL_SIZE if voxel_size is None else voxel_size
     n = int(g["n"])
     if n == 0:
-        return {"AspectRatio": 0.0, "EquiaxedFraction": 0.0, "NucleationDensity": 0.0,
-                "AvgGrainSize": 0.0, "GrainCount": 0, "DefectDensity": 0.0,
-                "Frac_W": 0.0, "Frac_Re": 0.0, "Frac_C": 0.0,
-                "C_boundary_frac": 0.0, "Re_boundary_frac": 0.0,
-                "Defect_voxel_count": 0, "Defect_voxel_frac": 0.0,
-                "Grain_d50_um": 0.0, "Grain_d90_um": 0.0,
-                "VOXEL_SIZE_m": voxel_size, "RANDOM_SEED": rng_seed}
+        return _no_grains(voxel_size, rng_seed)
     ar = grain_aspect_ratios(g)
     sizes = g["size"].astype(np.int64)
     volume = n_sites * (voxel_size ** 3)
@@ -78,6 +94,52 @@ def metrics_from_grains(g, n_sites, defects=None, voxel_size=None, rng_seed=None
         "Defect_voxel_frac": def_count / n_sites if n_sites > 0 else 0.0,
         "Grain_d50_um": _percentile_of_counts(diam, cnts, 50.0),
         "Grain_d90_um": _percentile_of_counts(diam, cnts, 90.0),
+        "VOXEL_SIZE_m": voxel_size, "RANDOM_SEED": rng_seed,
+    }
+
+
+def _no_grains(voxel_size, rng_seed):
+    return {"AspectRatio": 0.0, "EquiaxedFraction": 0.0, "NucleationDensity": 0.0,
+            "AvgGrainSize": 0.0, "GrainCount": 0, "DefectDensity": 0.0,
+            "Frac_W": 0.0, "Frac_Re": 0.0, "Frac_C": 0.0,
+            "C_boundary_frac": 0.0, "Re_boundary_frac": 0.0,
+            "Defect_voxel_count": 0, "Defect_voxel_frac": 0.0,
+            "Grain_d50_um": 0.0, "Grain_d90_um": 0.0,
+            "VOXEL_SIZE_m": voxel_size, "RANDOM_SEED": rng_seed}
+
+
+def metrics_from_summary(res, n_sites, voxel_size=None, rng_seed=None):
+    """metrics_from_grains(g, n_sites) from the per-lattice summary of cetkmc.metrics_group (n_grains, size_sum,
+    n_equiaxed, ar_sum in NumPy's pairwise order, and the percentile indices for percentile_positions(n_sites)):
+    the same dict, value for value and type for type.  np.mean over the AR list is pw(ar) / n, over the bool
+    array n_equiaxed / n, and over the int64 sizes size_sum / n, exact below 2^53."""
+    voxel_size = K.VOXEL_SIZE if voxel_size is None else voxel_size
+    n = int(res["n_grains"])
+    if n == 0:
+        return _no_grains(voxel_size, rng_seed)
+    volume = n_sites * (voxel_size ** 3)
+    def_count = 0
+    # the diameters of the grain numbers 0..n, as metrics_from_grains evaluates them
+    vals = np.arange(0, n + 1, dtype=np.float64)
+    diam = ((6.0 * (vals * (voxel_size ** 3)) / np.pi) ** (1.0 / 3.0)) * 1e6
+    idx = [int(i) for i in res["pct_index"]]
+    d = []
+    for k, q in enumerate(PERCENTILES):
+        pos, lo, _hi = _percentile_position(n_sites, q)
+        d.append(_interpolate(diam, pos, lo, idx[2 * k], idx[2 * k + 1]))
+    return {
+        "AspectRatio": np.float64(res["ar_sum"]) / n,
+        "EquiaxedFraction": np.float64(res["n_equiaxed"]) / n,
+        "NucleationDensity": n / volume if volume > 0 else 0.0,
+        "AvgGrainSize": np.float64(res["size_sum"]) / n * voxel_size * 1e6,
+        "GrainCount": n,
+        "DefectDensity": def_count / volume if volume > 0 else 0.0,
+        "Frac_W": 0.0, "Frac_Re": 0.0, "Frac_C": 0.0,
+        "C_boundary_frac": 0.0, "Re_boundary_frac": 0.0,
+        "Defect_voxel_count": def_count,
+        "Defect_voxel_frac": def_count / n_sites if n_sites > 0 else 0.0,
+        "Grain_d50_um": d[0],
+        "Grain_d90_um": d[1],
         "VOXEL_SIZE_m": voxel_size, "RANDOM_SEED": rng_seed,
     }
 

@@ -92,6 +92,31 @@ typedef struct cet_sweep_result {
     int64_t sites_refreshed;   /* sites whose rates the neighbour-rate updates re-evaluated */
 } cet_sweep_result;
 
+/* Per-context arguments of cet_metrics_group. */
+typedef struct cet_metrics_params {
+    double theta_threshold;    /* grain misorientation threshold in rad (metrics.py:43 passes 0.5) */
+    double ar_threshold;       /* n_equiaxed counts the grains with aspect ratio < ar_threshold */
+    int64_t pct_pos[4];        /* positions x whose searchsorted(cum, x, side="right") pct_index returns */
+    int32_t refresh;           /* != 0: redraw the defect mask first, as cet_defects_refresh(apply_to_state = 0) */
+    int32_t carbon_id;         /* the refresh's arguments (1..15) ... */
+    uint32_t epoch;
+    int32_t pad_;
+    uint64_t seed;
+    double prob_base, e_mig, kT, T_default;
+} cet_metrics_params;
+
+/* What one metrics row (metrics.py:41-96) needs of a lattice, from cet_metrics_group. */
+typedef struct cet_metrics_result {
+    int64_t counts[16];        /* histogram of the owned states (cet_counts) */
+    int64_t n_carbon;          /* the refresh's carbon sites and sites with the mask set (0 without a refresh) */
+    int64_t n_defects;
+    int64_t n_grains;
+    int64_t size_sum;          /* voxels over all grains */
+    int64_t n_equiaxed;        /* grains with aspect ratio < ar_threshold */
+    int64_t pct_index[4];      /* searchsorted(cum, pct_pos[k], side="right"), cum = cumsum([n_sites - size_sum, sizes...]) */
+    double ar_sum;             /* sum of the grains' aspect ratios in cluster order, in NumPy's pairwise order */
+} cet_metrics_result;
+
 /* ---- library ---- */
 const char *cet_last_error(void);
 int cet_abi_version(void);
@@ -220,6 +245,24 @@ int cet_grains_stats(cet_ctx *ctx, int64_t cap, int32_t *root, int32_t *size, in
                      int32_t *box_hi);
 /* Label volume: root site index per occupied site, -1 for empty sites (owned planes). */
 int cet_grains_download_labels(cet_ctx *ctx, int32_t *labels);
+
+/* ---- grouped metrics cadence (kmc_simulation.py:335-378 for many lattices at once) ----
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device; 1 <= n_ctx <= 64.
+ * The work is ordered on the stream of ctxs[0] after the work already queued on every context's stream, each
+ * kernel is one launch for the whole group, and the call returns when the work is done.
+ * cet_counts_group: counts[16 * q + s] = cet_counts(ctxs[q])[s]; one host synchronisation. */
+int cet_counts_group(cet_ctx *const *ctxs, int32_t n_ctx, int64_t *counts);
+/* Per context q: if mp[q].refresh, the defect mask is redrawn exactly as cet_defects_refresh(ctxs[q], draws[q],
+ * n_draws[q], mp[q].seed, mp[q].epoch, ..., apply_to_state = 0) redraws it (draws == NULL or draws[q] == NULL: the
+ * Philox stream; else n_draws[q] must cover the lattice's carbon sites); then the grains are labelled as
+ * cet_grains_label_ex(ctxs[q], mp[q].theta_threshold, 0, ...) labels them, and cet_grains_stats /
+ * cet_grains_download_labels report that labelling afterwards; res[q] receives the histogram, the refresh's counts
+ * and the grain reductions of a metrics row.  Everything but the carbon-site count is checked before the device
+ * is used; that count is checked before any mask byte is written: a rejected call leaves every context as it was.
+ * Three host synchronisations per call whatever n_ctx (carbon counts, grain counts, results); no device
+ * allocation once the per-context buffers have grown to the lattice's needs. */
+int cet_metrics_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_metrics_params *mp, const double *const *draws,
+                      const int64_t *n_draws, cet_metrics_result *res);
 /* The same for global planes [i_lo, i_hi) within the labelled planes of a slab (owned + 2 ghost planes per
  * cut face): what two neighbouring slabs compare to join the grains that cross their cut. */
 int cet_grains_download_planes(cet_ctx *ctx, int64_t i_lo, int64_t i_hi, int32_t *labels);

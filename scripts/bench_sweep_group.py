@@ -151,7 +151,7 @@ def driver(n_cases_side=4, L=96, n_sweeps=401, order=(None, 16, None, 16)):
 
     targets = [(campaign, "_upload_initial", "setup"), (_lib.Context, "__init__", "setup"),
                (_lib.Context, "set_rate_params", "setup"), (_lib.Context, "sweep_run", "sweeps"),
-               (_lib, "sweep_run_group", "sweeps"), (campaign, "_cadence", "cadence"),
+               (_lib, "sweep_run_group", "sweeps"), (campaign, "_cadence", "cadence"), (campaign, "_cadence_group", "cadence"),
                (_lib.Context, "download", "final_download"), (_lib.Context, "close", "close"),
                (ks, "_write_csv", "csv")]
     saved = [(obj, name, getattr(obj, name)) for obj, name, _k in targets]

@@ -101,6 +101,7 @@ SIGNATURES = {
     "cet_counts": [_VP, C.POINTER(_I64 * 16)],
     "cet_thermal_cet": [_VP, C.POINTER(ThermalParams)],
     "cet_thermal_full": [_VP, C.POINTER(ThermalFullParams), _VP],
+    "cet_thermal_full_group": [C.POINTER(_VP), _I32, C.POINTER(ThermalFullParams), C.POINTER(_VP), _I32],
     "cet_thermal_fill_gradient": [_VP, _F64, _F64],
     "cet_rates_build": [_VP],
     "cet_rates_total": [_VP, C.POINTER(_F64), C.POINTER(_I64)],
@@ -541,6 +542,30 @@ def sweep_run_group(ctxs, n_sweeps, sps, tps=None):
     res = (SweepResult * n)()
     check(lib().cet_sweep_run_group(handles, n, int(n_sweeps), sp_arr, tp_arr, res), "cet_sweep_run_group")
     return [{f: getattr(r, f) for f, _ in SweepResult._fields_ if f != "pad_"} for r in res]
+
+
+def thermal_full_group(ctxs, params, q_tops, snapshot=True):
+    """update_temperature on a group of whole-lattice Contexts of one L on one device, one stencil launch for the
+    group: context q takes params[q] (ThermalFullParams) and the source plane q_tops[q] (an (L, L) C-contiguous
+    float64 array, thermal_solver.laser_source_top).  Every context ends exactly as its own
+    ctx.thermal_full(params[q], q_tops[q]) followed, with snapshot=True, by ctx.snapshot_state() would leave it."""
+    ctxs, params, q_tops = list(ctxs), list(params), list(q_tops)
+    n = len(ctxs)
+    if len(params) != n:
+        raise ValueError(f"thermal_full_group: {len(params)} params for {n} contexts")
+    if len(q_tops) != n:
+        raise ValueError(f"thermal_full_group: {len(q_tops)} source planes for {n} contexts")
+    if any(not isinstance(p, ThermalFullParams) for p in params):
+        raise TypeError("thermal_full_group: params must be ThermalFullParams")
+    handles = _group_handles("thermal_full_group", ctxs)
+    for q, (c, a) in enumerate(zip(ctxs, q_tops)):
+        if not isinstance(a, np.ndarray) or a.dtype != np.float64 or not a.flags.c_contiguous:
+            raise TypeError(f"thermal_full_group: q_tops[{q}] must be a C-contiguous float64 array")
+        if tuple(a.shape) != tuple(c.shape[1:]):
+            raise ValueError(f"thermal_full_group: q_tops[{q}] has shape {a.shape}, the lattice needs {tuple(c.shape[1:])}")
+    tfp = (ThermalFullParams * n)(*params)
+    q_ptr = (C.c_void_p * n)(*[a.ctypes.data for a in q_tops])
+    check(lib().cet_thermal_full_group(handles, n, tfp, q_ptr, 1 if snapshot else 0), "cet_thermal_full_group")
 
 
 def _group_handles(fn, ctxs):

@@ -10,6 +10,9 @@
                                      18 columns; optionally the laser / latent-heat thermal step
                                      (thermal_solver.update_temperature, :36-105) with a melt pool
                                      moving along axis 1 at a fixed speed — SURVEY §8d config 3
+    run_melt_pool_map                a CET map over laser power x scan speed: one laser-driven
+                                     run_cet_sublattice per point, optionally advanced in groups
+                                     (cetkmc.thermal_full_group + sweep_run_group)
     run_gr_sweep                     config 5: independent lattices over a grid of (G, R), one per
                                      GPU (replicas only, no communication), one cet_map.csv and a tree
                                      the unmodified plot_cet.py reads (write_plot_cet_tree)
@@ -365,20 +368,27 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
 
 
 def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
-                       events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy"):
+                       events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy",
+                       lasers=None):
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
     around its host draws).  The metrics cadence of the group is one cetkmc.metrics_group call per row
-    (_cadence_group).  A case that terminates stops at the row it stops at alone and leaves the group."""
+    (_cadence_group).  A case that terminates stops at the row it stops at alone and leaves the group.
+    lasers: None, or one laser dict per case (run_cet_sublattice(laser=...)): every `thermal_every` sweeps one
+    cetkmc.thermal_full_group over the cases still running replaces their thermal_full + snapshot_state, and a case
+    that terminates leaves the group after the block of sweeps it terminated in, with its row at that block's last
+    sweep, as the laser driver of run_cet_sublattice stops it."""
     if mask_stream not in ("numpy", "philox"):
         raise ValueError("mask_stream must be 'numpy' or 'philox'")
+    if lasers is not None and int(thermal_every) <= 0:
+        raise ValueError("the laser variant needs thermal_every >= 1")
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
     philox_mask = mask_stream == "philox"
     runs = []
     try:
-        for prefix, temp, nu_dep in cases:
+        for q, (prefix, temp, nu_dep) in enumerate(cases):
             np.random.seed(seed)
             os.makedirs(f"outputs/{prefix}", exist_ok=True)
             ctx = _lib.Context(L=L, device=device)
@@ -387,28 +397,129 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
             runs.append(r)
             ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
             _upload_initial(ctx, L, n_seeds, temp, impurity_c, None, 0, L)
-            r["sp"], r["tp"] = _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction, thermal_every)
+            r["sp"], r["tp"] = _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction,
+                                            0 if lasers is not None else thermal_every)
             r["rng"] = np.random.get_state()
+            if lasers is not None:
+                r["laser"] = lasers[q]
+                r["tfp"] = thermal_full_params(float(lasers[q].get("dt", _ks.THERMAL_DT)))
+                r["pos"] = [float(x) for x in lasers[q].get("start", (0.0, 0.0))]
+                ctx.snapshot_state()
         sweep = 0
         active = runs
         while sweep < n_sweeps and active:
-            n = _stop_at(sweep, every, n_sweeps) - sweep + 1
-            tps = None if active[0]["tp"] is None else [r["tp"] for r in active]     # one thermal_every for all cases
-            results = _lib.sweep_run_group([r["ctx"] for r in active], n, [r["sp"] for r in active], tps)
-            sweep += n
-            for r, res in zip(active, results):
-                if res["overflow"]:
-                    raise RuntimeError("fired-event list overflowed: lower events_per_sweep")
-                r["total_time"] += res["time"]
-                r["nucleation_count"] += res["nucleation_count"]
-                r["terminated"] = bool(res["terminated"]) or res["sweeps_done"] == 0
-            _cadence_group(active, sweep - 1, every, philox_mask, seed)
+            end = _stop_at(sweep, every, n_sweeps) + 1
+            if lasers is None:
+                tps = None if active[0]["tp"] is None else [r["tp"] for r in active]     # one thermal_every for all cases
+                _absorb(active, _lib.sweep_run_group([r["ctx"] for r in active], end - sweep, [r["sp"] for r in active], tps))
+                sweep = end
+            else:
+                while sweep < end and active:
+                    blk = min(end - sweep, thermal_every - sweep % thermal_every)
+                    if sweep % thermal_every == 0:
+                        _laser_step_group(active, L)
+                    _absorb(active, _lib.sweep_run_group([r["ctx"] for r in active], blk, [r["sp"] for r in active]))
+                    sweep += blk
+                    stopped = [r for r in active if r["terminated"]]
+                    if stopped:
+                        _cadence_group(stopped, sweep - 1, every, philox_mask, seed)
+                        active = [r for r in active if not r["terminated"]]
+            if active:
+                _cadence_group(active, sweep - 1, every, philox_mask, seed)
             active = [r for r in active if not r["terminated"]]
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
     finally:
         for r in runs:
             r["ctx"].close()
+
+
+def _absorb(runs, results):
+    """Add the sweep results of a group to its cases' running totals."""
+    for r, res in zip(runs, results):
+        if res["overflow"]:
+            raise RuntimeError("fired-event list overflowed: lower events_per_sweep")
+        r["total_time"] += res["time"]
+        r["nucleation_count"] += res["nucleation_count"]
+        r["terminated"] = bool(res["terminated"]) or res["sweeps_done"] == 0
+
+
+def _laser_step_group(runs, L):
+    """The laser driver's thermal step of run_cet_sublattice (thermal_full, snapshot_state, the melt pool moves on)
+    for every case of `runs`, one cetkmc.thermal_full_group call."""
+    q_tops = []
+    for r in runs:
+        las = r["laser"]
+        q_tops.append(laser_source_top(L, tuple(r["pos"]), float(las["power"]),
+                                       float(las.get("beam_radius", DEFAULT_BEAM_RADIUS)),
+                                       float(las.get("absorptivity", DEFAULT_ABSORPTIVITY))))
+    _lib.thermal_full_group([r["ctx"] for r in runs], [r["tfp"] for r in runs], q_tops, snapshot=True)
+    for r in runs:
+        r["pos"][1] += float(r["laser"].get("speed", 0.0))
+
+
+def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None, start=(0.0, 0.0), dt=None,
+                      beam_radius=DEFAULT_BEAM_RADIUS, absorptivity=DEFAULT_ABSORPTIVITY, impurity_c=0.0, n_seeds=20,
+                      defect_fraction=0.0, output_root="melt_pool_map", rank=None, world=None, devices=None,
+                      batch=None, **kw):
+    """A CET map over the two quantities of the moving melt pool a user sets: beam power (W) and scan speed (voxels
+    per thermal step along axis 1).  Case q of powers x speeds (in that order) is run_cet_sublattice(laser=dict(
+    power=P, speed=V, start=start, dt=dt, beam_radius=..., absorptivity=...), output_prefix=
+    "<output_root>/P<P>_V<V>"), every case with the same temp, nu_dep, seed and cadence.  Cases are partitioned over
+    ranks and devices as in run_gr_sweep (gr_partition).  Every case writes its own metrics.csv; each rank writes
+    outputs/<output_root>/melt_pool_map_rank<r>.csv (case, power, speed, T_sub, NU_DEP, G, R, G_over_R and the final
+    row's Step, Time, AspectRatio, EquiaxedFraction, GrainCount, AvgGrainSize, NucleationCount, CET_Class,
+    CET_Detected) and adds its cases to the plot_cet tree; merge_melt_pool_map() joins the rank files.
+    batch=k: the cases of one device advance in groups of up to k lattices (cetkmc.sweep_run_group for the sweeps,
+    cetkmc.thermal_full_group for the laser steps); every output file is the same as with batch=None.  Not with
+    `checkpoint_every`, `resume_from` or `lattice`."""
+    rank = int(os.environ.get("RANK", 0)) if rank is None else rank
+    world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
+    local = int(os.environ.get("LOCAL_RANK", 0))
+    devices = [local] if devices is None else list(devices)
+    powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
+    if not powers or not speeds:
+        raise ValueError("run_melt_pool_map: needs at least one power and one speed")
+    if int(kw.get("thermal_every", _ks.THERMAL_EVERY)) < 1:
+        raise ValueError("run_melt_pool_map: the laser step needs thermal_every >= 1")
+    if batch is not None:
+        bad = [k for k in ("checkpoint_every", "resume_from", "lattice") if kw.get(k)]
+        if bad:
+            raise ValueError(f"run_melt_pool_map: batch does not take {', '.join(bad)}")
+    temp = constants.T_SUB if temp is None else float(temp)
+    nu_dep = constants.NU_DEP if nu_dep is None else float(nu_dep)
+    dt = _ks.THERMAL_DT if dt is None else float(dt)
+    cases = [(p, v) for p in powers for v in speeds]
+    lasers = [dict(power=p, speed=v, start=tuple(start), dt=dt, beam_radius=beam_radius, absorptivity=absorptivity)
+              for p, v in cases]
+    prefix = [f"{output_root}/P{p:g}_V{v:g}" for p, v in cases]
+    out_dir = f"outputs/{output_root}"
+    os.makedirs(out_dir, exist_ok=True)
+    parts = gr_partition(len(cases), rank, world, devices, batch)
+    for device, qs in parts:
+        if batch is None:
+            q = qs[0]
+            run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=temp, nu_dep=nu_dep, impurity_c=impurity_c, n_seeds=n_seeds,
+                               defect_fraction=defect_fraction, output_prefix=prefix[q], laser=lasers[q], device=device,
+                               verbose=False, **kw)
+        else:
+            _run_cases_grouped([(prefix[q], temp, nu_dep) for q in qs], L=L, n_sweeps=n_sweeps, impurity_c=impurity_c,
+                               n_seeds=n_seeds, defect_fraction=defect_fraction, device=device,
+                               lasers=[lasers[q] for q in qs], **kw)
+    import csv
+    G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
+    rows = []
+    for q in sorted(q for _d, qs in parts for q in qs):
+        with open(f"outputs/{prefix[q]}/metrics.csv") as fh:
+            last = list(csv.DictReader(fh))[-1]
+        rows.append({"case": q, "power": cases[q][0], "speed": cases[q][1], "T_sub": temp, "NU_DEP": nu_dep, "G": G,
+                     "R": R, "G_over_R": G / R if R > 0 else np.inf,
+                     **{k: last[k] for k in ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize",
+                                             "NucleationCount", "CET_Class", "CET_Detected")}})
+    _write_rows(rows, os.path.join(out_dir, f"melt_pool_map_rank{rank}.csv"))
+    write_plot_cet_tree([(r["case"], f"outputs/{prefix[r['case']]}/metrics.csv") for r in rows],
+                        os.path.join(out_dir, "plot_cet"))
+    return rows
 
 
 def write_plot_cet_tree(cases, root):
@@ -437,14 +548,24 @@ def _write_rows(rows, path):
         w.writerows(rows)
 
 
-def merge_cet_map(output_root="gr_sweep"):
-    """Join the per-rank files of run_gr_sweep into outputs/<output_root>/cet_map.csv (sorted by case)."""
+def _merge_rank_files(output_root, name):
+    """Join outputs/<output_root>/<name>_rank*.csv into outputs/<output_root>/<name>.csv (sorted by case)."""
     import csv
     import glob
     rows = []
-    for p in sorted(glob.glob(f"outputs/{output_root}/cet_map_rank*.csv")):
+    for p in sorted(glob.glob(f"outputs/{output_root}/{name}_rank*.csv")):
         with open(p) as fh:
             rows += list(csv.DictReader(fh))
     rows.sort(key=lambda r: int(r["case"]))
-    _write_rows(rows, f"outputs/{output_root}/cet_map.csv")
+    _write_rows(rows, f"outputs/{output_root}/{name}.csv")
     return rows
+
+
+def merge_cet_map(output_root="gr_sweep"):
+    """Join the per-rank files of run_gr_sweep into outputs/<output_root>/cet_map.csv (sorted by case)."""
+    return _merge_rank_files(output_root, "cet_map")
+
+
+def merge_melt_pool_map(output_root="melt_pool_map"):
+    """Join the per-rank files of run_melt_pool_map into outputs/<output_root>/melt_pool_map.csv (sorted by case)."""
+    return _merge_rank_files(output_root, "melt_pool_map")

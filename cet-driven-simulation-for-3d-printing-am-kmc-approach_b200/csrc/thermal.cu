@@ -16,6 +16,7 @@
 // in registers, so each T value is fetched from L2/HBM once along i; the j and k neighbours
 // come from L1 (same CTA touches the adjacent rows) and warp shuffles.
 #include "ctx.cuh"
+#include "tile_state.cuh"
 
 namespace cet {
 
@@ -49,10 +50,26 @@ constexpr int TH_TK = 128;   // threads along k
 constexpr int TH_TJ = 4;     // rows per CTA
 constexpr int TH_PLANES = 8; // planes marched per CTA
 
+// What cet_thermal_full_group fuses into the full stencil pass of a lattice: the thread that reads vox_prev[s] and
+// vox[s] for its centre site s then writes vox_prev[s] = vox[s] (cet_snapshot_state), and, while the lattice's tile
+// state is valid, an empty site's pair operand takes its new temperature (tile_pairop_T).  Kept out of ThermalArgs,
+// which the solo kernels take by value.
+struct ThermalFuse {
+    uint8_t *vox_prev;               // snapshot target (NULL: no snapshot)
+    const uint8_t *cvox;             // NULL: the tile state is stale and stays so
+    double *pairop;
+};
+__device__ __forceinline__ void thermal_fuse_site(const ThermalArgs &a, const ThermalFuse *x, int64_t s, double v)
+{
+    if (x->vox_prev) x->vox_prev[s] = a.vox[s];
+    if (x->cvox && (x->cvox[s] & 15u) == TC_EMPTY) x->pairop[s] = v;
+}
+
 // The kernel bodies take their arguments by reference and the plane block `zb` (blockIdx.z of a solo launch): the
-// grouped launches of cet_sweep_run_group run them for the table entry of their lattice.
-template <bool FULL>
-__device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb)
+// grouped launches of cet_sweep_run_group and cet_thermal_full_group run them for the table entry of their lattice.
+// FUSE (full variant, whole-lattice contexts, no stop flag): x holds the fused writes of ThermalFuse.
+template <bool FULL, bool FUSE = false>
+__device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb, const ThermalFuse *x = nullptr)
 {
     const int k = blockIdx.x * TH_TK + threadIdx.x;
     const int j = blockIdx.y * TH_TJ + threadIdx.y;
@@ -102,6 +119,7 @@ __device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb)
         if (v < a.lo) v = a.lo;       // np.clip: NaN stays NaN
         if (v > a.hi) v = a.hi;
         a.Tout[(int64_t)p * plane + (int64_t)j * a.n2 + k] = v;
+        if constexpr (FUSE) thermal_fuse_site(a, x, (int64_t)p * plane + (int64_t)j * a.n2 + k, v);
         below = centre;
         centre = above;
     }
@@ -134,8 +152,8 @@ struct RowVec {
     }
 };
 
-template <bool FULL, bool NANFIX, int V>
-__device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb)
+template <bool FULL, bool NANFIX, int V, bool FUSE = false>
+__device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb, const ThermalFuse *x = nullptr)
 {
     const int lane = threadIdx.x;
     const int k0 = (blockIdx.x * 32 + lane) * V;
@@ -207,6 +225,10 @@ __device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb)
                 if (stop) o = *reinterpret_cast<const double2 *>(pc + e);
                 else { o.x = out[e]; o.y = out[e + 1]; }
                 *reinterpret_cast<double2 *>(po + e) = o;
+            }
+            if constexpr (FUSE) {                             // lanes past n2 read a borrowed address: they write nothing
+#pragma unroll
+                for (int e = 0; e < V; ++e) thermal_fuse_site(a, x, (int64_t)p * plane + (int64_t)j * a.n2 + kc + e, out[e]);
             }
         }
         below = centre;
@@ -387,6 +409,50 @@ int thermal_cet_step_group(cet_ctx *const *cs, const cet_thermal_params *const *
     return 0;
 }
 
+// Grouped update_temperature (cet_thermal_full_group): blockIdx.z = lattice * nzb + plane block, the full stencil
+// with the fused snapshot / pair-operand writes.  V = 0: the scalar kernel (odd n2).
+struct ThermalFullGroupArgs {
+    ThermalArgs t;
+    ThermalFuse x;
+};
+static_assert(group_fits<ThermalFullGroupArgs>(), "a table of GROUP_MAX entries must fit the kernel parameter space");
+
+template <int V, int CAP>
+__global__ void __launch_bounds__(V ? 32 * TH2_TJ : TH_TK * TH_TJ)
+thermal_full_group_kernel(const __grid_constant__ GroupArgs<ThermalFullGroupArgs, CAP> g, int nzb)
+{
+    const ThermalFullGroupArgs &a = g.a[blockIdx.z / nzb];
+    if constexpr (V == 0) thermal_body<true, true>(a.t, blockIdx.z % nzb, &a.x);
+    else thermal_v2_body<true, false, V, true>(a.t, blockIdx.z % nzb, &a.x);
+}
+
+template <int V, int CAP>
+static int thermal_full_group_launch(cet_ctx *c0, const ThermalFullGroupArgs *args, int n)
+{
+    GroupArgs<ThermalFullGroupArgs, CAP> g;
+    for (int q = 0; q < n; ++q) g.a[q] = args[q];
+    const int planes = args[0].t.p_hi - args[0].t.p_lo;
+    dim3 block, grid;
+    int nzb;
+    if (V) {
+        nzb = (planes + TH2_PLANES - 1) / TH2_PLANES;
+        block = dim3(32, TH2_TJ);
+        grid = dim3((unsigned)((c0->n2 / V + 31) / 32), (unsigned)((c0->n1 + TH2_TJ - 1) / TH2_TJ), (unsigned)(nzb * n));
+    } else {
+        nzb = (planes + TH_PLANES - 1) / TH_PLANES;
+        block = dim3(TH_TK, TH_TJ);
+        grid = dim3((unsigned)((c0->n2 + TH_TK - 1) / TH_TK), (unsigned)((c0->n1 + TH_TJ - 1) / TH_TJ), (unsigned)(nzb * n));
+    }
+    thermal_full_group_kernel<V, CAP><<<grid, block, 0, c0->stream>>>(g, nzb);
+    CET_CUDA(cudaGetLastError());
+    return 0;
+}
+template <int V>
+static int thermal_full_group_launch(cet_ctx *c0, const ThermalFullGroupArgs *args, int n)
+{
+    return n <= 16 ? thermal_full_group_launch<V, 16>(c0, args, n) : thermal_full_group_launch<V, GROUP_MAX>(c0, args, n);
+}
+
 }  // namespace cet
 
 using namespace cet;
@@ -419,6 +485,69 @@ int cet_thermal_full(cet_ctx *c, const cet_thermal_full_params *p, const double 
     c->tile_valid = false;
     if (rc) return rc;
     CET_CUDA(cudaStreamSynchronize(c->stream));   // q_top host pointer is borrowed for the call only
+    return 0;
+}
+
+// cet_thermal_full (+ cet_snapshot_state) for a group of whole-lattice contexts of one L: one stencil launch for the
+// group, on the stream of ctxs[0] after the work queued on every context's stream, one host synchronisation.
+int cet_thermal_full_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_thermal_full_params *p,
+                           const double *const *q_top, int32_t snapshot)
+{
+    CET_REQUIRE(ctxs && p && q_top, "cet_thermal_full_group: NULL argument");
+    CET_REQUIRE(n_ctx >= 1 && n_ctx <= GROUP_MAX, "cet_thermal_full_group: need 1 <= n_ctx <= %d, got %d", GROUP_MAX,
+                (int)n_ctx);
+    for (int q = 0; q < n_ctx; ++q) {
+        const cet_ctx *c = ctxs[q];
+        CET_REQUIRE(c, "cet_thermal_full_group: context %d is NULL", q);
+        for (int r = 0; r < q; ++r) CET_REQUIRE(ctxs[r] != c, "cet_thermal_full_group: context %d repeats context %d", q, r);
+        CET_REQUIRE(c->device == ctxs[0]->device, "cet_thermal_full_group: context %d is on another device", q);
+        CET_REQUIRE(c->world == 1 && c->halo == 0 && c->i_begin == 0 && c->i_end == c->n0,
+                    "cet_thermal_full_group: context %d is a slab; groups take whole-lattice contexts", q);
+        CET_REQUIRE(c->cubic, "cet_thermal_full_group: context %d is not a cubic lattice", q);
+        CET_REQUIRE(c->n1 == ctxs[0]->n1, "cet_thermal_full_group: context %d has L = %lld, context 0 L = %lld", q,
+                    (long long)c->n1, (long long)ctxs[0]->n1);
+        CET_REQUIRE(q_top[q], "cet_thermal_full_group: q_top[%d] is NULL", q);
+        CET_REQUIRE(c->vox_prev != nullptr,
+                    "cet_thermal_full_group: context %d: no previous state (call cet_upload_prev_state or cet_snapshot_state)", q);
+    }
+    cet::DeviceGuard dg(ctxs[0]->device);
+    cet_ctx *c0 = ctxs[0];
+    ThermalFullGroupArgs args[GROUP_MAX];
+    for (int q = 0; q < n_ctx; ++q) {
+        cet_ctx *c = ctxs[q];
+        ThermalFullGroupArgs &g = args[q];
+        memset(&g, 0, sizeof(g));
+        ThermalArgs &a = g.t;
+        a.vox = c->vox; a.vox_prev = c->vox_prev;
+        a.inv_dx2 = p[q].inv_dx2; a.lo = p[q].lo; a.hi = p[q].hi;
+        a.dt = p[q].dt; a.alpha = p[q].alpha; a.rho_cp = p[q].rho_cp; a.latent_over_cp = p[q].latent_over_cp;
+        a.inv_dt_latent = 1.0 / (p[q].dt > 1e-12 ? p[q].dt : 1e-12);   // as cet_thermal_full
+        thermal_geometry(c, a);
+        CET_REQUIRE(a.p_lo == 0 && a.p_hi == (int)c->np, "cet_thermal_full_group: whole-lattice contexts only");
+        g.x.vox_prev = snapshot ? c->vox_prev : nullptr;
+        if (c->tile_valid) { g.x.cvox = c->cvox; g.x.pairop = c->pairop; }
+    }
+    for (int q = 0; q < n_ctx; ++q) {
+        cet_ctx *c = ctxs[q];
+        if (!c->q_top) CET_CUDA(cudaMalloc(&c->q_top, c->plane * sizeof(double)));
+        args[q].t.q_top = c->q_top;
+        if (c != c0) {
+            if (!c->ev_group) CET_CUDA(cudaEventCreateWithFlags(&c->ev_group, cudaEventDisableTiming));
+            CET_CUDA(cudaEventRecord(c->ev_group, c->stream));
+            CET_CUDA(cudaStreamWaitEvent(c0->stream, c->ev_group, 0));
+        }
+    }
+    for (int q = 0; q < n_ctx; ++q)
+        CET_CUDA(cudaMemcpyAsync(ctxs[q]->q_top, q_top[q], c0->plane * sizeof(double), cudaMemcpyHostToDevice, c0->stream));
+    {
+        ProfScope ps(c0, PROF_THERMAL);
+        const int V = c0->n2 % 4 == 0 ? 4 : c0->n2 % 2 == 0 ? 2 : 0;
+        const int rc = V == 4 ? thermal_full_group_launch<4>(c0, args, n_ctx)
+                     : V == 2 ? thermal_full_group_launch<2>(c0, args, n_ctx) : thermal_full_group_launch<0>(c0, args, n_ctx);
+        if (rc) return rc;
+    }
+    CET_CUDA(cudaStreamSynchronize(c0->stream));   // the q_top host pointers are borrowed for the call only
+    for (int q = 0; q < n_ctx; ++q) thermal_done(ctxs[q], args[q].t, true);   // tile_valid as it was: see ThermalFuse
     return 0;
 }
 

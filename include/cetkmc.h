@@ -160,6 +160,19 @@ int cet_counts(cet_ctx *ctx, int64_t counts[16]); /* histogram of state values, 
 int cet_thermal_cet(cet_ctx *ctx, const cet_thermal_params *p);
 /* update_temperature (thermal_solver.py:36): q_top[n1*n2] = I_surface/VOXEL_SIZE (host pointer). */
 int cet_thermal_full(cet_ctx *ctx, const cet_thermal_full_params *p, const double *q_top);
+/* update_temperature for n_ctx whole-lattice contexts of one L in one stencil launch: context q takes p[q] and the
+ * host source plane q_top[q] (L*L doubles, borrowed for the call).  Each context ends exactly as
+ * cet_thermal_full(ctxs[q], &p[q], q_top[q]) followed, when snapshot != 0, by cet_snapshot_state(ctxs[q]) would
+ * leave it; the snapshot is written by the stencil pass itself.  A context whose sweep tile state is current also
+ * gets the new temperature of its empty sites' pair operands in that pass and keeps its tile state (a solo call
+ * drops it and the next sweep rebuilds it, with the same bits); a stale tile state stays stale.
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device, each with a
+ * previous state (cet_upload_prev_state / cet_snapshot_state); 1 <= n_ctx <= 64.  Everything is checked before
+ * anything is copied or launched, so a rejected call leaves every context as it was.  The work is ordered on the
+ * stream of ctxs[0] after the work already queued on every context's stream: one H2D copy per context, one launch,
+ * one host synchronisation.  When profiling is enabled on ctxs[0], the launch is recorded there as a thermal span. */
+int cet_thermal_full_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_thermal_full_params *p,
+                           const double *const *q_top, int32_t snapshot);
 /* build_temperature_field (thermal_solver.py:15): T[i,:,:] = t0 + g*i. */
 int cet_thermal_fill_gradient(cet_ctx *ctx, double t0, double g);
 

@@ -49,6 +49,43 @@ def initialize_lattice(lattice_size=None, n_seeds=None, T_sub=None, T_melt=None,
     return state, theta, phi, T, atom_type
 
 
+def initial_nuclei(L, n_seeds, T_sub, random_seed, impurity_c, T_melt=None):
+    """initialize_lattice(L, n_seeds, T_sub, T_melt, random_seed, impurity_c) followed by
+    introduce_defects(state, atom_type, T, apply_to_state=False) in sparse form, consuming NumPy's global stream
+    exactly as that pair does.  The initial lattice is empty but for the nuclei on the k = 0 plane, and T depends
+    on k only.  Returns (site, byte, theta, phi, T_row):
+        site   int64 (n,)  C-order flat site index of each nucleus, in draw order
+        byte   uint8 (n,)  atom | defect << 4
+        theta, phi  float64 (n,)
+        T_row  float64 (L,)  the temperature along k that the dense T repeats over (i, j)."""
+    T_melt = K.T_MELT if T_melt is None else T_melt
+    np.random.seed(random_seed)
+    grad = (T_melt - T_sub) / L
+    T_row = T_sub + grad * np.arange(L)
+    flat = np.random.choice(L * L, n_seeds, replace=False)
+    n = len(flat)
+    atom = np.empty(n, np.uint8)
+    theta, phi = np.empty(n), np.empty(n)
+    for q in range(n):
+        r = np.random.random()
+        atom[q] = 2 if r < K.IMPURITY_RE else (3 if r < K.IMPURITY_RE + impurity_c else 1)
+        theta[q] = np.random.uniform(0, np.pi)
+        phi[q] = np.random.uniform(0, 2 * np.pi)
+    site = np.asarray(flat, dtype=np.int64) * L
+    defect = np.zeros(n, np.uint8)
+    carbon = np.flatnonzero(atom == 3)
+    if len(carbon):
+        # introduce_defects draws one number per carbon site in C order, and every carbon site has T = T_row[0]
+        carbon = carbon[np.argsort(site[carbon])]
+        tv = np.full(len(carbon), T_row[0])
+        with np.errstate(divide="ignore", invalid="ignore"):
+            tv = np.where(tv > 0, tv, K.T_SUB)
+            prob = K.DEFECT_PROB_BASE * np.exp(-0.3 / (K.K_T * tv))
+        prob = np.clip(prob, 0.0, 1.0)
+        defect[carbon] = np.random.random(len(carbon)) < prob
+    return site, atom | (defect << 4), theta, phi, T_row
+
+
 def introduce_defects(state, atom_type, T=None, apply_to_state=False, voxel_size=5e-6):
     """defects.py:4-31 — Bernoulli defect mask on carbon sites (one global-stream draw each)."""
     L = state.shape[0]

@@ -63,6 +63,11 @@ class SweepResult(C.Structure):                     # cet_sweep_result
                 ("terminated", C.c_int32), ("overflow", C.c_int32), ("sites_refreshed", C.c_int64)]
 
 
+class InitDesc(C.Structure):                        # cet_init_desc
+    _fields_ = [("n_nuclei", C.c_int64), ("site", C.c_void_p), ("byte", C.c_void_p), ("theta", C.c_void_p),
+                ("phi", C.c_void_p), ("T_row", C.c_void_p)]
+
+
 class MetricsParams(C.Structure):                   # cet_metrics_params
     _fields_ = [("theta_threshold", C.c_double), ("ar_threshold", C.c_double), ("pct_pos", C.c_int64 * 4),
                 ("refresh", C.c_int32), ("carbon_id", C.c_int32), ("epoch", C.c_uint32), ("pad_", C.c_int32),
@@ -129,6 +134,7 @@ SIGNATURES = {
     "cet_grains_stats": [_VP, _I64, _VP, _VP, _VP, _VP],
     "cet_grains_download_labels": [_VP, _VP],
     "cet_grains_download_planes": [_VP, _I64, _I64, _VP],
+    "cet_init_group": [C.POINTER(_VP), _I32, C.POINTER(InitDesc), _I32],
     "cet_counts_group": [C.POINTER(_VP), _I32, C.POINTER(_I64)],
     "cet_metrics_group": [C.POINTER(_VP), _I32, C.POINTER(MetricsParams), C.POINTER(_VP), C.POINTER(_I64),
                           C.POINTER(MetricsResult)],
@@ -572,6 +578,32 @@ def _group_handles(fn, ctxs):
     if any(not isinstance(c, Context) for c in ctxs):
         raise TypeError(f"{fn}: ctxs must be Context objects")
     return (C.c_void_p * len(ctxs))(*[c._h.value for c in ctxs])
+
+
+def init_group(ctxs, nuclei, snapshot=False):
+    """The initial lattices of a group of whole-lattice Contexts of one L on one device, built on the device with one
+    copy and two launches.  nuclei[q] = (site, byte, theta, phi, T_row) as _host.initial_nuclei returns them: int64,
+    uint8, float64 and float64 arrays of one length and a float64 array of L.  Context q ends exactly as
+    ctxs[q].upload() of the dense arrays would leave it (followed, with snapshot=True, by ctxs[q].snapshot_state())."""
+    ctxs, nuclei = list(ctxs), list(nuclei)
+    n = len(ctxs)
+    if len(nuclei) != n:
+        raise ValueError(f"init_group: {len(nuclei)} nucleus sets for {n} contexts")
+    handles = _group_handles("init_group", ctxs)
+    dtypes = (np.int64, np.uint8, np.float64, np.float64, np.float64)
+    for q, (c, nu) in enumerate(zip(ctxs, nuclei)):
+        if len(nu) != 5:
+            raise ValueError(f"init_group: nuclei[{q}] must be (site, byte, theta, phi, T_row)")
+        for a, dt in zip(nu, dtypes):
+            if not isinstance(a, np.ndarray) or a.dtype != dt or a.ndim != 1 or not a.flags.c_contiguous:
+                raise TypeError(f"init_group: nuclei[{q}] needs 1-D C-contiguous arrays of "
+                                "int64, uint8, float64, float64, float64")
+        if len({len(a) for a in nu[:4]}) != 1:
+            raise ValueError(f"init_group: nuclei[{q}]: site, byte, theta and phi differ in length")
+        if len(nu[4]) != c.shape[2]:
+            raise ValueError(f"init_group: nuclei[{q}]: T_row has {len(nu[4])} values, the lattice needs {c.shape[2]}")
+    desc = (InitDesc * n)(*[InitDesc(len(nu[0]), *[a.ctypes.data for a in nu]) for nu in nuclei])
+    check(lib().cet_init_group(handles, n, desc, 1 if snapshot else 0), "cet_init_group")
 
 
 def counts_group(ctxs):

@@ -16,6 +16,8 @@
     run_gr_sweep                     config 5: independent lattices over a grid of (G, R), one per
                                      GPU (replicas only, no communication), one cet_map.csv and a tree
                                      the unmodified plot_cet.py reads (write_plot_cet_tree)
+    ensemble_stats                   mean, standard error and equiaxed fraction over the replicas of
+                                     each point of a map (run_gr_sweep / run_melt_pool_map, replicas=n)
 """
 from __future__ import annotations
 
@@ -24,7 +26,7 @@ import os
 
 import numpy as np
 
-from . import _lib
+from . import _host, _lib
 from . import defects as _defects
 from . import kmc_simulation as _ks
 from . import metrics as _metrics
@@ -116,10 +118,19 @@ def _slab_comm(world):
 
 def _upload_initial(ctx, L, n_seeds, temp, impurity_c, lattice, i_begin, i_end):
     """The run's initial lattice on the device: initialize_lattice + introduce_defects (NumPy's global stream,
-    seeded by the caller), or the given `lattice`."""
+    seeded with ctx.init_seed when the driver set one, else with initialize_lattice's default 42), or the given
+    `lattice`.  A context whose driver set ctx.init_nuclei to a list (the grouped driver) gets a generated lattice
+    appended there in sparse form instead (_host.initial_nuclei, the same draws); the driver then builds the
+    lattices of its whole group with one cetkmc.init_group call."""
+    init_seed = getattr(ctx, "init_seed", None)
+    if lattice is None and getattr(ctx, "init_nuclei", None) is not None:
+        ctx.init_nuclei.append(_host.initial_nuclei(L, n_seeds, temp, 42 if init_seed is None else init_seed,
+                                                    impurity_c))
+        return
     if lattice is None:
-        state, theta, phi, T, atom_type = _ks.initialize_lattice(lattice_size=L, n_seeds=n_seeds, T_sub=temp,
-                                                                 impurity_c=impurity_c)
+        state, theta, phi, T, atom_type = _ks.initialize_lattice(
+            lattice_size=L, n_seeds=n_seeds, T_sub=temp, impurity_c=impurity_c,
+            **({} if init_seed is None else {"random_seed": init_seed}))
         defects_mask, _ = _ks.introduce_defects(state, atom_type, T, apply_to_state=False)
     else:
         state, theta, phi, T, atom_type = lattice[:5]
@@ -164,7 +175,8 @@ def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_
 
 def _cadence_group(runs, last, every, philox_mask, seed):
     """_cadence for every case of a group at once (cetkmc.metrics_group, one launch per kernel for the group): the
-    defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  With NumPy's
+    defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  The Philox
+    stream is keyed by r["seed"] where a case has one, else by `seed`.  With NumPy's
     stream each case draws its mask from its own saved position (r["rng"]), in group order, as refresh_resident
     draws it."""
     ctxs = [r["ctx"] for r in runs]
@@ -178,11 +190,11 @@ def _cadence_group(runs, last, every, philox_mask, seed):
             r["rng"] = np.random.get_state()
     n_sites = int(np.prod(ctxs[0].owned_shape))
     params = []
-    for _r in runs:
+    for run in runs:
         p = _lib.MetricsParams()
         p.theta_threshold, p.ar_threshold = 0.5, constants.CET_AR_THRESHOLD
         p.pct_pos[:] = _metrics.percentile_positions(n_sites)
-        p.refresh, p.carbon_id, p.epoch, p.seed = int(refresh), _defects.CARBON_ID, last // every, seed
+        p.refresh, p.carbon_id, p.epoch, p.seed = int(refresh), _defects.CARBON_ID, last // every, run.get("seed", seed)
         p.prob_base, p.e_mig, p.kT, p.T_default = constants.DEFECT_PROB_BASE, _defects.E_MIGRATION, constants.K_T, constants.T_SUB
         params.append(p)
     for r, res in zip(runs, _lib.metrics_group(ctxs, params, draws)):
@@ -196,7 +208,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
                        output_prefix="cet_sublattice", metrics_every=None, events_per_sweep=None, p_max=0.1,
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
                        checkpoint_every=0, resume_from=None, lattice=None, verbose=True, rank=0, world=1,
-                       mask_stream="numpy"):
+                       mask_stream="numpy", init_seed=None):
     """run_kmc's large-lattice sibling.  Same set-up (initialize_lattice + introduce_defects with the
     run's seed), same cadence and CSV; the steps are synchronous-sublattice sweeps (csrc/sweep.cu), so
     `Step` counts sweeps and `Time` is the accumulated sweep interval.
@@ -206,6 +218,8 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
            beam_radius=m, absorptivity=) -> thermal_solver.update_temperature with the moving source.
     lattice: optional (state, theta, phi, T, atom_type[, defects]) to start from instead of
            initialize_lattice.  Returns (state, atom_type, total_time, theta, phi) like run_kmc.
+    init_seed: the random_seed of initialize_lattice (None: its default, 42).  `seed` keys the sweeps and the
+           defect-mask stream; init_seed picks the initial nuclei.
     world > 1: the lattice is split into z-slabs, one per rank / GPU (launch every rank with the same
            arguments plus its rank; torch.distributed.run provides the rendezvous).  The trajectory and
            the CSV do not depend on the number of slabs.  Rank 0 writes the CSV; every rank returns its
@@ -236,6 +250,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     all_gather = None
     i_begin, i_end = _ks.slab_bounds(L, world, rank)
     ctx = _lib.Context(L=L, device=device, i_begin=i_begin, i_end=i_end, halo=_ks.SWEEP_HALO if world > 1 else 0)
+    ctx.init_seed = init_seed
     try:
         ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
         sweep0, total_time, nucleation_count, cet_detected, rows = 0, 0.0, 0, False, []
@@ -318,7 +333,7 @@ def gr_partition(n_cases, rank, world, devices, batch=None):
 
 
 def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20, defect_fraction=0.0,
-                 output_root="gr_sweep", rank=None, world=None, devices=None, batch=None, **kw):
+                 output_root="gr_sweep", rank=None, world=None, devices=None, batch=None, replicas=None, **kw):
     """SURVEY §8d config 5: one independent lattice per (T_sub, NU_DEP) grid point — T_sub sets the
     thermal gradient G = (T_MELT - T_sub) / (L dx), NU_DEP the growth velocity R (kmc_simulation.py:
     236-239).  Replicas only: case q runs on rank q % world (torchrun: RANK / WORLD_SIZE / LOCAL_RANK)
@@ -328,48 +343,134 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
     EquiaxedFraction, GrainCount, CET_Class, ...).
     batch=k: the cases of one device advance in groups of up to k lattices, one kernel launch per group
     and kernel (cetkmc.sweep_run_group) instead of one per lattice; every output file is the same as
-    with batch=None.  Not with `laser`, `checkpoint_every`, `resume_from` or `lattice`."""
+    with batch=None.  Not with `laser`, `checkpoint_every`, `resume_from` or `lattice`.
+    replicas=n: every case runs n times, replica r as run_cet_sublattice(seed=seed + r, init_seed=42 + r) writing
+    outputs/<prefix>/metrics.csv for r = 0 and outputs/<prefix>/rep<r>/metrics.csv for r >= 1; the (case, replica)
+    lattices are partitioned and grouped as cases are.  cet_map_rank<r>.csv and the plot_cet tree come from
+    replica 0, so they equal those of a run without replicas; each rank also writes cet_map_replicas_rank<r>.csv
+    (one row per (case, replica), the map's columns).  Returns (map rows, ensemble_stats rows; None when
+    world > 1) instead of the map rows.  Not with `checkpoint_every`, `resume_from` or `lattice`."""
     rank = int(os.environ.get("RANK", 0)) if rank is None else rank
     world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
     local = int(os.environ.get("LOCAL_RANK", 0))
     devices = [local] if devices is None else list(devices)
+    n_rep = _check_replicas("run_gr_sweep", replicas, kw)
     if batch is not None:
         bad = [k for k in ("laser", "checkpoint_every", "resume_from", "lattice") if kw.get(k)]
         if bad:
             raise ValueError(f"run_gr_sweep: batch does not take {', '.join(bad)}")
     cases = [(float(t), float(r)) for t in temps for r in nu_deps]
-    out_dir = f"outputs/{output_root}"
-    os.makedirs(out_dir, exist_ok=True)
+    os.makedirs(f"outputs/{output_root}", exist_ok=True)
     prefix = [f"{output_root}/T{temp:g}_R{nu_dep:g}" for temp, nu_dep in cases]
-    for device, qs in gr_partition(len(cases), rank, world, devices, batch):
+    lats = _map_lattices(prefix, n_rep)
+    parts = gr_partition(len(lats), rank, world, devices, batch)
+    for device, ls in parts:
         if batch is None:
-            q = qs[0]
+            q, r, p = lats[ls[0]]
             run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=cases[q][0], nu_dep=cases[q][1], impurity_c=impurity_c,
-                               n_seeds=n_seeds, defect_fraction=defect_fraction, output_prefix=prefix[q],
-                               device=device, verbose=False, **kw)
+                               n_seeds=n_seeds, defect_fraction=defect_fraction, output_prefix=p,
+                               device=device, verbose=False, **_replica_kw(kw, replicas, r))
         else:
-            _run_cases_grouped([(prefix[q],) + cases[q] for q in qs], L=L, n_sweeps=n_sweeps, impurity_c=impurity_c,
-                               n_seeds=n_seeds, defect_fraction=defect_fraction, device=device, **kw)
-    import csv
-    rows = []
-    for q in (q for _d, qs in gr_partition(len(cases), rank, world, devices, batch) for q in qs):
+            _run_cases_grouped([(lats[l][2],) + cases[lats[l][0]] for l in ls], L=L, n_sweeps=n_sweeps,
+                               impurity_c=impurity_c, n_seeds=n_seeds, defect_fraction=defect_fraction, device=device,
+                               replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
+
+    def case_row(q):
         temp, nu_dep = cases[q]
-        with open(f"outputs/{prefix[q]}/metrics.csv") as fh:
-            last = list(csv.DictReader(fh))[-1]
         G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
-        rows.append({"case": q, "T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R, "G_over_R": G / R if R > 0 else np.inf,
-                     **{k: last[k] for k in ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize",
-                                             "NucleationCount", "CET_Class", "CET_Detected")}})
-    rows.sort(key=lambda r: r["case"])
-    _write_rows(rows, os.path.join(out_dir, f"cet_map_rank{rank}.csv"))
-    write_plot_cet_tree([(r["case"], f"outputs/{output_root}/T{r['T_sub']:g}_R{r['NU_DEP']:g}/metrics.csv") for r in rows],
+        return {"T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R, "G_over_R": G / R if R > 0 else np.inf}
+    return _map_outputs(output_root, "cet_map", lats, [l for _d, ls in parts for l in ls], case_row,
+                        ("T_sub", "NU_DEP"), replicas, rank, world)
+
+
+_MAP_FINAL = ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount",
+              "CET_Class", "CET_Detected")
+ENSEMBLE_COLUMNS = ("AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount", "Step")
+
+
+def _check_replicas(fn, replicas, kw):
+    """Replicas per case of a map driver (1 for replicas=None), refusing what a replica run does not take."""
+    if replicas is None:
+        return 1
+    if int(replicas) < 1:
+        raise ValueError(f"{fn}: replicas must be >= 1, got {replicas}")
+    bad = [k for k in ("lattice", "resume_from", "checkpoint_every") if kw.get(k)]
+    if bad:
+        raise ValueError(f"{fn}: replicas does not take {', '.join(bad)}")
+    return int(replicas)
+
+
+def _map_lattices(prefix, n_rep):
+    """The lattices of a map, case by case: (case, replica, output prefix).  Replica 0 of case q writes to prefix[q],
+    replica r >= 1 to <prefix[q]>/rep<r>."""
+    return [(q, r, p if r == 0 else f"{p}/rep{r}") for q, p in enumerate(prefix) for r in range(n_rep)]
+
+
+def _replica_kw(kw, replicas, r):
+    """run_cet_sublattice's keywords for replica r of a case: seed + r and init_seed = 42 + r (kw itself without
+    replicas)."""
+    if replicas is None:
+        return kw
+    seed = kw.get("seed")
+    return dict(kw, seed=(constants.RANDOM_SEED if seed is None else int(seed)) + r, init_seed=42 + r)
+
+
+def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world):
+    """The per-rank files of a map driver over the lattices `mine` (indices into `lats`) this rank ran:
+    <name>_rank<rank>.csv (case, case_row(case), the final row's _MAP_FINAL columns) and the plot_cet tree from
+    replica 0 of each case, and with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica).  Returns
+    the map rows; with replicas (map rows, ensemble_stats of the replica rows), the latter None when world > 1
+    (merge_* joins the ranks)."""
+    import csv
+    rows, rep_rows = [], []
+    for l in sorted(mine):
+        q, r, p = lats[l]
+        with open(f"outputs/{p}/metrics.csv") as fh:
+            last = list(csv.DictReader(fh))[-1]
+        row = {"case": q, **case_row(q), **{k: last[k] for k in _MAP_FINAL}}
+        rep_rows.append({"case": q, "replica": r, **{k: v for k, v in row.items() if k != "case"}})
+        if r == 0:
+            rows.append(row)
+    out_dir = f"outputs/{output_root}"
+    _write_rows(rows, os.path.join(out_dir, f"{name}_rank{rank}.csv"))
+    write_plot_cet_tree([(row["case"], f"outputs/{lats[l][2]}/metrics.csv")
+                         for row, l in zip(rows, sorted(l for l in mine if lats[l][1] == 0))],
                         os.path.join(out_dir, "plot_cet"))
-    return rows
+    if replicas is None:
+        return rows
+    _write_rows(rep_rows, os.path.join(out_dir, f"{name}_replicas_rank{rank}.csv"))
+    return rows, (ensemble_stats(rep_rows, axes) if world == 1 else None)
+
+
+def ensemble_stats(rows, axes):
+    """One row per case over the replica rows `rows` of a map (dicts with case, the axis columns `axes`, G, R,
+    G_over_R, ENSEMBLE_COLUMNS, CET_Class and CET_Detected; numbers, or the strings a CSV gives back), in case order:
+    case, the axes, G, R, G_over_R, replicas (n), <col>_mean and <col>_se for every column of ENSEMBLE_COLUMNS (the
+    standard error is the sample standard deviation, ddof=1, over sqrt(n); empty for n = 1), p_equiaxed (the
+    fraction of replicas whose final CET_Class is Equiaxed) with its binomial standard error sqrt(p (1 - p) / n)
+    as p_equiaxed_se, and p_cet_detected (the fraction with CET_Detected)."""
+    by_case = {}
+    for r in rows:
+        by_case.setdefault(int(r["case"]), []).append(r)
+    out = []
+    for case in sorted(by_case):
+        rs = by_case[case]
+        n = len(rs)
+        e = {"case": case, **{k: rs[0][k] for k in tuple(axes) + ("G", "R", "G_over_R")}, "replicas": n}
+        for col in ENSEMBLE_COLUMNS:
+            v = np.array([float(r[col]) for r in rs])
+            e[f"{col}_mean"] = float(np.mean(v))
+            e[f"{col}_se"] = float(np.std(v, ddof=1) / np.sqrt(n)) if n > 1 else ""
+        p = float(np.mean([r["CET_Class"] == "Equiaxed" for r in rs]))
+        e["p_equiaxed"], e["p_equiaxed_se"] = p, float(np.sqrt(p * (1.0 - p) / n))
+        e["p_cet_detected"] = float(np.mean([str(r["CET_Detected"]) == "True" for r in rs]))
+        out.append(e)
+    return out
 
 
 def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
                        events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy",
-                       lasers=None):
+                       lasers=None, replicas=None):
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
@@ -378,7 +479,10 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     lasers: None, or one laser dict per case (run_cet_sublattice(laser=...)): every `thermal_every` sweeps one
     cetkmc.thermal_full_group over the cases still running replaces their thermal_full + snapshot_state, and a case
     that terminates leaves the group after the block of sweeps it terminated in, with its row at that block's last
-    sweep, as the laser driver of run_cet_sublattice stops it."""
+    sweep, as the laser driver of run_cet_sublattice stops it.
+    replicas: None, or the replica number r of each case: the case then runs as run_cet_sublattice(seed=seed + r,
+    init_seed=42 + r).  The generated initial lattices of the group are built on the device by one cetkmc.init_group
+    call (_upload_initial)."""
     if mask_stream not in ("numpy", "philox"):
         raise ValueError("mask_stream must be 'numpy' or 'philox'")
     if lasers is not None and int(thermal_every) <= 0:
@@ -386,25 +490,35 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
     philox_mask = mask_stream == "philox"
+    reps = [0] * len(cases) if replicas is None else [int(r) for r in replicas]
     runs = []
     try:
         for q, (prefix, temp, nu_dep) in enumerate(cases):
-            np.random.seed(seed)
+            seed_q = seed + reps[q]
+            np.random.seed(seed_q)
             os.makedirs(f"outputs/{prefix}", exist_ok=True)
             ctx = _lib.Context(L=L, device=device)
-            r = dict(ctx=ctx, prefix=prefix, consts=_gr(L, temp, nu_dep), rows=[], total_time=0.0, nucleation_count=0,
-                     cet_detected=False, terminated=False)
+            ctx.init_seed = None if replicas is None else 42 + reps[q]
+            ctx.init_nuclei = []
+            r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], total_time=0.0,
+                     nucleation_count=0, cet_detected=False, terminated=False)
             runs.append(r)
             ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
             _upload_initial(ctx, L, n_seeds, temp, impurity_c, None, 0, L)
-            r["sp"], r["tp"] = _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction,
+            r["sp"], r["tp"] = _sweep_setup(L, seed_q, temp, events_per_sweep, p_max, defect_fraction,
                                             0 if lasers is not None else thermal_every)
             r["rng"] = np.random.get_state()
             if lasers is not None:
                 r["laser"] = lasers[q]
                 r["tfp"] = thermal_full_params(float(lasers[q].get("dt", _ks.THERMAL_DT)))
                 r["pos"] = [float(x) for x in lasers[q].get("start", (0.0, 0.0))]
-                ctx.snapshot_state()
+        gen = [r["ctx"] for r in runs if r["ctx"].init_nuclei]
+        if gen:
+            _lib.init_group(gen, [c.init_nuclei[0] for c in gen], snapshot=lasers is not None)
+        if lasers is not None:
+            for r in runs:
+                if not r["ctx"].init_nuclei:                         # uploaded dense: a given lattice
+                    r["ctx"].snapshot_state()
         sweep = 0
         active = runs
         while sweep < n_sweeps and active:
@@ -461,7 +575,7 @@ def _laser_step_group(runs, L):
 def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None, start=(0.0, 0.0), dt=None,
                       beam_radius=DEFAULT_BEAM_RADIUS, absorptivity=DEFAULT_ABSORPTIVITY, impurity_c=0.0, n_seeds=20,
                       defect_fraction=0.0, output_root="melt_pool_map", rank=None, world=None, devices=None,
-                      batch=None, **kw):
+                      batch=None, replicas=None, **kw):
     """A CET map over the two quantities of the moving melt pool a user sets: beam power (W) and scan speed (voxels
     per thermal step along axis 1).  Case q of powers x speeds (in that order) is run_cet_sublattice(laser=dict(
     power=P, speed=V, start=start, dt=dt, beam_radius=..., absorptivity=...), output_prefix=
@@ -472,11 +586,18 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     CET_Detected) and adds its cases to the plot_cet tree; merge_melt_pool_map() joins the rank files.
     batch=k: the cases of one device advance in groups of up to k lattices (cetkmc.sweep_run_group for the sweeps,
     cetkmc.thermal_full_group for the laser steps); every output file is the same as with batch=None.  Not with
-    `checkpoint_every`, `resume_from` or `lattice`."""
+    `checkpoint_every`, `resume_from` or `lattice`.
+    replicas=n: every case runs n times, replica r as run_cet_sublattice(seed=seed + r, init_seed=42 + r) writing
+    outputs/<prefix>/metrics.csv for r = 0 and outputs/<prefix>/rep<r>/metrics.csv for r >= 1; the (case, replica)
+    lattices are partitioned and grouped as cases are.  The map file and the plot_cet tree come from replica 0, so
+    they equal those of a run without replicas; each rank also writes melt_pool_map_replicas_rank<r>.csv (one row
+    per (case, replica), the map's columns).  Returns (map rows, ensemble_stats rows; None when world > 1).
+    Not with `checkpoint_every`, `resume_from` or `lattice`."""
     rank = int(os.environ.get("RANK", 0)) if rank is None else rank
     world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
     local = int(os.environ.get("LOCAL_RANK", 0))
     devices = [local] if devices is None else list(devices)
+    n_rep = _check_replicas("run_melt_pool_map", replicas, kw)
     powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
     if not powers or not speeds:
         raise ValueError("run_melt_pool_map: needs at least one power and one speed")
@@ -493,33 +614,27 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     lasers = [dict(power=p, speed=v, start=tuple(start), dt=dt, beam_radius=beam_radius, absorptivity=absorptivity)
               for p, v in cases]
     prefix = [f"{output_root}/P{p:g}_V{v:g}" for p, v in cases]
-    out_dir = f"outputs/{output_root}"
-    os.makedirs(out_dir, exist_ok=True)
-    parts = gr_partition(len(cases), rank, world, devices, batch)
-    for device, qs in parts:
+    os.makedirs(f"outputs/{output_root}", exist_ok=True)
+    lats = _map_lattices(prefix, n_rep)
+    parts = gr_partition(len(lats), rank, world, devices, batch)
+    for device, ls in parts:
         if batch is None:
-            q = qs[0]
+            q, r, p = lats[ls[0]]
             run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=temp, nu_dep=nu_dep, impurity_c=impurity_c, n_seeds=n_seeds,
-                               defect_fraction=defect_fraction, output_prefix=prefix[q], laser=lasers[q], device=device,
-                               verbose=False, **kw)
+                               defect_fraction=defect_fraction, output_prefix=p, laser=lasers[q], device=device,
+                               verbose=False, **_replica_kw(kw, replicas, r))
         else:
-            _run_cases_grouped([(prefix[q], temp, nu_dep) for q in qs], L=L, n_sweeps=n_sweeps, impurity_c=impurity_c,
+            _run_cases_grouped([(lats[l][2], temp, nu_dep) for l in ls], L=L, n_sweeps=n_sweeps, impurity_c=impurity_c,
                                n_seeds=n_seeds, defect_fraction=defect_fraction, device=device,
-                               lasers=[lasers[q] for q in qs], **kw)
-    import csv
+                               lasers=[lasers[lats[l][0]] for l in ls],
+                               replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
     G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
-    rows = []
-    for q in sorted(q for _d, qs in parts for q in qs):
-        with open(f"outputs/{prefix[q]}/metrics.csv") as fh:
-            last = list(csv.DictReader(fh))[-1]
-        rows.append({"case": q, "power": cases[q][0], "speed": cases[q][1], "T_sub": temp, "NU_DEP": nu_dep, "G": G,
-                     "R": R, "G_over_R": G / R if R > 0 else np.inf,
-                     **{k: last[k] for k in ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize",
-                                             "NucleationCount", "CET_Class", "CET_Detected")}})
-    _write_rows(rows, os.path.join(out_dir, f"melt_pool_map_rank{rank}.csv"))
-    write_plot_cet_tree([(r["case"], f"outputs/{prefix[r['case']]}/metrics.csv") for r in rows],
-                        os.path.join(out_dir, "plot_cet"))
-    return rows
+
+    def case_row(q):
+        return {"power": cases[q][0], "speed": cases[q][1], "T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R,
+                "G_over_R": G / R if R > 0 else np.inf}
+    return _map_outputs(output_root, "melt_pool_map", lats, [l for _d, ls in parts for l in ls], case_row,
+                        ("power", "speed", "T_sub", "NU_DEP"), replicas, rank, world)
 
 
 def write_plot_cet_tree(cases, root):
@@ -549,23 +664,34 @@ def _write_rows(rows, path):
 
 
 def _merge_rank_files(output_root, name):
-    """Join outputs/<output_root>/<name>_rank*.csv into outputs/<output_root>/<name>.csv (sorted by case)."""
+    """Join outputs/<output_root>/<name>_rank*.csv into outputs/<output_root>/<name>.csv (sorted by case and
+    replica)."""
     import csv
     import glob
     rows = []
     for p in sorted(glob.glob(f"outputs/{output_root}/{name}_rank*.csv")):
         with open(p) as fh:
             rows += list(csv.DictReader(fh))
-    rows.sort(key=lambda r: int(r["case"]))
+    rows.sort(key=lambda r: (int(r["case"]), int(r.get("replica", 0))))
     _write_rows(rows, f"outputs/{output_root}/{name}.csv")
     return rows
 
 
+def _merge_map(output_root, name, axes):
+    rows = _merge_rank_files(output_root, name)
+    reps = _merge_rank_files(output_root, f"{name}_replicas")
+    if reps:
+        _write_rows(ensemble_stats(reps, axes), f"outputs/{output_root}/{name}_ensemble.csv")
+    return rows
+
+
 def merge_cet_map(output_root="gr_sweep"):
-    """Join the per-rank files of run_gr_sweep into outputs/<output_root>/cet_map.csv (sorted by case)."""
-    return _merge_rank_files(output_root, "cet_map")
+    """Join the per-rank files of run_gr_sweep into outputs/<output_root>/cet_map.csv (sorted by case); after a run
+    with replicas also cet_map_replicas.csv and cet_map_ensemble.csv (ensemble_stats, one row per case)."""
+    return _merge_map(output_root, "cet_map", ("T_sub", "NU_DEP"))
 
 
 def merge_melt_pool_map(output_root="melt_pool_map"):
-    """Join the per-rank files of run_melt_pool_map into outputs/<output_root>/melt_pool_map.csv (sorted by case)."""
-    return _merge_rank_files(output_root, "melt_pool_map")
+    """Join the per-rank files of run_melt_pool_map into outputs/<output_root>/melt_pool_map.csv (sorted by case);
+    after a run with replicas also melt_pool_map_replicas.csv and melt_pool_map_ensemble.csv (ensemble_stats)."""
+    return _merge_map(output_root, "melt_pool_map", ("power", "speed", "T_sub", "NU_DEP"))

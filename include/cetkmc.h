@@ -259,6 +259,26 @@ int cet_grains_stats(cet_ctx *ctx, int64_t cap, int32_t *root, int32_t *size, in
 /* Label volume: root site index per occupied site, -1 for empty sites (owned planes). */
 int cet_grains_download_labels(cet_ctx *ctx, int32_t *labels);
 
+/* ---- initial lattices of a group (lattice_init.py:10-59 + defects.py:4-31, in sparse form) ----
+ * One context's initial lattice: n_nuclei nuclei, each at a C-order flat site of the k = 0 plane with its voxel byte
+ * (state 1..3 | defect 0..1 << 4), theta and phi; every other site is empty with theta = phi = 0; T[i, j, k] =
+ * T_row[k].  Host pointers, borrowed for the call. */
+typedef struct cet_init_desc {
+    int64_t n_nuclei;
+    const int64_t *site;
+    const uint8_t *byte;
+    const double *theta, *phi;
+    const double *T_row;          /* L values */
+} cet_init_desc;
+/* Context q ends exactly as cet_upload(ctxs[q], state, theta, phi, T, defects) of the dense arrays of d[q] would
+ * leave it, followed, when snapshot != 0, by cet_snapshot_state(ctxs[q]).  The contexts must be distinct
+ * whole-lattice contexts (no slabs) of one cubic L on one device; 1 <= n_ctx <= 64; no two nuclei of a context share
+ * a site.  Everything is checked before anything is copied or launched, so a rejected call leaves every context as it
+ * was.  The work is ordered on the stream of ctxs[0] after the work already queued on every context's stream: one
+ * H2D copy of a packed table for the group, one fill launch over every site of the group, one scatter launch of the
+ * nuclei (none when the group has no nuclei), one host synchronisation. */
+int cet_init_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_init_desc *d, int32_t snapshot);
+
 /* ---- grouped metrics cadence (kmc_simulation.py:335-378 for many lattices at once) ----
  * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device; 1 <= n_ctx <= 64.
  * The work is ordered on the stream of ctxs[0] after the work already queued on every context's stream, each

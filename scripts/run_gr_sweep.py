@@ -2,12 +2,15 @@
 GPUs of one box, producing cet_map.csv and the tree the reference's plot_cet.py reads.
 
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29541 \
-        scripts/run_gr_sweep.py [--L 64] [--sweeps 400] [--out gr_sweep] [--batch 16]
+        scripts/run_gr_sweep.py [--L 64] [--sweeps 400] [--out gr_sweep] [--batch 16] [--replicas 4]
 
 --batch k: the cases of a GPU advance in groups of up to k lattices (one kernel launch per group and kernel);
 the outputs are the same as without it.
+--replicas n: every case runs n times (replica r with seed + r and initial-lattice seed 42 + r); rank 0 also writes
+cet_map_ensemble.csv (mean, standard error and equiaxed fraction over the replicas of each case) and prints it.
 """
 import argparse
+import csv
 import json
 import os
 import sys
@@ -26,13 +29,14 @@ def main():
     ap.add_argument("--sweeps", type=int, default=401)
     ap.add_argument("--out", default="gr_sweep")
     ap.add_argument("--batch", type=int, default=None)
+    ap.add_argument("--replicas", type=int, default=None)
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     temps = [2600.0, 2800.0, 3000.0, 3200.0]                      # T_sub -> G = (T_MELT - T_sub) / (L dx)
     nu_deps = [1e12, 5e12, 2e13, 1e14]                            # NU_DEP -> R
     t0 = time.perf_counter()
     rows = campaign.run_gr_sweep(temps, nu_deps, L=args.L, n_sweeps=args.sweeps, n_seeds=20, defect_fraction=3e-3,
-                                 impurity_c=0.1, output_root=args.out, metrics_every=100, batch=args.batch)
+                                 impurity_c=0.1, output_root=args.out, metrics_every=100, batch=args.batch, replicas=args.replicas)
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -42,13 +46,17 @@ def main():
     if rank == 0:
         merged = campaign.merge_cet_map(args.out)
         wall = time.perf_counter() - t0
-        sites = len(temps) * len(nu_deps) * args.L ** 3 * args.sweeps
-        print(json.dumps({"cases": len(merged), "world": world, "L": args.L, "sweeps": args.sweeps, "batch": args.batch, "wall_s": wall,
+        sites = len(temps) * len(nu_deps) * (args.replicas or 1) * args.L ** 3 * args.sweeps
+        print(json.dumps({"cases": len(merged), "world": world, "L": args.L, "sweeps": args.sweeps, "batch": args.batch, "replicas": args.replicas, "wall_s": wall,
                           "rank0_s": dt, "site_updates_per_s": sites / wall,
                           "classes": sorted(set(r["CET_Class"] for r in merged))}))
         for r in merged:
             print(f"case {int(r['case']):2d} T_sub {float(r['T_sub']):6.0f} NU_DEP {float(r['NU_DEP']):8.1e} G/R {float(r['G_over_R']):9.3e} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} {r['CET_Class']}")
+        if args.replicas is not None:
+            with open(f"outputs/{args.out}/cet_map_ensemble.csv") as fh:
+                for e in csv.DictReader(fh):
+                    print(json.dumps(e))
     if world > 1:
         dist.destroy_process_group()
 

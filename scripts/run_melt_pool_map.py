@@ -2,12 +2,15 @@
 one box, producing melt_pool_map.csv and the tree the reference's plot_cet.py reads.
 
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29542 \
-        scripts/run_melt_pool_map.py [--L 64] [--sweeps 401] [--out melt_pool_map] [--batch 16]
+        scripts/run_melt_pool_map.py [--L 64] [--sweeps 401] [--out melt_pool_map] [--batch 16] [--replicas 4]
 
 --batch k: the cases of a GPU advance in groups of up to k lattices (one kernel launch per group and kernel for the
 sweeps and for the laser step); the outputs are the same as without it.
+--replicas n: every case runs n times (replica r with seed + r and initial-lattice seed 42 + r); rank 0 also writes
+melt_pool_map_ensemble.csv (mean, standard error and equiaxed fraction over the replicas of each case) and prints it.
 """
 import argparse
+import csv
 import json
 import os
 import sys
@@ -25,6 +28,7 @@ def main():
     ap.add_argument("--sweeps", type=int, default=401)
     ap.add_argument("--out", default="melt_pool_map")
     ap.add_argument("--batch", type=int, default=None)
+    ap.add_argument("--replicas", type=int, default=None)
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     powers = [100.0, 200.0, 300.0, 400.0]                         # W
@@ -32,7 +36,7 @@ def main():
     t0 = time.perf_counter()
     campaign.run_melt_pool_map(powers, speeds, L=args.L, n_sweeps=args.sweeps, start=(args.L / 2, 0.0),
                                n_seeds=20, defect_fraction=3e-3, impurity_c=0.1, output_root=args.out,
-                               metrics_every=100, batch=args.batch)
+                               metrics_every=100, batch=args.batch, replicas=args.replicas)
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -42,14 +46,18 @@ def main():
     if rank == 0:
         merged = campaign.merge_melt_pool_map(args.out)
         wall = time.perf_counter() - t0
-        sites = len(powers) * len(speeds) * args.L ** 3 * args.sweeps
-        print(json.dumps({"cases": len(merged), "world": world, "L": args.L, "sweeps": args.sweeps, "batch": args.batch,
+        sites = len(powers) * len(speeds) * (args.replicas or 1) * args.L ** 3 * args.sweeps
+        print(json.dumps({"cases": len(merged), "world": world, "L": args.L, "sweeps": args.sweeps, "batch": args.batch, "replicas": args.replicas,
                           "wall_s": wall, "rank0_s": dt, "site_updates_per_s": sites / wall,
                           "classes": sorted(set(r["CET_Class"] for r in merged))}))
         for r in merged:
             print(f"case {int(r['case']):2d} P {float(r['power']):6.1f} W V {float(r['speed']):5.2f} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} "
                   f"step {r['Step']} {r['CET_Class']}")
+        if args.replicas is not None:
+            with open(f"outputs/{args.out}/melt_pool_map_ensemble.csv") as fh:
+                for e in csv.DictReader(fh):
+                    print(json.dumps(e))
     if world > 1:
         dist.destroy_process_group()
 

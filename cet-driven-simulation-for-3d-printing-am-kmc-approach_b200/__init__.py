@@ -10,4 +10,4 @@ Import the package as `import cetkmc` (alias module at the repository root).
 __version__ = "0.1.0"
 
 from . import _lib  # noqa: F401  (ctypes binding; the shared library is loaded on first use)
-from ._lib import Context, build, counts_group, device_count, init_group, metrics_group, sweep_run_group, thermal_full_group  # noqa: F401
+from ._lib import Context, build, counts_group, device_count, grain_profile_group, init_group, metrics_group, sweep_run_group, thermal_full_group  # noqa: F401

@@ -138,6 +138,7 @@ SIGNATURES = {
     "cet_counts_group": [C.POINTER(_VP), _I32, C.POINTER(_I64)],
     "cet_metrics_group": [C.POINTER(_VP), _I32, C.POINTER(MetricsParams), C.POINTER(_VP), C.POINTER(_I64),
                           C.POINTER(MetricsResult)],
+    "cet_grain_profile_group": [C.POINTER(_VP), _I32, _I32, _F64, C.POINTER(_I64)],
     "cet_debug_nst_mismatches": [_VP, C.POINTER(_I64)],
     "cet_debug_flags": [_VP, C.c_int],
     "cet_profile_enable": [_VP, C.c_int],
@@ -648,6 +649,30 @@ def metrics_group(ctxs, params, draws=None):
         d["counts"] = np.array(list(r.counts), np.int64)
         d["pct_index"] = np.array(list(r.pct_index), np.int64)
         out.append(d)
+    return out
+
+
+PROFILE_COLUMNS = ("Solid", "EquiaxedSolid", "GrainsSpanning", "EquiaxedGrainsSpanning")    # cet_grain_profile_group's f
+
+
+def grain_profile_group(ctxs, axis, ar_threshold):
+    """Per-plane grain profile of the last grain labelling (Context.grains(), metrics_group) of every context of `ctxs`
+    (whole-lattice Contexts of one L on one device), along `axis` (0, 1 or 2), with five launches and one copy for the
+    group.  Returns an (n, 4, L) int64 array: for context q and plane z, [q, 0, z] occupied sites, [q, 1, z] of those
+    the sites of grains with aspect ratio < ar_threshold, [q, 2, z] grains whose bounding box along `axis` contains z,
+    [q, 3, z] of those the grains with aspect ratio < ar_threshold (PROFILE_COLUMNS).  The call does not relabel and
+    changes nothing the next metrics row or sweep reads."""
+    ctxs = list(ctxs)
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"grain_profile_group: axis must be 0, 1 or 2, got {axis!r}")
+    thr = float(ar_threshold)
+    if not np.isfinite(thr):
+        raise ValueError(f"grain_profile_group: ar_threshold must be finite, got {ar_threshold!r}")
+    handles = _group_handles("grain_profile_group", ctxs)
+    L = ctxs[0].shape[2] if ctxs else 0
+    out = np.zeros((len(ctxs), 4, L), np.int64)
+    check(lib().cet_grain_profile_group(handles, len(ctxs), int(axis), thr, out.ctypes.data_as(C.POINTER(C.c_int64))),
+          "cet_grain_profile_group")
     return out
 
 

@@ -18,6 +18,10 @@
                                      the unmodified plot_cet.py reads (write_plot_cet_tree)
     ensemble_stats                   mean, standard error and equiaxed fraction over the replicas of
                                      each point of a map (run_gr_sweep / run_melt_pool_map, replicas=n)
+    profile_axis=0|1|2               (run_cet_sublattice and the map drivers) per-plane grain profiles of
+                                     every metrics row in outputs/<prefix>/cet_profile.csv
+                                     (cetkmc.grain_profile_group), and per map the CET height of every
+                                     lattice (metrics.cet_profile_summary) in <map>_profile.csv
 """
 from __future__ import annotations
 
@@ -173,12 +177,13 @@ def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_
                             all_gather=all_gather)
 
 
-def _cadence_group(runs, last, every, philox_mask, seed):
+def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None):
     """_cadence for every case of a group at once (cetkmc.metrics_group, one launch per kernel for the group): the
     defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  The Philox
     stream is keyed by r["seed"] where a case has one, else by `seed`.  With NumPy's
     stream each case draws its mask from its own saved position (r["rng"]), in group order, as refresh_resident
-    draws it."""
+    draws it.  profile_axis: one cetkmc.grain_profile_group call over the labelling the rows used appends each
+    case's (step, profile) to r["profiles"]."""
     ctxs = [r["ctx"] for r in runs]
     refresh = last % every == 0
     draws = None
@@ -202,13 +207,56 @@ def _cadence_group(runs, last, every, philox_mask, seed):
         row, r["cet_detected"] = _ks._row_from_metrics(last, r["total_time"], r["nucleation_count"], r["cet_detected"],
                                                        r["consts"], res["counts"], m, n_sites, verbose=False)
         r["rows"].append(row)
+    if profile_axis is not None:
+        for r, prof in zip(runs, _lib.grain_profile_group(ctxs, profile_axis, constants.CET_AR_THRESHOLD)):
+            r["profiles"].append((last, prof))
+
+
+PROFILE_CSV = "cet_profile.csv"
+
+
+def _check_profile_axis(fn, profile_axis, world=1, checkpoint_every=0, resume_from=None):
+    """Refuse what a run with per-plane grain profiles does not take: an axis outside {0, 1, 2}, a lattice split into
+    slabs (their labels are slab-local) and checkpoints (they do not carry the profile history)."""
+    if profile_axis is None:
+        return
+    if isinstance(profile_axis, bool) or not isinstance(profile_axis, (int, np.integer)) or int(profile_axis) not in (0, 1, 2):
+        raise ValueError(f"{fn}: profile_axis must be None, 0, 1 or 2, got {profile_axis!r}")
+    if world > 1:
+        raise ValueError(f"{fn}: profile_axis needs a whole lattice on one GPU (world = 1)")
+    if checkpoint_every or resume_from:
+        raise ValueError(f"{fn}: profile_axis does not take checkpoint_every or resume_from")
+
+
+def _write_profile_csv(profiles, output_dir):
+    """outputs/<prefix>/cet_profile.csv: one row per (metrics row, plane) of the (step, (4, L) profile) pairs."""
+    import csv
+    if not profiles:
+        return
+    with open(os.path.join(output_dir, PROFILE_CSV), "w", newline="") as fh:
+        w = csv.writer(fh)
+        w.writerow(("Step", "Plane") + _lib.PROFILE_COLUMNS)
+        for step, prof in profiles:
+            for z in range(prof.shape[1]):
+                w.writerow([int(step), z] + [int(v) for v in prof[:, z]])
+
+
+def read_profile_csv(path):
+    """The last metrics row's profile of a cet_profile.csv: (step, (4, L) int64 array)."""
+    import csv
+    with open(path) as fh:
+        rows = list(csv.DictReader(fh))
+    step = rows[-1]["Step"]
+    last = [r for r in rows if r["Step"] == step]
+    prof = np.array([[int(r[c]) for r in last] for c in _lib.PROFILE_COLUMNS], np.int64)
+    return int(step), prof
 
 
 def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_seeds=5, impurity_c=0.0,
                        output_prefix="cet_sublattice", metrics_every=None, events_per_sweep=None, p_max=0.1,
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
                        checkpoint_every=0, resume_from=None, lattice=None, verbose=True, rank=0, world=1,
-                       mask_stream="numpy", init_seed=None):
+                       mask_stream="numpy", init_seed=None, profile_axis=None):
     """run_kmc's large-lattice sibling.  Same set-up (initialize_lattice + introduce_defects with the
     run's seed), same cadence and CSV; the steps are synchronous-sublattice sweeps (csrc/sweep.cu), so
     `Step` counts sweeps and `Time` is the accumulated sweep interval.
@@ -220,6 +268,11 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
            initialize_lattice.  Returns (state, atom_type, total_time, theta, phi) like run_kmc.
     init_seed: the random_seed of initialize_lattice (None: its default, 42).  `seed` keys the sweeps and the
            defect-mask stream; init_seed picks the initial nuclei.
+    profile_axis: None, or 0, 1 or 2: every metrics row also takes the per-plane grain profile of the labelling it
+           used along that axis (cetkmc.grain_profile_group), written to outputs/<prefix>/cet_profile.csv with the
+           columns Step, Plane, Solid, EquiaxedSolid, GrainsSpanning, EquiaxedGrainsSpanning, one row per (metrics
+           row, plane).  Every other output is the same as without it.  Not with world > 1, checkpoint_every or
+           resume_from.
     world > 1: the lattice is split into z-slabs, one per rank / GPU (launch every rank with the same
            arguments plus its rank; torch.distributed.run provides the rendezvous).  The trajectory and
            the CSV do not depend on the number of slabs.  Rank 0 writes the CSV; every rank returns its
@@ -237,6 +290,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     nu_dep = constants.NU_DEP if nu_dep is None else nu_dep
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
+    _check_profile_axis("run_cet_sublattice", profile_axis, world, checkpoint_every, resume_from)
     np.random.seed(seed)                                    # a resumed run restores the stream position below
     output_dir = f"outputs/{output_prefix}"
     os.makedirs(output_dir, exist_ok=True)
@@ -253,7 +307,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     ctx.init_seed = init_seed
     try:
         ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
-        sweep0, total_time, nucleation_count, cet_detected, rows = 0, 0.0, 0, False, []
+        sweep0, total_time, nucleation_count, cet_detected, rows, profiles = 0, 0.0, 0, False, [], []
         if resume_from:
             meta = resume(ctx, resume_from)
             sweep0, total_time = int(meta.get("sweep", 0)), float(meta.get("time", 0.0))
@@ -304,12 +358,15 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             row, cet_detected = _cadence(ctx, sweep - 1, every, philox_mask, seed, world, total_time, nucleation_count,
                                          cet_detected, consts, verbose=verbose and rank == 0, all_gather=all_gather)
             rows.append(row)
+            if profile_axis is not None:
+                profiles.append((sweep - 1, _lib.grain_profile_group([ctx], profile_axis, constants.CET_AR_THRESHOLD)[0]))
             if checkpoint_every and (len(rows) % checkpoint_every == 0):
                 checkpoint(ctx, os.path.join(output_dir, "checkpoint"), sweep=sweep, time=total_time,
                            nucleation_count=nucleation_count, cet_detected=cet_detected,
                            rows=[{k: (v if not isinstance(v, (np.generic,)) else v.item()) for k, v in r.items()} for r in rows])
         if rank == 0:
             _ks._write_csv(rows, output_dir)
+            _write_profile_csv(profiles, output_dir)
         f = ctx.download(state=True, atom_type=True, theta=True, phi=True)
     finally:
         ctx.close()
@@ -349,12 +406,15 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
     lattices are partitioned and grouped as cases are.  cet_map_rank<r>.csv and the plot_cet tree come from
     replica 0, so they equal those of a run without replicas; each rank also writes cet_map_replicas_rank<r>.csv
     (one row per (case, replica), the map's columns).  Returns (map rows, ensemble_stats rows; None when
-    world > 1) instead of the map rows.  Not with `checkpoint_every`, `resume_from` or `lattice`."""
+    world > 1) instead of the map rows.  Not with `checkpoint_every`, `resume_from` or `lattice`.
+    profile_axis=a (through **kw): every case writes outputs/<prefix>/cet_profile.csv (run_cet_sublattice), and each
+    rank writes cet_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it."""
     rank = int(os.environ.get("RANK", 0)) if rank is None else rank
     world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
     local = int(os.environ.get("LOCAL_RANK", 0))
     devices = [local] if devices is None else list(devices)
     n_rep = _check_replicas("run_gr_sweep", replicas, kw)
+    _check_profile_axis("run_gr_sweep", kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     if batch is not None:
         bad = [k for k in ("laser", "checkpoint_every", "resume_from", "lattice") if kw.get(k)]
         if bad:
@@ -380,7 +440,7 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
         G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
         return {"T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R, "G_over_R": G / R if R > 0 else np.inf}
     return _map_outputs(output_root, "cet_map", lats, [l for _d, ls in parts for l in ls], case_row,
-                        ("T_sub", "NU_DEP"), replicas, rank, world)
+                        ("T_sub", "NU_DEP"), replicas, rank, world, kw.get("profile_axis"))
 
 
 _MAP_FINAL = ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount",
@@ -415,12 +475,12 @@ def _replica_kw(kw, replicas, r):
     return dict(kw, seed=(constants.RANDOM_SEED if seed is None else int(seed)) + r, init_seed=42 + r)
 
 
-def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world):
+def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world, profile_axis=None):
     """The per-rank files of a map driver over the lattices `mine` (indices into `lats`) this rank ran:
     <name>_rank<rank>.csv (case, case_row(case), the final row's _MAP_FINAL columns) and the plot_cet tree from
-    replica 0 of each case, and with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica).  Returns
-    the map rows; with replicas (map rows, ensemble_stats of the replica rows), the latter None when world > 1
-    (merge_* joins the ranks)."""
+    replica 0 of each case, with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica), and with
+    profile_axis <name>_profile_rank<rank>.csv (_map_profile_rows).  Returns the map rows; with replicas (map rows,
+    ensemble_stats of the replica rows), the latter None when world > 1 (merge_* joins the ranks)."""
     import csv
     rows, rep_rows = [], []
     for l in sorted(mine):
@@ -433,6 +493,9 @@ def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, 
             rows.append(row)
     out_dir = f"outputs/{output_root}"
     _write_rows(rows, os.path.join(out_dir, f"{name}_rank{rank}.csv"))
+    if profile_axis is not None:
+        _write_rows(_map_profile_rows(lats, sorted(mine), case_row, axes),
+                    os.path.join(out_dir, f"{name}_profile_rank{rank}.csv"))
     write_plot_cet_tree([(row["case"], f"outputs/{lats[l][2]}/metrics.csv")
                          for row, l in zip(rows, sorted(l for l in mine if lats[l][1] == 0))],
                         os.path.join(out_dir, "plot_cet"))
@@ -440,6 +503,41 @@ def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, 
         return rows
     _write_rows(rep_rows, os.path.join(out_dir, f"{name}_replicas_rank{rank}.csv"))
     return rows, (ensemble_stats(rep_rows, axes) if world == 1 else None)
+
+
+def _map_profile_rows(lats, mine, case_row, axes):
+    """One row per lattice of `mine` (case, replica, the map's axis columns, CET_Height and Front_Height of
+    metrics.cet_profile_summary over the final row's profile in outputs/<prefix>/cet_profile.csv)."""
+    out = []
+    for l in mine:
+        q, r, p = lats[l]
+        _step, prof = read_profile_csv(f"outputs/{p}/{PROFILE_CSV}")
+        s = _metrics.cet_profile_summary(prof, prof.shape[1] ** 2)
+        c = case_row(q)
+        out.append({"case": q, "replica": r, **{k: c[k] for k in axes}, "CET_Height": s["CET_Height"],
+                    "Front_Height": s["Front_Height"]})
+    return out
+
+
+def profile_ensemble_stats(rows, axes):
+    """One row per case over the rows of a <map>_profile.csv (dicts with case, replica, the axis columns `axes`,
+    CET_Height; numbers or the strings a CSV gives back), in case order: case, the axes, replicas (n), p_cet_height
+    (the fraction of replicas with a CET height >= 0) and CET_Height_mean / CET_Height_se over those replicas (the
+    standard error is the sample standard deviation, ddof=1, over the square root of their number; empty below 2,
+    the mean empty when no replica has a CET height)."""
+    by_case = {}
+    for r in rows:
+        by_case.setdefault(int(r["case"]), []).append(r)
+    out = []
+    for case in sorted(by_case):
+        rs = by_case[case]
+        h = np.array([int(r["CET_Height"]) for r in rs])
+        v = h[h >= 0].astype(np.float64)
+        out.append({"case": case, **{k: rs[0][k] for k in axes}, "replicas": len(rs),
+                    "p_cet_height": float(np.mean(h >= 0)),
+                    "CET_Height_mean": float(np.mean(v)) if v.size else "",
+                    "CET_Height_se": float(np.std(v, ddof=1) / np.sqrt(v.size)) if v.size > 1 else ""})
+    return out
 
 
 def ensemble_stats(rows, axes):
@@ -470,7 +568,7 @@ def ensemble_stats(rows, axes):
 
 def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
                        events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy",
-                       lasers=None, replicas=None):
+                       lasers=None, replicas=None, profile_axis=None):
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
@@ -482,11 +580,14 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     sweep, as the laser driver of run_cet_sublattice stops it.
     replicas: None, or the replica number r of each case: the case then runs as run_cet_sublattice(seed=seed + r,
     init_seed=42 + r).  The generated initial lattices of the group are built on the device by one cetkmc.init_group
-    call (_upload_initial)."""
+    call (_upload_initial).
+    profile_axis: every metrics row also takes its cases' grain profiles with one cetkmc.grain_profile_group call
+    (_cadence_group), and each case writes the cet_profile.csv run_cet_sublattice(profile_axis=...) writes."""
     if mask_stream not in ("numpy", "philox"):
         raise ValueError("mask_stream must be 'numpy' or 'philox'")
     if lasers is not None and int(thermal_every) <= 0:
         raise ValueError("the laser variant needs thermal_every >= 1")
+    _check_profile_axis("_run_cases_grouped", profile_axis)
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
     philox_mask = mask_stream == "philox"
@@ -500,7 +601,7 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
             ctx = _lib.Context(L=L, device=device)
             ctx.init_seed = None if replicas is None else 42 + reps[q]
             ctx.init_nuclei = []
-            r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], total_time=0.0,
+            r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], profiles=[], total_time=0.0,
                      nucleation_count=0, cet_detected=False, terminated=False)
             runs.append(r)
             ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
@@ -536,13 +637,14 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
                     sweep += blk
                     stopped = [r for r in active if r["terminated"]]
                     if stopped:
-                        _cadence_group(stopped, sweep - 1, every, philox_mask, seed)
+                        _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis)
                         active = [r for r in active if not r["terminated"]]
             if active:
-                _cadence_group(active, sweep - 1, every, philox_mask, seed)
+                _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis)
             active = [r for r in active if not r["terminated"]]
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
+            _write_profile_csv(r["profiles"], f"outputs/{r['prefix']}")
     finally:
         for r in runs:
             r["ctx"].close()
@@ -592,12 +694,15 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     lattices are partitioned and grouped as cases are.  The map file and the plot_cet tree come from replica 0, so
     they equal those of a run without replicas; each rank also writes melt_pool_map_replicas_rank<r>.csv (one row
     per (case, replica), the map's columns).  Returns (map rows, ensemble_stats rows; None when world > 1).
-    Not with `checkpoint_every`, `resume_from` or `lattice`."""
+    Not with `checkpoint_every`, `resume_from` or `lattice`.
+    profile_axis=a (through **kw): every case writes outputs/<prefix>/cet_profile.csv (run_cet_sublattice), and each
+    rank writes melt_pool_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it."""
     rank = int(os.environ.get("RANK", 0)) if rank is None else rank
     world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
     local = int(os.environ.get("LOCAL_RANK", 0))
     devices = [local] if devices is None else list(devices)
     n_rep = _check_replicas("run_melt_pool_map", replicas, kw)
+    _check_profile_axis("run_melt_pool_map", kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
     if not powers or not speeds:
         raise ValueError("run_melt_pool_map: needs at least one power and one speed")
@@ -634,7 +739,7 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
         return {"power": cases[q][0], "speed": cases[q][1], "T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R,
                 "G_over_R": G / R if R > 0 else np.inf}
     return _map_outputs(output_root, "melt_pool_map", lats, [l for _d, ls in parts for l in ls], case_row,
-                        ("power", "speed", "T_sub", "NU_DEP"), replicas, rank, world)
+                        ("power", "speed", "T_sub", "NU_DEP"), replicas, rank, world, kw.get("profile_axis"))
 
 
 def write_plot_cet_tree(cases, root):
@@ -682,16 +787,22 @@ def _merge_map(output_root, name, axes):
     reps = _merge_rank_files(output_root, f"{name}_replicas")
     if reps:
         _write_rows(ensemble_stats(reps, axes), f"outputs/{output_root}/{name}_ensemble.csv")
+    prof = _merge_rank_files(output_root, f"{name}_profile")
+    if prof and reps:
+        _write_rows(profile_ensemble_stats(prof, axes), f"outputs/{output_root}/{name}_profile_ensemble.csv")
     return rows
 
 
 def merge_cet_map(output_root="gr_sweep"):
     """Join the per-rank files of run_gr_sweep into outputs/<output_root>/cet_map.csv (sorted by case); after a run
-    with replicas also cet_map_replicas.csv and cet_map_ensemble.csv (ensemble_stats, one row per case)."""
+    with replicas also cet_map_replicas.csv and cet_map_ensemble.csv (ensemble_stats, one row per case); after a run
+    with profile_axis also cet_map_profile.csv (sorted by case and replica), and with replicas
+    cet_map_profile_ensemble.csv (profile_ensemble_stats)."""
     return _merge_map(output_root, "cet_map", ("T_sub", "NU_DEP"))
 
 
 def merge_melt_pool_map(output_root="melt_pool_map"):
     """Join the per-rank files of run_melt_pool_map into outputs/<output_root>/melt_pool_map.csv (sorted by case);
-    after a run with replicas also melt_pool_map_replicas.csv and melt_pool_map_ensemble.csv (ensemble_stats)."""
+    after a run with replicas also melt_pool_map_replicas.csv and melt_pool_map_ensemble.csv (ensemble_stats); after
+    a run with profile_axis also melt_pool_map_profile.csv and, with replicas, melt_pool_map_profile_ensemble.csv."""
     return _merge_map(output_root, "melt_pool_map", ("power", "speed", "T_sub", "NU_DEP"))

@@ -258,6 +258,15 @@ __device__ __forceinline__ void grain_stat_init(GrainStat *g, int root)
     *g = t;
 }
 
+// utils.py:104-111 as metrics.grain_aspect_ratios evaluates it; a grain is equiaxed when this is below the
+// AR threshold (metrics_reduce_group_kernel's n_equiaxed, cet_grain_profile_group's class)
+__device__ __forceinline__ double grain_ar(const GrainStat &s)
+{
+    const int d0 = s.hi[0] - s.lo[0] + 1, d1 = s.hi[1] - s.lo[1] + 1, d2 = s.hi[2] - s.lo[2] + 1;
+    const int mx = max(d0, max(d1, d2)), mn = min(d0, min(d1, d2));
+    return __ddiv_rn((double)mx, (double)max(mn, 1));
+}
+
 // One atomic set per (warp, grain): lanes holding voxels of the same grain elect a leader.
 __device__ __forceinline__ void grains_stats_body(const int *__restrict__ label, const int *__restrict__ gid, int64_t lo,
                                                   int64_t hi, GrainStat *st, int L, int i_off)

@@ -176,6 +176,8 @@ struct cet_ctx {
     size_t cap_grain_st = 0;
     void *group_tab = nullptr;        // result table of the groups this context leads (GROUP_MAX entries)
     cudaEvent_t ev_group = nullptr;   // orders this context's stream before the work of a group led by another context
+    void *profile_tab = nullptr;      // grain-profile tables and span differences of the groups this context leads, grow-only
+    size_t cap_profile_tab = 0;
 
     // per-kernel-kind device timing (cet_profile_*): event pairs recorded around the dominant
     // kernels on the context stream, resolved when the totals are read
@@ -213,6 +215,11 @@ int orient_update(cet_ctx *c, int64_t p_lo, int64_t p_hi);
 int nst_build(cet_ctx *c, int p_lo, int p_hi);     // rebuild the neighbour-state cache of local planes [p_lo, p_hi)
 int nst_ensure(cet_ctx *c);                          // ... of every plane it can be built for, if it is stale
 int sm_count(cet_ctx *c);                            // multiprocessors of the context's device
+// groups of contexts (metrics_group.cu): the common argument checks (distinct whole-lattice cubic contexts of one L
+// on one device, 1 <= n_ctx <= GROUP_MAX), and the order of the group's work on ctxs[0]'s stream after the work
+// already queued on every member's stream
+int group_check(const char *fn, cet_ctx *const *ctxs, int32_t n_ctx);
+int group_order(cet_ctx *const *ctxs, int n);
 // every writer of vox / theta / phi / T / defects other than the tile-aware sweep kernels calls this
 inline void lattice_changed(cet_ctx *c) { c->tile_valid = false; c->rates_valid = false; c->sweep_rates_valid = false; }
 enum { PROF_DECIDE = 0, PROF_APPLY = 1, PROF_THERMAL = 2, PROF_RATES = 3, PROF_HALO = 4, PROF_STEP = 5, PROF_PICK = 6,

@@ -154,14 +154,6 @@ __global__ void metrics_stats_group_kernel(const __grid_constant__ GroupArgs<MgA
     grains_stats_body(a.label, a.gid, 0, n, a.st, L, 0);
 }
 
-// utils.py:104-111 as metrics.grain_aspect_ratios evaluates it
-__device__ __forceinline__ double grain_ar(const GrainStat &s)
-{
-    const int d0 = s.hi[0] - s.lo[0] + 1, d1 = s.hi[1] - s.lo[1] + 1, d2 = s.hi[2] - s.lo[2] + 1;
-    const int mx = max(d0, max(d1, d2)), mn = min(d0, min(d1, d2));
-    return __ddiv_rn((double)mx, (double)max(mn, 1));
-}
-
 // NumPy's pairwise_sum of a[lo, lo + m) for m <= PW_LEAF
 __device__ double pw_leaf(const GrainStat *st, int lo, int m)
 {
@@ -283,7 +275,7 @@ __global__ void __launch_bounds__(1024) metrics_reduce_group_kernel(const __grid
 
 // ---- host side ----
 
-static int mg_check(const char *fn, cet_ctx *const *ctxs, int32_t n_ctx)
+int group_check(const char *fn, cet_ctx *const *ctxs, int32_t n_ctx)
 {
     CET_REQUIRE(ctxs, "%s: NULL argument", fn);
     CET_REQUIRE(n_ctx >= 1 && n_ctx <= GROUP_MAX, "%s: need 1 <= n_ctx <= %d, got %d", fn, GROUP_MAX, (int)n_ctx);
@@ -302,18 +294,25 @@ static int mg_check(const char *fn, cet_ctx *const *ctxs, int32_t n_ctx)
     return 0;
 }
 
-// the group's work goes to ctxs[0]'s stream, after the work already queued on every member's stream; the result
-// table lives in ctxs[0]
-static int mg_begin(cet_ctx *const *ctxs, int n)
+// the group's work goes to ctxs[0]'s stream, after the work already queued on every member's stream
+int group_order(cet_ctx *const *ctxs, int n)
 {
     cet_ctx *c0 = ctxs[0];
-    if (!c0->group_tab) CET_CUDA(cudaMalloc(&c0->group_tab, GROUP_MAX * sizeof(MgEntry)));
     for (int q = 1; q < n; ++q) {
         cet_ctx *c = ctxs[q];
         if (!c->ev_group) CET_CUDA(cudaEventCreateWithFlags(&c->ev_group, cudaEventDisableTiming));
         CET_CUDA(cudaEventRecord(c->ev_group, c->stream));
         CET_CUDA(cudaStreamWaitEvent(c0->stream, c->ev_group, 0));
     }
+    return 0;
+}
+
+// group_order, and the result table (in ctxs[0]) zeroed
+static int mg_begin(cet_ctx *const *ctxs, int n)
+{
+    cet_ctx *c0 = ctxs[0];
+    if (!c0->group_tab) CET_CUDA(cudaMalloc(&c0->group_tab, GROUP_MAX * sizeof(MgEntry)));
+    if (int rc = group_order(ctxs, n)) return rc;
     CET_CUDA(cudaMemsetAsync(c0->group_tab, 0, (size_t)n * sizeof(MgEntry), c0->stream));
     return 0;
 }
@@ -464,7 +463,7 @@ using namespace cet;
 
 extern "C" int cet_counts_group(cet_ctx *const *ctxs, int32_t n_ctx, int64_t *counts)
 {
-    if (int rc = mg_check("cet_counts_group", ctxs, n_ctx)) return rc;
+    if (int rc = group_check("cet_counts_group", ctxs, n_ctx)) return rc;
     CET_REQUIRE(counts, "cet_counts_group: NULL argument");
     cet::DeviceGuard dg(ctxs[0]->device);
     if (int rc = mg_begin(ctxs, n_ctx)) return rc;
@@ -474,7 +473,7 @@ extern "C" int cet_counts_group(cet_ctx *const *ctxs, int32_t n_ctx, int64_t *co
 extern "C" int cet_metrics_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_metrics_params *mp, const double *const *draws,
                                  const int64_t *n_draws, cet_metrics_result *res)
 {
-    if (int rc = mg_check("cet_metrics_group", ctxs, n_ctx)) return rc;
+    if (int rc = group_check("cet_metrics_group", ctxs, n_ctx)) return rc;
     CET_REQUIRE(mp && res, "cet_metrics_group: NULL argument");
     for (int q = 0; q < n_ctx; ++q) {
         if (!mp[q].refresh) continue;

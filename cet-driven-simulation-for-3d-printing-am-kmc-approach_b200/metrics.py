@@ -144,6 +144,37 @@ def metrics_from_summary(res, n_sites, voxel_size=None, rng_seed=None):
     }
 
 
+def cet_profile_summary(profile, plane_sites, eq_threshold=K.CET_EQ_THRESHOLD, min_solid=0.5):
+    """Where along the profile's axis a lattice turns equiaxed, from one (4, L) grain profile of
+    cetkmc.grain_profile_group (rows Solid, EquiaxedSolid, GrainsSpanning, EquiaxedGrainsSpanning).
+
+    The solidified planes P are the planes z with Solid[z] >= min_solid * plane_sites (plane_sites: the
+    sites of one plane, L * L), so melt or vapour planes above the front do not count; a plane without
+    solid is never in P.
+        Front_Height  the largest z in P; -1 when P is empty.
+        CET_Height    with eq[z] = EquiaxedSolid[z] / Solid[z], the smallest z in P such that
+                      eq[z'] >= eq_threshold for every z' in P with z' >= z; -1 when P is empty or the
+                      top plane of P is below the threshold.
+    A lattice equiaxed through every solidified plane gets the lowest plane of P (0 when the substrate
+    plane is solidified); a lattice columnar at its front gets -1; an equiaxed plane below a columnar band
+    does not count.  Returns {"CET_Height": int, "Front_Height": int}."""
+    p = np.asarray(profile)
+    if p.ndim != 2 or p.shape[0] != 4:
+        raise ValueError(f"cet_profile_summary: need a (4, L) profile, got shape {p.shape}")
+    solid, eq_solid = p[0].astype(np.float64), p[1].astype(np.float64)
+    planes = np.nonzero(solid >= float(min_solid) * float(plane_sites))[0]
+    planes = planes[solid[planes] > 0]
+    if planes.size == 0:
+        return {"CET_Height": -1, "Front_Height": -1}
+    eq = eq_solid[planes] / solid[planes]
+    cet = -1
+    for k in range(planes.size - 1, -1, -1):            # walk down from the front while the planes stay equiaxed
+        if eq[k] < eq_threshold:
+            break
+        cet = int(planes[k])
+    return {"CET_Height": cet, "Front_Height": int(planes[-1])}
+
+
 def grains_distributed(ctx, all_gather, theta_threshold=0.5):
     """Grains of a lattice that is split into z-slabs over several contexts (one per rank), in the form
     Context.grains() returns for a whole lattice — the reference's clusters (utils.py:28-84) in its

@@ -296,6 +296,26 @@ int cet_counts_group(cet_ctx *const *ctxs, int32_t n_ctx, int64_t *counts);
  * allocation once the per-context buffers have grown to the lattice's needs. */
 int cet_metrics_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_metrics_params *mp, const double *const *draws,
                       const int64_t *n_draws, cet_metrics_result *res);
+/* ---- per-plane grain profile of a group (where along a growth axis the grains turn equiaxed) ----
+ * Per-plane profile of the last grain labelling (cet_grains_label[_ex] or cet_metrics_group) of each context, along
+ * `axis` (0, 1 or 2).  out[(q * 4 + f) * L + z], int64, for context q and plane z:
+ *   f = 0  Solid                    occupied sites (label >= 0) with coordinate z
+ *   f = 1  EquiaxedSolid            of those, sites whose grain has aspect ratio < ar_threshold
+ *   f = 2  GrainsSpanning           grains whose bounding box along `axis` contains z
+ *   f = 3  EquiaxedGrainsSpanning   of those, grains with aspect ratio < ar_threshold
+ * The aspect ratio is metrics.grain_aspect_ratios' (utils.py:104-111), evaluated exactly as cet_metrics_group
+ * evaluates it, so a grain's class is the one its EquiaxedFraction counts.  Grains are joined through the 14-offset
+ * neighbourhood, which steps +-2 along each axis, so a grain can hold sites on planes z and z + 2 and none on
+ * z + 1: the spanning columns count the grains whose bounding box (what the aspect ratio measures) covers z, not
+ * the grains with a site on z.
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device, 1 <= n_ctx <= 64,
+ * each with a labelling of the whole lattice (a context never labelled is rejected).  The call reports that
+ * labelling as cet_grains_stats does and does not relabel; it is read-only on the lattice, the labels and the mask,
+ * so the next metrics row and the next sweeps are what they would have been without it.  Everything, `out`
+ * included, is checked before anything is launched or written: a rejected call leaves every context and `out` as
+ * they were.  The work is ordered on the stream of ctxs[0] after the work already queued on every context's
+ * stream: one memset, five launches for the whole group, one D2H copy of the table, one host synchronisation. */
+int cet_grain_profile_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, double ar_threshold, int64_t *out);
 /* The same for global planes [i_lo, i_hi) within the labelled planes of a slab (owned + 2 ghost planes per
  * cut face): what two neighbouring slabs compare to join the grains that cross their cut. */
 int cet_grains_download_planes(cet_ctx *ctx, int64_t i_lo, int64_t i_hi, int32_t *labels);

@@ -8,6 +8,9 @@ GPUs of one box, producing cet_map.csv and the tree the reference's plot_cet.py 
 the outputs are the same as without it.
 --replicas n: every case runs n times (replica r with seed + r and initial-lattice seed 42 + r); rank 0 also writes
 cet_map_ensemble.csv (mean, standard error and equiaxed fraction over the replicas of each case) and prints it.
+--profile-axis a: every case also records per-plane grain profiles along axis a (0, 1 or 2; the generated lattices
+grow along 2) in <case>/cet_profile.csv; rank 0 writes cet_map_profile.csv (CET height and front height of every
+lattice) and prints it, and with --replicas also cet_map_profile_ensemble.csv.
 """
 import argparse
 import csv
@@ -30,13 +33,15 @@ def main():
     ap.add_argument("--out", default="gr_sweep")
     ap.add_argument("--batch", type=int, default=None)
     ap.add_argument("--replicas", type=int, default=None)
+    ap.add_argument("--profile-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     temps = [2600.0, 2800.0, 3000.0, 3200.0]                      # T_sub -> G = (T_MELT - T_sub) / (L dx)
     nu_deps = [1e12, 5e12, 2e13, 1e14]                            # NU_DEP -> R
     t0 = time.perf_counter()
     rows = campaign.run_gr_sweep(temps, nu_deps, L=args.L, n_sweeps=args.sweeps, n_seeds=20, defect_fraction=3e-3,
-                                 impurity_c=0.1, output_root=args.out, metrics_every=100, batch=args.batch, replicas=args.replicas)
+                                 impurity_c=0.1, output_root=args.out, metrics_every=100, batch=args.batch, replicas=args.replicas,
+                                 **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -53,6 +58,11 @@ def main():
         for r in merged:
             print(f"case {int(r['case']):2d} T_sub {float(r['T_sub']):6.0f} NU_DEP {float(r['NU_DEP']):8.1e} G/R {float(r['G_over_R']):9.3e} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} {r['CET_Class']}")
+        if args.profile_axis is not None:
+            for fn in ("cet_map_profile.csv",) + (("cet_map_profile_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.replicas is not None:
             with open(f"outputs/{args.out}/cet_map_ensemble.csv") as fh:
                 for e in csv.DictReader(fh):

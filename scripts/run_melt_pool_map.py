@@ -8,6 +8,9 @@ one box, producing melt_pool_map.csv and the tree the reference's plot_cet.py re
 sweeps and for the laser step); the outputs are the same as without it.
 --replicas n: every case runs n times (replica r with seed + r and initial-lattice seed 42 + r); rank 0 also writes
 melt_pool_map_ensemble.csv (mean, standard error and equiaxed fraction over the replicas of each case) and prints it.
+--profile-axis a: every case also records per-plane grain profiles along axis a (0, 1 or 2; the generated lattices
+grow along 2) in <case>/cet_profile.csv; rank 0 writes melt_pool_map_profile.csv (CET height and front height of every
+lattice) and prints it, and with --replicas also melt_pool_map_profile_ensemble.csv.
 """
 import argparse
 import csv
@@ -29,6 +32,7 @@ def main():
     ap.add_argument("--out", default="melt_pool_map")
     ap.add_argument("--batch", type=int, default=None)
     ap.add_argument("--replicas", type=int, default=None)
+    ap.add_argument("--profile-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     powers = [100.0, 200.0, 300.0, 400.0]                         # W
@@ -36,7 +40,8 @@ def main():
     t0 = time.perf_counter()
     campaign.run_melt_pool_map(powers, speeds, L=args.L, n_sweeps=args.sweeps, start=(args.L / 2, 0.0),
                                n_seeds=20, defect_fraction=3e-3, impurity_c=0.1, output_root=args.out,
-                               metrics_every=100, batch=args.batch, replicas=args.replicas)
+                               metrics_every=100, batch=args.batch, replicas=args.replicas,
+                               **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -54,6 +59,11 @@ def main():
             print(f"case {int(r['case']):2d} P {float(r['power']):6.1f} W V {float(r['speed']):5.2f} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} "
                   f"step {r['Step']} {r['CET_Class']}")
+        if args.profile_axis is not None:
+            for fn in ("melt_pool_map_profile.csv",) + (("melt_pool_map_profile_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.replicas is not None:
             with open(f"outputs/{args.out}/melt_pool_map_ensemble.csv") as fh:
                 for e in csv.DictReader(fh):

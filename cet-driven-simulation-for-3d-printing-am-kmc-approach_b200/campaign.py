@@ -228,6 +228,15 @@ def _check_profile_axis(fn, profile_axis, world=1, checkpoint_every=0, resume_fr
         raise ValueError(f"{fn}: profile_axis does not take checkpoint_every or resume_from")
 
 
+def _check_mask_and_laser(fn, mask_stream, laser, thermal_every):
+    """Refuse a defect-mask stream other than "numpy" or "philox", and a laser run (`laser` true) without a thermal
+    step (thermal_every < 1)."""
+    if mask_stream not in ("numpy", "philox"):
+        raise ValueError("mask_stream must be 'numpy' or 'philox'")
+    if laser and int(thermal_every) < 1:
+        raise ValueError(f"{fn}: the laser variant needs thermal_every >= 1")
+
+
 def _write_profile_csv(profiles, output_dir):
     """outputs/<prefix>/cet_profile.csv: one row per (metrics row, plane) of the (step, (4, L) profile) pairs."""
     import csv
@@ -298,8 +307,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
 
     if world > 1 and (laser or checkpoint_every or resume_from):
         raise ValueError("run_cet_sublattice: the laser variant and checkpoint / resume are single-GPU")
-    if mask_stream not in ("numpy", "philox"):
-        raise ValueError("mask_stream must be 'numpy' or 'philox'")
+    _check_mask_and_laser("run_cet_sublattice", mask_stream, laser, thermal_every)
     philox_mask = world > 1 or mask_stream == "philox"
     all_gather = None
     i_begin, i_end = _ks.slab_bounds(L, world, rank)
@@ -320,8 +328,6 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             ctx.comm_init(bcast_bytes(_lib.comm_unique_id() if rank == 0 else None), rank, world)
             ctx.halo_exchange(7)
         sp, tp = _sweep_setup(L, seed, temp, events_per_sweep, p_max, defect_fraction, 0 if laser else thermal_every)
-        if laser and int(thermal_every) <= 0:
-            raise ValueError("run_cet_sublattice: the laser variant needs thermal_every >= 1")
         if laser:
             l_dt = float(laser.get("dt", _ks.THERMAL_DT))
             l_pos = [float(x) for x in laser.get("start", (0.0, 0.0))]
@@ -409,38 +415,50 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
     world > 1) instead of the map rows.  Not with `checkpoint_every`, `resume_from` or `lattice`.
     profile_axis=a (through **kw): every case writes outputs/<prefix>/cet_profile.csv (run_cet_sublattice), and each
     rank writes cet_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it."""
-    rank = int(os.environ.get("RANK", 0)) if rank is None else rank
-    world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
-    local = int(os.environ.get("LOCAL_RANK", 0))
-    devices = [local] if devices is None else list(devices)
-    n_rep = _check_replicas("run_gr_sweep", replicas, kw)
-    _check_profile_axis("run_gr_sweep", kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
-    if batch is not None:
-        bad = [k for k in ("laser", "checkpoint_every", "resume_from", "lattice") if kw.get(k)]
-        if bad:
-            raise ValueError(f"run_gr_sweep: batch does not take {', '.join(bad)}")
     cases = [(float(t), float(r)) for t in temps for r in nu_deps]
-    os.makedirs(f"outputs/{output_root}", exist_ok=True)
-    prefix = [f"{output_root}/T{temp:g}_R{nu_dep:g}" for temp, nu_dep in cases]
-    lats = _map_lattices(prefix, n_rep)
-    parts = gr_partition(len(lats), rank, world, devices, batch)
-    for device, ls in parts:
-        if batch is None:
-            q, r, p = lats[ls[0]]
-            run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=cases[q][0], nu_dep=cases[q][1], impurity_c=impurity_c,
-                               n_seeds=n_seeds, defect_fraction=defect_fraction, output_prefix=p,
-                               device=device, verbose=False, **_replica_kw(kw, replicas, r))
-        else:
-            _run_cases_grouped([(lats[l][2],) + cases[lats[l][0]] for l in ls], L=L, n_sweeps=n_sweeps,
-                               impurity_c=impurity_c, n_seeds=n_seeds, defect_fraction=defect_fraction, device=device,
-                               replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
 
     def case_row(q):
         temp, nu_dep = cases[q]
         G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
         return {"T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R, "G_over_R": G / R if R > 0 else np.inf}
-    return _map_outputs(output_root, "cet_map", lats, [l for _d, ls in parts for l in ls], case_row,
-                        ("T_sub", "NU_DEP"), replicas, rank, world, kw.get("profile_axis"))
+    return _run_map("run_gr_sweep", "cet_map", ("T_sub", "NU_DEP"), case_row, output_root,
+                    [(f"{output_root}/T{temp:g}_R{nu_dep:g}", temp, nu_dep) for temp, nu_dep in cases], None,
+                    ("laser", "checkpoint_every", "resume_from", "lattice"), rank, world, devices, batch, replicas,
+                    dict(kw, L=L, n_sweeps=n_sweeps, impurity_c=impurity_c, n_seeds=n_seeds,
+                         defect_fraction=defect_fraction))
+
+
+def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses, rank, world, devices, batch,
+             replicas, kw):
+    """The body of the map driver `fn` (run_gr_sweep, run_melt_pool_map): every replica of case q of `cases` (output
+    prefix, temp, nu_dep) is run_cet_sublattice(output_prefix=..., temp=..., nu_dep=..., laser=lasers[q] unless
+    lasers is None, **kw), partitioned over ranks and devices by gr_partition; batch=k advances them in groups
+    (_run_cases_grouped) and refuses the keywords `batch_refuses`.  Writes and returns the map `name` (_map_outputs)."""
+    rank = int(os.environ.get("RANK", 0)) if rank is None else rank
+    world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
+    devices = [int(os.environ.get("LOCAL_RANK", 0))] if devices is None else list(devices)
+    n_rep = _check_replicas(fn, replicas, kw)
+    _check_profile_axis(fn, kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
+    _check_mask_and_laser(fn, kw.get("mask_stream", "numpy"), lasers is not None or kw.get("laser"),
+                          kw.get("thermal_every", _ks.THERMAL_EVERY))
+    if batch is not None:
+        bad = [k for k in batch_refuses if kw.get(k)]
+        if bad:
+            raise ValueError(f"{fn}: batch does not take {', '.join(bad)}")
+    os.makedirs(f"outputs/{output_root}", exist_ok=True)
+    lats = _map_lattices([p for p, _t, _r in cases], n_rep)
+    parts = gr_partition(len(lats), rank, world, devices, batch)
+    for device, ls in parts:
+        if batch is None:
+            q, r, p = lats[ls[0]]
+            run_cet_sublattice(output_prefix=p, temp=cases[q][1], nu_dep=cases[q][2], device=device, verbose=False,
+                               **({} if lasers is None else {"laser": lasers[q]}), **_replica_kw(kw, replicas, r))
+        else:
+            _run_cases_grouped([(lats[l][2],) + cases[lats[l][0]][1:] for l in ls], device=device,
+                               lasers=None if lasers is None else [lasers[lats[l][0]] for l in ls],
+                               replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
+    return _map_outputs(output_root, name, lats, [l for _d, ls in parts for l in ls], case_row, axes, replicas, rank,
+                        world, kw.get("profile_axis"))
 
 
 _MAP_FINAL = ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount",
@@ -573,20 +591,17 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
     around its host draws).  The metrics cadence of the group is one cetkmc.metrics_group call per row
-    (_cadence_group).  A case that terminates stops at the row it stops at alone and leaves the group.
+    (_cadence_group).  A case that terminates leaves the group after the block of sweeps it terminated in, with its
+    row at that block's last sweep, as run_cet_sublattice stops it; a block is a metrics interval, or with lasers the
+    part of one between two thermal steps.
     lasers: None, or one laser dict per case (run_cet_sublattice(laser=...)): every `thermal_every` sweeps one
-    cetkmc.thermal_full_group over the cases still running replaces their thermal_full + snapshot_state, and a case
-    that terminates leaves the group after the block of sweeps it terminated in, with its row at that block's last
-    sweep, as the laser driver of run_cet_sublattice stops it.
+    cetkmc.thermal_full_group over the cases still running replaces their thermal_full + snapshot_state.
     replicas: None, or the replica number r of each case: the case then runs as run_cet_sublattice(seed=seed + r,
     init_seed=42 + r).  The generated initial lattices of the group are built on the device by one cetkmc.init_group
     call (_upload_initial).
     profile_axis: every metrics row also takes its cases' grain profiles with one cetkmc.grain_profile_group call
     (_cadence_group), and each case writes the cet_profile.csv run_cet_sublattice(profile_axis=...) writes."""
-    if mask_stream not in ("numpy", "philox"):
-        raise ValueError("mask_stream must be 'numpy' or 'philox'")
-    if lasers is not None and int(thermal_every) <= 0:
-        raise ValueError("the laser variant needs thermal_every >= 1")
+    _check_mask_and_laser("_run_cases_grouped", mask_stream, lasers is not None, thermal_every)
     _check_profile_axis("_run_cases_grouped", profile_axis)
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
@@ -624,24 +639,19 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
         active = runs
         while sweep < n_sweeps and active:
             end = _stop_at(sweep, every, n_sweeps) + 1
-            if lasers is None:
+            while sweep < end and active:
+                blk = end - sweep if lasers is None else min(end - sweep, thermal_every - sweep % thermal_every)
+                if lasers is not None and sweep % thermal_every == 0:
+                    _laser_step_group(active, L)
                 tps = None if active[0]["tp"] is None else [r["tp"] for r in active]     # one thermal_every for all cases
-                _absorb(active, _lib.sweep_run_group([r["ctx"] for r in active], end - sweep, [r["sp"] for r in active], tps))
-                sweep = end
-            else:
-                while sweep < end and active:
-                    blk = min(end - sweep, thermal_every - sweep % thermal_every)
-                    if sweep % thermal_every == 0:
-                        _laser_step_group(active, L)
-                    _absorb(active, _lib.sweep_run_group([r["ctx"] for r in active], blk, [r["sp"] for r in active]))
-                    sweep += blk
-                    stopped = [r for r in active if r["terminated"]]
-                    if stopped:
-                        _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis)
-                        active = [r for r in active if not r["terminated"]]
+                _absorb(active, _lib.sweep_run_group([r["ctx"] for r in active], blk, [r["sp"] for r in active], tps))
+                sweep += blk
+                stopped = [r for r in active if r["terminated"]]
+                if stopped:
+                    _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis)
+                    active = [r for r in active if not r["terminated"]]
             if active:
                 _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis)
-            active = [r for r in active if not r["terminated"]]
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
             _write_profile_csv(r["profiles"], f"outputs/{r['prefix']}")
@@ -697,49 +707,25 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     Not with `checkpoint_every`, `resume_from` or `lattice`.
     profile_axis=a (through **kw): every case writes outputs/<prefix>/cet_profile.csv (run_cet_sublattice), and each
     rank writes melt_pool_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it."""
-    rank = int(os.environ.get("RANK", 0)) if rank is None else rank
-    world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
-    local = int(os.environ.get("LOCAL_RANK", 0))
-    devices = [local] if devices is None else list(devices)
-    n_rep = _check_replicas("run_melt_pool_map", replicas, kw)
-    _check_profile_axis("run_melt_pool_map", kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
     if not powers or not speeds:
         raise ValueError("run_melt_pool_map: needs at least one power and one speed")
-    if int(kw.get("thermal_every", _ks.THERMAL_EVERY)) < 1:
-        raise ValueError("run_melt_pool_map: the laser step needs thermal_every >= 1")
-    if batch is not None:
-        bad = [k for k in ("checkpoint_every", "resume_from", "lattice") if kw.get(k)]
-        if bad:
-            raise ValueError(f"run_melt_pool_map: batch does not take {', '.join(bad)}")
     temp = constants.T_SUB if temp is None else float(temp)
     nu_dep = constants.NU_DEP if nu_dep is None else float(nu_dep)
     dt = _ks.THERMAL_DT if dt is None else float(dt)
     cases = [(p, v) for p in powers for v in speeds]
     lasers = [dict(power=p, speed=v, start=tuple(start), dt=dt, beam_radius=beam_radius, absorptivity=absorptivity)
               for p, v in cases]
-    prefix = [f"{output_root}/P{p:g}_V{v:g}" for p, v in cases]
-    os.makedirs(f"outputs/{output_root}", exist_ok=True)
-    lats = _map_lattices(prefix, n_rep)
-    parts = gr_partition(len(lats), rank, world, devices, batch)
-    for device, ls in parts:
-        if batch is None:
-            q, r, p = lats[ls[0]]
-            run_cet_sublattice(L=L, n_sweeps=n_sweeps, temp=temp, nu_dep=nu_dep, impurity_c=impurity_c, n_seeds=n_seeds,
-                               defect_fraction=defect_fraction, output_prefix=p, laser=lasers[q], device=device,
-                               verbose=False, **_replica_kw(kw, replicas, r))
-        else:
-            _run_cases_grouped([(lats[l][2], temp, nu_dep) for l in ls], L=L, n_sweeps=n_sweeps, impurity_c=impurity_c,
-                               n_seeds=n_seeds, defect_fraction=defect_fraction, device=device,
-                               lasers=[lasers[lats[l][0]] for l in ls],
-                               replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
     G, R, _rp, _gr_phys = _gr(L, temp, nu_dep)
 
     def case_row(q):
         return {"power": cases[q][0], "speed": cases[q][1], "T_sub": temp, "NU_DEP": nu_dep, "G": G, "R": R,
                 "G_over_R": G / R if R > 0 else np.inf}
-    return _map_outputs(output_root, "melt_pool_map", lats, [l for _d, ls in parts for l in ls], case_row,
-                        ("power", "speed", "T_sub", "NU_DEP"), replicas, rank, world, kw.get("profile_axis"))
+    return _run_map("run_melt_pool_map", "melt_pool_map", ("power", "speed", "T_sub", "NU_DEP"), case_row, output_root,
+                    [(f"{output_root}/P{p:g}_V{v:g}", temp, nu_dep) for p, v in cases], lasers,
+                    ("checkpoint_every", "resume_from", "lattice"), rank, world, devices, batch, replicas,
+                    dict(kw, L=L, n_sweeps=n_sweeps, impurity_c=impurity_c, n_seeds=n_seeds,
+                         defect_fraction=defect_fraction))
 
 
 def write_plot_cet_tree(cases, root):

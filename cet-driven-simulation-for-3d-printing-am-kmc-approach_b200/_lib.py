@@ -139,6 +139,7 @@ SIGNATURES = {
     "cet_metrics_group": [C.POINTER(_VP), _I32, C.POINTER(MetricsParams), C.POINTER(_VP), C.POINTER(_I64),
                           C.POINTER(MetricsResult)],
     "cet_grain_profile_group": [C.POINTER(_VP), _I32, _I32, _F64, C.POINTER(_I64)],
+    "cet_grain_shape_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, _I64, C.POINTER(_I64)],
     "cet_debug_nst_mismatches": [_VP, C.POINTER(_I64)],
     "cet_debug_flags": [_VP, C.c_int],
     "cet_profile_enable": [_VP, C.c_int],
@@ -674,6 +675,49 @@ def grain_profile_group(ctxs, axis, ar_threshold):
     check(lib().cet_grain_profile_group(handles, len(ctxs), int(axis), thr, out.ctypes.data_as(C.POINTER(C.c_int64))),
           "cet_grain_profile_group")
     return out
+
+
+SHAPE_EDGES = (1.0, 1.5, 2.0, 3.0, 4.0, 6.0, 8.0, 12.0, 16.0, 32.0)   # grain_shape_group's default bin edges of A
+SHAPE_MIN_SIZE = 8                  # grains below this many sites go to the small bucket: a +-2 pair (A = sqrt(13)) is no column
+SHAPE_EDGES_MAX = 62
+
+
+def grain_shape_group(ctxs, axis, edges=SHAPE_EDGES, min_size=SHAPE_MIN_SIZE):
+    """Histogram of the growth-axis elongation of every grain of the last grain labelling (Context.grains(),
+    metrics_group) of every context of `ctxs` (whole-lattice Contexts of one L on one device), with three launches and
+    one copy for the group.  A grain's elongation along `axis` (0, 1 or 2) is A = sqrt(2 Q_a / (Q_b + Q_c)) with Q_x
+    its exact second moment along x, each site a unit cube (include/cetkmc.h: cet_grain_shape_group): a single site
+    has A = 1, a 1 x 1 x h column along the axis A = h.  Returns an (n, 2, len(edges) + 2) int64 array: for context
+    q, [q, 0, b] grains and [q, 1, b] their sites in bin b, where bin b <= len(edges) holds the grains of >= min_size
+    sites with edges[b - 1] <= A < edges[b] (edges[-1] = 0, edges[len(edges)] = inf) and bin len(edges) + 1 every
+    grain of fewer than min_size sites.  edges: 1 to 62 finite values > 0, strictly ascending.  The call does not
+    relabel and changes nothing the next metrics row, profile or sweep reads."""
+    ctxs = list(ctxs)
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"grain_shape_group: axis must be 0, 1 or 2, got {axis!r}")
+    e = _shape_edges("grain_shape_group", edges)
+    if isinstance(min_size, bool) or not isinstance(min_size, (int, np.integer)) or int(min_size) < 1:
+        raise ValueError(f"grain_shape_group: min_size must be an integer >= 1, got {min_size!r}")
+    handles = _group_handles("grain_shape_group", ctxs)
+    out = np.zeros((len(ctxs), 2, e.size + 2), np.int64)
+    check(lib().cet_grain_shape_group(handles, len(ctxs), int(axis), e.ctypes.data_as(C.POINTER(C.c_double)), e.size,
+                                      int(min_size), out.ctypes.data_as(C.POINTER(C.c_int64))), "cet_grain_shape_group")
+    return out
+
+
+def _shape_edges(fn, edges):
+    """The bin edges of a grain-shape histogram as a float64 array, refusing what cet_grain_shape_group refuses."""
+    try:
+        e = np.ascontiguousarray(np.asarray(edges, dtype=np.float64))
+    except (TypeError, ValueError):
+        raise ValueError(f"{fn}: edges must be numbers, got {edges!r}") from None
+    if e.ndim != 1 or not 1 <= e.size <= SHAPE_EDGES_MAX:
+        raise ValueError(f"{fn}: edges must be 1 to {SHAPE_EDGES_MAX} values, got shape {e.shape}")
+    if not np.all(np.isfinite(e)) or not np.all(e > 0.0):
+        raise ValueError(f"{fn}: edges must be finite and > 0, got {edges!r}")
+    if not np.all(np.diff(e) > 0.0):
+        raise ValueError(f"{fn}: edges must ascend strictly, got {edges!r}")
+    return e
 
 
 def comm_unique_id() -> bytes:

@@ -22,6 +22,10 @@
                                      every metrics row in outputs/<prefix>/cet_profile.csv
                                      (cetkmc.grain_profile_group), and per map the CET height of every
                                      lattice (metrics.cet_profile_summary) in <map>_profile.csv
+    shape_axis=0|1|2                 (run_cet_sublattice and the map drivers) the growth-axis elongation histogram
+                                     of every metrics row in outputs/<prefix>/grain_shape.csv
+                                     (cetkmc.grain_shape_group), and per map the columnar volume fraction of every
+                                     lattice (metrics.grain_shape_summary) in <map>_shape.csv
 """
 from __future__ import annotations
 
@@ -177,13 +181,14 @@ def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_
                             all_gather=all_gather)
 
 
-def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None):
+def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shape_axis=None):
     """_cadence for every case of a group at once (cetkmc.metrics_group, one launch per kernel for the group): the
     defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  The Philox
     stream is keyed by r["seed"] where a case has one, else by `seed`.  With NumPy's
     stream each case draws its mask from its own saved position (r["rng"]), in group order, as refresh_resident
     draws it.  profile_axis: one cetkmc.grain_profile_group call over the labelling the rows used appends each
-    case's (step, profile) to r["profiles"]."""
+    case's (step, profile) to r["profiles"]; shape_axis: one cetkmc.grain_shape_group call over that labelling appends
+    each case's (step, histogram) to r["shapes"]."""
     ctxs = [r["ctx"] for r in runs]
     refresh = last % every == 0
     draws = None
@@ -210,22 +215,27 @@ def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None):
     if profile_axis is not None:
         for r, prof in zip(runs, _lib.grain_profile_group(ctxs, profile_axis, constants.CET_AR_THRESHOLD)):
             r["profiles"].append((last, prof))
+    if shape_axis is not None:
+        for r, hist in zip(runs, _lib.grain_shape_group(ctxs, shape_axis)):
+            r["shapes"].append((last, hist))
 
 
 PROFILE_CSV = "cet_profile.csv"
+SHAPE_CSV = "grain_shape.csv"
 
 
-def _check_profile_axis(fn, profile_axis, world=1, checkpoint_every=0, resume_from=None):
-    """Refuse what a run with per-plane grain profiles does not take: an axis outside {0, 1, 2}, a lattice split into
-    slabs (their labels are slab-local) and checkpoints (they do not carry the profile history)."""
-    if profile_axis is None:
+def _check_axis_kw(fn, name, axis, world=1, checkpoint_every=0, resume_from=None):
+    """Refuse what a run with per-plane grain profiles (name "profile_axis") or grain-shape histograms ("shape_axis")
+    does not take: an axis outside {0, 1, 2}, a lattice split into slabs (their labels are slab-local) and checkpoints
+    (they do not carry the profile or shape history)."""
+    if axis is None:
         return
-    if isinstance(profile_axis, bool) or not isinstance(profile_axis, (int, np.integer)) or int(profile_axis) not in (0, 1, 2):
-        raise ValueError(f"{fn}: profile_axis must be None, 0, 1 or 2, got {profile_axis!r}")
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"{fn}: {name} must be None, 0, 1 or 2, got {axis!r}")
     if world > 1:
-        raise ValueError(f"{fn}: profile_axis needs a whole lattice on one GPU (world = 1)")
+        raise ValueError(f"{fn}: {name} needs a whole lattice on one GPU (world = 1)")
     if checkpoint_every or resume_from:
-        raise ValueError(f"{fn}: profile_axis does not take checkpoint_every or resume_from")
+        raise ValueError(f"{fn}: {name} does not take checkpoint_every or resume_from")
 
 
 def _check_mask_and_laser(fn, mask_stream, laser, thermal_every):
@@ -250,6 +260,36 @@ def _write_profile_csv(profiles, output_dir):
                 w.writerow([int(step), z] + [int(v) for v in prof[:, z]])
 
 
+def _write_shape_csv(shapes, output_dir, edges=_lib.SHAPE_EDGES):
+    """outputs/<prefix>/grain_shape.csv: one row per (metrics row, bin) of the (step, (2, len(edges) + 2) histogram)
+    pairs; bins 0..len(edges) with their edges Lo <= A < Hi, the small-grain bucket as Bin -1 with Lo and Hi empty."""
+    import csv
+    if not shapes:
+        return
+    e = [float(x) for x in edges]
+    lo, hi = [0.0] + e, e + [float("inf")]
+    with open(os.path.join(output_dir, SHAPE_CSV), "w", newline="") as fh:
+        w = csv.writer(fh)
+        w.writerow(("Step", "Bin", "Lo", "Hi", "Grains", "Sites"))
+        for step, hist in shapes:
+            for b in range(len(e) + 1):
+                w.writerow([int(step), b, repr(lo[b]), repr(hi[b]), int(hist[0, b]), int(hist[1, b])])
+            w.writerow([int(step), -1, "", "", int(hist[0, -1]), int(hist[1, -1])])
+
+
+def read_shape_csv(path):
+    """The last metrics row's histogram of a grain_shape.csv: (step, (2, n_edges + 2) int64 array, edges)."""
+    import csv
+    with open(path) as fh:
+        rows = list(csv.DictReader(fh))
+    step = rows[-1]["Step"]
+    last = [r for r in rows if r["Step"] == step]
+    binned = sorted((r for r in last if int(r["Bin"]) >= 0), key=lambda r: int(r["Bin"]))
+    small = [r for r in last if int(r["Bin"]) < 0]
+    hist = np.array([[int(r[c]) for r in binned + small] for c in ("Grains", "Sites")], np.int64)
+    return int(step), hist, tuple(float(r["Hi"]) for r in binned[:-1])
+
+
 def read_profile_csv(path):
     """The last metrics row's profile of a cet_profile.csv: (step, (4, L) int64 array)."""
     import csv
@@ -265,7 +305,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
                        output_prefix="cet_sublattice", metrics_every=None, events_per_sweep=None, p_max=0.1,
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
                        checkpoint_every=0, resume_from=None, lattice=None, verbose=True, rank=0, world=1,
-                       mask_stream="numpy", init_seed=None, profile_axis=None):
+                       mask_stream="numpy", init_seed=None, profile_axis=None, shape_axis=None):
     """run_kmc's large-lattice sibling.  Same set-up (initialize_lattice + introduce_defects with the
     run's seed), same cadence and CSV; the steps are synchronous-sublattice sweeps (csrc/sweep.cu), so
     `Step` counts sweeps and `Time` is the accumulated sweep interval.
@@ -282,6 +322,11 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
            columns Step, Plane, Solid, EquiaxedSolid, GrainsSpanning, EquiaxedGrainsSpanning, one row per (metrics
            row, plane).  Every other output is the same as without it.  Not with world > 1, checkpoint_every or
            resume_from.
+    shape_axis: None, or 0, 1 or 2: every metrics row also takes the growth-axis elongation histogram of the labelling
+           it used along that axis (cetkmc.grain_shape_group with its default edges and min_size), written to
+           outputs/<prefix>/grain_shape.csv with the columns Step, Bin, Lo, Hi, Grains, Sites, one row per (metrics
+           row, bin) and Bin -1 for the grains below min_size.  Every other output is the same as without it.  Not
+           with world > 1, checkpoint_every or resume_from.
     world > 1: the lattice is split into z-slabs, one per rank / GPU (launch every rank with the same
            arguments plus its rank; torch.distributed.run provides the rendezvous).  The trajectory and
            the CSV do not depend on the number of slabs.  Rank 0 writes the CSV; every rank returns its
@@ -299,7 +344,8 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     nu_dep = constants.NU_DEP if nu_dep is None else nu_dep
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
-    _check_profile_axis("run_cet_sublattice", profile_axis, world, checkpoint_every, resume_from)
+    _check_axis_kw("run_cet_sublattice", "profile_axis", profile_axis, world, checkpoint_every, resume_from)
+    _check_axis_kw("run_cet_sublattice", "shape_axis", shape_axis, world, checkpoint_every, resume_from)
     np.random.seed(seed)                                    # a resumed run restores the stream position below
     output_dir = f"outputs/{output_prefix}"
     os.makedirs(output_dir, exist_ok=True)
@@ -315,7 +361,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     ctx.init_seed = init_seed
     try:
         ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
-        sweep0, total_time, nucleation_count, cet_detected, rows, profiles = 0, 0.0, 0, False, [], []
+        sweep0, total_time, nucleation_count, cet_detected, rows, profiles, shapes = 0, 0.0, 0, False, [], [], []
         if resume_from:
             meta = resume(ctx, resume_from)
             sweep0, total_time = int(meta.get("sweep", 0)), float(meta.get("time", 0.0))
@@ -366,6 +412,8 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             rows.append(row)
             if profile_axis is not None:
                 profiles.append((sweep - 1, _lib.grain_profile_group([ctx], profile_axis, constants.CET_AR_THRESHOLD)[0]))
+            if shape_axis is not None:
+                shapes.append((sweep - 1, _lib.grain_shape_group([ctx], shape_axis)[0]))
             if checkpoint_every and (len(rows) % checkpoint_every == 0):
                 checkpoint(ctx, os.path.join(output_dir, "checkpoint"), sweep=sweep, time=total_time,
                            nucleation_count=nucleation_count, cet_detected=cet_detected,
@@ -373,6 +421,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
         if rank == 0:
             _ks._write_csv(rows, output_dir)
             _write_profile_csv(profiles, output_dir)
+            _write_shape_csv(shapes, output_dir)
         f = ctx.download(state=True, atom_type=True, theta=True, phi=True)
     finally:
         ctx.close()
@@ -414,7 +463,9 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
     (one row per (case, replica), the map's columns).  Returns (map rows, ensemble_stats rows; None when
     world > 1) instead of the map rows.  Not with `checkpoint_every`, `resume_from` or `lattice`.
     profile_axis=a (through **kw): every case writes outputs/<prefix>/cet_profile.csv (run_cet_sublattice), and each
-    rank writes cet_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it."""
+    rank writes cet_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it.
+    shape_axis=a (through **kw): every case writes outputs/<prefix>/grain_shape.csv (run_cet_sublattice), and each rank
+    writes cet_map_shape_rank<r>.csv (_map_shape_rows); every other file is the same as without it."""
     cases = [(float(t), float(r)) for t in temps for r in nu_deps]
 
     def case_row(q):
@@ -438,7 +489,8 @@ def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses
     world = int(os.environ.get("WORLD_SIZE", 1)) if world is None else world
     devices = [int(os.environ.get("LOCAL_RANK", 0))] if devices is None else list(devices)
     n_rep = _check_replicas(fn, replicas, kw)
-    _check_profile_axis(fn, kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
+    _check_axis_kw(fn, "profile_axis", kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
+    _check_axis_kw(fn, "shape_axis", kw.get("shape_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_mask_and_laser(fn, kw.get("mask_stream", "numpy"), lasers is not None or kw.get("laser"),
                           kw.get("thermal_every", _ks.THERMAL_EVERY))
     if batch is not None:
@@ -458,7 +510,7 @@ def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses
                                lasers=None if lasers is None else [lasers[lats[l][0]] for l in ls],
                                replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
     return _map_outputs(output_root, name, lats, [l for _d, ls in parts for l in ls], case_row, axes, replicas, rank,
-                        world, kw.get("profile_axis"))
+                        world, kw.get("profile_axis"), kw.get("shape_axis"))
 
 
 _MAP_FINAL = ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount",
@@ -493,11 +545,13 @@ def _replica_kw(kw, replicas, r):
     return dict(kw, seed=(constants.RANDOM_SEED if seed is None else int(seed)) + r, init_seed=42 + r)
 
 
-def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world, profile_axis=None):
+def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world, profile_axis=None,
+                 shape_axis=None):
     """The per-rank files of a map driver over the lattices `mine` (indices into `lats`) this rank ran:
     <name>_rank<rank>.csv (case, case_row(case), the final row's _MAP_FINAL columns) and the plot_cet tree from
-    replica 0 of each case, with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica), and with
-    profile_axis <name>_profile_rank<rank>.csv (_map_profile_rows).  Returns the map rows; with replicas (map rows,
+    replica 0 of each case, with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica), with
+    profile_axis <name>_profile_rank<rank>.csv (_map_profile_rows) and with shape_axis <name>_shape_rank<rank>.csv
+    (_map_shape_rows).  Returns the map rows; with replicas (map rows,
     ensemble_stats of the replica rows), the latter None when world > 1 (merge_* joins the ranks)."""
     import csv
     rows, rep_rows = [], []
@@ -514,6 +568,8 @@ def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, 
     if profile_axis is not None:
         _write_rows(_map_profile_rows(lats, sorted(mine), case_row, axes),
                     os.path.join(out_dir, f"{name}_profile_rank{rank}.csv"))
+    if shape_axis is not None:
+        _write_rows(_map_shape_rows(lats, sorted(mine), case_row, axes), os.path.join(out_dir, f"{name}_shape_rank{rank}.csv"))
     write_plot_cet_tree([(row["case"], f"outputs/{lats[l][2]}/metrics.csv")
                          for row, l in zip(rows, sorted(l for l in mine if lats[l][1] == 0))],
                         os.path.join(out_dir, "plot_cet"))
@@ -534,6 +590,42 @@ def _map_profile_rows(lats, mine, case_row, axes):
         c = case_row(q)
         out.append({"case": q, "replica": r, **{k: c[k] for k in axes}, "CET_Height": s["CET_Height"],
                     "Front_Height": s["Front_Height"]})
+    return out
+
+
+SHAPE_FRACTIONS = ("ColumnarVolumeFraction", "ColumnarGrainFraction")
+
+
+def _map_shape_rows(lats, mine, case_row, axes):
+    """One row per lattice of `mine` (case, replica, the map's axis columns, and ColumnarVolumeFraction,
+    ColumnarGrainFraction and ShapedGrains of metrics.grain_shape_summary over the final row's histogram in
+    outputs/<prefix>/grain_shape.csv)."""
+    out = []
+    for l in mine:
+        q, r, p = lats[l]
+        _step, hist, edges = read_shape_csv(f"outputs/{p}/{SHAPE_CSV}")
+        c = case_row(q)
+        out.append({"case": q, "replica": r, **{k: c[k] for k in axes}, **_metrics.grain_shape_summary(hist, edges)})
+    return out
+
+
+def shape_ensemble_stats(rows, axes):
+    """One row per case over the rows of a <map>_shape.csv (dicts with case, replica, the axis columns `axes` and
+    SHAPE_FRACTIONS; numbers or the strings a CSV gives back), in case order: case, the axes, replicas (n), and per
+    fraction <col>_mean and <col>_se (the sample standard deviation, ddof=1, over sqrt(n); empty for n = 1)."""
+    by_case = {}
+    for r in rows:
+        by_case.setdefault(int(r["case"]), []).append(r)
+    out = []
+    for case in sorted(by_case):
+        rs = by_case[case]
+        n = len(rs)
+        e = {"case": case, **{k: rs[0][k] for k in axes}, "replicas": n}
+        for col in SHAPE_FRACTIONS:
+            v = np.array([float(r[col]) for r in rs])
+            e[f"{col}_mean"] = float(np.mean(v))
+            e[f"{col}_se"] = float(np.std(v, ddof=1) / np.sqrt(n)) if n > 1 else ""
+        out.append(e)
     return out
 
 
@@ -586,7 +678,7 @@ def ensemble_stats(rows, axes):
 
 def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
                        events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy",
-                       lasers=None, replicas=None, profile_axis=None):
+                       lasers=None, replicas=None, profile_axis=None, shape_axis=None):
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
@@ -600,9 +692,12 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     init_seed=42 + r).  The generated initial lattices of the group are built on the device by one cetkmc.init_group
     call (_upload_initial).
     profile_axis: every metrics row also takes its cases' grain profiles with one cetkmc.grain_profile_group call
-    (_cadence_group), and each case writes the cet_profile.csv run_cet_sublattice(profile_axis=...) writes."""
+    (_cadence_group), and each case writes the cet_profile.csv run_cet_sublattice(profile_axis=...) writes.
+    shape_axis: the same with one cetkmc.grain_shape_group call per row, and the grain_shape.csv of
+    run_cet_sublattice(shape_axis=...)."""
     _check_mask_and_laser("_run_cases_grouped", mask_stream, lasers is not None, thermal_every)
-    _check_profile_axis("_run_cases_grouped", profile_axis)
+    _check_axis_kw("_run_cases_grouped", "profile_axis", profile_axis)
+    _check_axis_kw("_run_cases_grouped", "shape_axis", shape_axis)
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
     philox_mask = mask_stream == "philox"
@@ -616,7 +711,7 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
             ctx = _lib.Context(L=L, device=device)
             ctx.init_seed = None if replicas is None else 42 + reps[q]
             ctx.init_nuclei = []
-            r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], profiles=[], total_time=0.0,
+            r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], profiles=[], shapes=[], total_time=0.0,
                      nucleation_count=0, cet_detected=False, terminated=False)
             runs.append(r)
             ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
@@ -648,13 +743,14 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
                 sweep += blk
                 stopped = [r for r in active if r["terminated"]]
                 if stopped:
-                    _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis)
+                    _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis)
                     active = [r for r in active if not r["terminated"]]
             if active:
-                _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis)
+                _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis)
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
             _write_profile_csv(r["profiles"], f"outputs/{r['prefix']}")
+            _write_shape_csv(r["shapes"], f"outputs/{r['prefix']}")
     finally:
         for r in runs:
             r["ctx"].close()
@@ -706,7 +802,9 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     per (case, replica), the map's columns).  Returns (map rows, ensemble_stats rows; None when world > 1).
     Not with `checkpoint_every`, `resume_from` or `lattice`.
     profile_axis=a (through **kw): every case writes outputs/<prefix>/cet_profile.csv (run_cet_sublattice), and each
-    rank writes melt_pool_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it."""
+    rank writes melt_pool_map_profile_rank<r>.csv (_map_profile_rows); every other file is the same as without it.
+    shape_axis=a (through **kw): every case writes outputs/<prefix>/grain_shape.csv (run_cet_sublattice), and each rank
+    writes melt_pool_map_shape_rank<r>.csv (_map_shape_rows); every other file is the same as without it."""
     powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
     if not powers or not speeds:
         raise ValueError("run_melt_pool_map: needs at least one power and one speed")
@@ -776,6 +874,9 @@ def _merge_map(output_root, name, axes):
     prof = _merge_rank_files(output_root, f"{name}_profile")
     if prof and reps:
         _write_rows(profile_ensemble_stats(prof, axes), f"outputs/{output_root}/{name}_profile_ensemble.csv")
+    shape = _merge_rank_files(output_root, f"{name}_shape")
+    if shape and reps:
+        _write_rows(shape_ensemble_stats(shape, axes), f"outputs/{output_root}/{name}_shape_ensemble.csv")
     return rows
 
 
@@ -783,12 +884,14 @@ def merge_cet_map(output_root="gr_sweep"):
     """Join the per-rank files of run_gr_sweep into outputs/<output_root>/cet_map.csv (sorted by case); after a run
     with replicas also cet_map_replicas.csv and cet_map_ensemble.csv (ensemble_stats, one row per case); after a run
     with profile_axis also cet_map_profile.csv (sorted by case and replica), and with replicas
-    cet_map_profile_ensemble.csv (profile_ensemble_stats)."""
+    cet_map_profile_ensemble.csv (profile_ensemble_stats); after a run with shape_axis also cet_map_shape.csv and, with
+    replicas, cet_map_shape_ensemble.csv (shape_ensemble_stats)."""
     return _merge_map(output_root, "cet_map", ("T_sub", "NU_DEP"))
 
 
 def merge_melt_pool_map(output_root="melt_pool_map"):
     """Join the per-rank files of run_melt_pool_map into outputs/<output_root>/melt_pool_map.csv (sorted by case);
     after a run with replicas also melt_pool_map_replicas.csv and melt_pool_map_ensemble.csv (ensemble_stats); after
-    a run with profile_axis also melt_pool_map_profile.csv and, with replicas, melt_pool_map_profile_ensemble.csv."""
+    a run with profile_axis also melt_pool_map_profile.csv and, with replicas, melt_pool_map_profile_ensemble.csv;
+    after a run with shape_axis also melt_pool_map_shape.csv and, with replicas, melt_pool_map_shape_ensemble.csv."""
     return _merge_map(output_root, "melt_pool_map", ("power", "speed", "T_sub", "NU_DEP"))

@@ -178,6 +178,10 @@ struct cet_ctx {
     cudaEvent_t ev_group = nullptr;   // orders this context's stream before the work of a group led by another context
     void *profile_tab = nullptr;      // grain-profile tables and span differences of the groups this context leads, grow-only
     size_t cap_profile_tab = 0;
+    void *grain_mom = nullptr;        // per-grain moments of cet_grain_shape_group (grain_shape.cuh), at gid, grow-only
+    size_t cap_grain_mom = 0;
+    void *shape_tab = nullptr;        // grain-shape histograms of the groups this context leads, grow-only
+    size_t cap_shape_tab = 0;
 
     // per-kernel-kind device timing (cet_profile_*): event pairs recorded around the dominant
     // kernels on the context stream, resolved when the totals are read

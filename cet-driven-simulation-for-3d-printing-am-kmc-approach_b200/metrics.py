@@ -175,6 +175,30 @@ def cet_profile_summary(profile, plane_sites, eq_threshold=K.CET_EQ_THRESHOLD, m
     return {"CET_Height": cet, "Front_Height": int(planes[-1])}
 
 
+def grain_shape_summary(hist, edges, threshold=K.CET_AR_THRESHOLD):
+    """How columnar a lattice is, from one (2, len(edges) + 2) grain-shape histogram of cetkmc.grain_shape_group (row
+    0 grains, row 1 sites; bins 0..len(edges) by growth-axis elongation A, the last bin the grains below min_size).
+    `threshold` must be one of `edges`, so that a bin lies wholly on one side of it; a grain is columnar when
+    A >= threshold.
+        ColumnarVolumeFraction  sites of columnar grains / all occupied sites (small grains included); 0.0 when the
+                                lattice has none
+        ColumnarGrainFraction   columnar grains / grains of >= min_size sites; 0.0 when there are none
+        ShapedGrains            grains of >= min_size sites"""
+    e = [float(x) for x in edges]
+    h = np.asarray(hist)
+    if h.ndim != 2 or h.shape != (2, len(e) + 2):
+        raise ValueError(f"grain_shape_summary: need a (2, {len(e) + 2}) histogram, got shape {h.shape}")
+    if float(threshold) not in e:
+        raise ValueError(f"grain_shape_summary: threshold {threshold!r} must be one of the edges {tuple(e)}")
+    first = e.index(float(threshold)) + 1                       # bin b >= first: A >= edges[b - 1] >= threshold
+    grains, sites = h[0].astype(np.int64), h[1].astype(np.int64)
+    shaped = int(grains[:len(e) + 1].sum())
+    col_sites, col_grains, all_sites = int(sites[first:len(e) + 1].sum()), int(grains[first:len(e) + 1].sum()), int(sites.sum())
+    return {"ColumnarVolumeFraction": col_sites / all_sites if all_sites else 0.0,
+            "ColumnarGrainFraction": col_grains / shaped if shaped else 0.0,
+            "ShapedGrains": shaped}
+
+
 def grains_distributed(ctx, all_gather, theta_threshold=0.5):
     """Grains of a lattice that is split into z-slabs over several contexts (one per rank), in the form
     Context.grains() returns for a whole lattice — the reference's clusters (utils.py:28-84) in its

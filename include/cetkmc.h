@@ -316,6 +316,29 @@ int cet_metrics_group(cet_ctx *const *ctxs, int32_t n_ctx, const cet_metrics_par
  * they were.  The work is ordered on the stream of ctxs[0] after the work already queued on every context's
  * stream: one memset, five launches for the whole group, one D2H copy of the table, one host synchronisation. */
 int cet_grain_profile_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, double ar_threshold, int64_t *out);
+/* ---- grain elongation along a growth axis of a group (volume-weighted columnar fraction) ----
+ * Histogram of the growth-axis elongation A of every grain of the last grain labelling (cet_grains_label[_ex] or
+ * cet_metrics_group) of each context.  A grain of n sites at coordinates c = (i, j, k) has per axis x the exact sums
+ * S_x = sum c_x, S_xx = sum c_x^2 and Q_x = 12 (n S_xx - S_x^2) + n^2 (n^2 times 12 (variance along x + 1/12), each
+ * site a unit cube); along growth axis `axis` = a with b, c the other two axes,
+ *     A = sqrt(fl(2 Q_a) / fl(Q_b + Q_c)),
+ * fl() the round-to-nearest-even conversion of the exact integer to fp64, the division and square root IEEE round to
+ * nearest.  A single site has A = 1, a 1 x 1 x h column along a has A = h, an a x b x c box sqrt(2a^2 / (b^2 + c^2)).
+ * Unlike the bounding-box aspect ratio, A is directional, weighs every site, and sees a sparse grain as sparse.
+ * out[(q * 2 + f) * (n_edges + 2) + b], int64, for context q: f = 0 the number of grains, f = 1 their total sites, in
+ *   bin b (0 <= b <= n_edges): grains of >= min_size sites with e_{b-1} <= A < e_b (e_{-1} = 0, e_{n_edges} = inf);
+ *   bin n_edges + 1: every grain of fewer than min_size sites.
+ * So the sites of a lattice sum to its occupied sites and the grains to its grain count.  edges: n_edges values, 1 <=
+ * n_edges <= 62, finite, > 0 and strictly ascending; min_size >= 1; axis 0, 1 or 2.
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device, 1 <= n_ctx <= 64,
+ * each with a labelling of the whole lattice (a context never labelled is rejected).  The call does not relabel; it
+ * is read-only on the lattice, the labels and the mask, so the next metrics row, profile and sweeps are what they
+ * would have been without it.  Everything, `out` included, is checked before anything is launched or written: a
+ * rejected call leaves every context and `out` as they were.  The work is ordered on the stream of ctxs[0] after the
+ * work already queued on every context's stream: one memset, three launches for the whole group, one D2H copy of the
+ * table, one host synchronisation. */
+int cet_grain_shape_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, const double *edges, int32_t n_edges,
+                          int64_t min_size, int64_t *out);
 /* The same for global planes [i_lo, i_hi) within the labelled planes of a slab (owned + 2 ghost planes per
  * cut face): what two neighbouring slabs compare to join the grains that cross their cut. */
 int cet_grains_download_planes(cet_ctx *ctx, int64_t i_lo, int64_t i_hi, int32_t *labels);

@@ -253,11 +253,12 @@ int cet_destroy(cet_ctx *c)
     void *ptrs[] = {c->vox, c->vox_prev, c->theta, c->phi, c->v, c->nst, c->T, c->T2, c->site_rate, c->dep_rate,
                     c->row_occ, c->row_emp, c->row_dep, c->row_depcnt, c->seg, c->total, c->q_top,
                     c->stage, c->kmc, c->d_py, c->d_np, c->d_sp, c->d_log, c->sweep, c->claim,
-                    c->records, c->blk_sum, c->blk_max, c->plane_sum, c->stamp, c->dirty, c->fired,
+                    c->records, c->blk_sum, c->blk_max, c->plane_sum, c->stamp, c->t_changed, c->dirty, c->fired,
                     c->grain_label, c->grain_gid, c->grain_st, c->group_tab, c->profile_tab, c->grain_mom, c->shape_tab, c->rate_tab, c->cvox, c->pairop, c->tile_flag,
                     c->delta_send[0], c->delta_send[1], c->delta_recv[0], c->delta_recv[1]};
     for (void *p : ptrs)
         if (p) cudaFree(p);
+    if (c->t_count_host) cudaFreeHost(c->t_count_host);
     for (auto &sp : c->prof_spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
     for (auto e : c->prof_pool) cudaEventDestroy(e);
     if (c->ev0) cudaEventDestroy(c->ev0);

@@ -58,7 +58,8 @@ struct SweepState {
     unsigned int n_fired;                           // fired-site list length of the current sweep
     unsigned int n_dirty, n_dirty_emp;              // refresh list length (one mixed list; n_dirty_emp stays 0, kept for the layout)
     unsigned int overflow, dirty_overflow, pad0_;   // the fired list overflowed (events dropped)
-    unsigned int pad_line1_[26];
+    unsigned int n_t_changed, n_t_stale;            // thermal step: sites whose T changed, sites whose rates that made stale
+    unsigned int pad_line1_[24];
     // line 2 — written by the single-CTA finalize kernel only
     double sum_rate, max_rate;                      // totals of the rates seen by the last sweep
     double tau, time;                               // interval of the next sweep; accumulated time
@@ -147,6 +148,8 @@ struct cet_ctx {
     void *records = nullptr;
     size_t cap_records = 0;
     int64_t sweep_index = 0;
+    uint32_t *t_changed = nullptr;    // sites whose T the last thermal step of a sweep changed, one bit per local site
+    unsigned int *t_count_host = nullptr;   // pinned: the thermal step's counts (SweepState n_t_changed, n_t_stale)
     int64_t last_thermal_index = -1;  // sweep index whose thermal step has already run (priming pass)
     double *blk_sum = nullptr, *blk_max = nullptr, *plane_sum = nullptr;
     int64_t n_blk = 0;

@@ -22,8 +22,8 @@
 //           arithmetic, so the resident rates stay bit-identical to a full rebuild);
 //   tau     for the next sweep from the totals of this one:
 //           tau = min(events_per_sweep / R_total, -ln(1-p_max) / R_max).
-// A thermal step (every thermal_every sweeps) changes every rate: it is followed by a dense
-// rebuild (rates_rows).
+// A thermal step (every thermal_every sweeps) is followed by a refresh of the rates that read a
+// changed temperature (thermal_refresh) or, when those are many, by a dense rebuild.
 // Slabs: a context with halo H >= 6 evaluates ghost sites to depth 4 and resolves claims to
 // depth 2, which is everything that can write an owned site; after the one halo exchange per
 // sweep (comm.cu) the rates of the evaluated ghost planes and of the two outermost owned planes
@@ -40,6 +40,8 @@
 namespace cet {
 
 int thermal_cet_step(cet_ctx *c, const cet_thermal_params *p, const int32_t *stop_flag);
+int thermal_cet_step_tracked(cet_ctx *c, const cet_thermal_params *p, const int32_t *stop_flag, uint32_t *changed,
+                             unsigned int *n_changed);
 int rates_rows(cet_ctx *c, int p_lo, int p_hi);                                  // rates.cu
 int rates_rows_dirty(cet_ctx *c, int p_lo, int p_hi, const uint32_t *stamp, int32_t *list, unsigned int *counter);
 int comm_sweep_reduce(cet_ctx *c, double *plane_sum, int n, double *max_inout);   // comm.cu
@@ -796,6 +798,69 @@ static int refresh_tiled(cet_ctx *c, const SlabRanges &R)
     return rates_rows_dirty_compact(c, R.eval_lo, R.eval_hi, c->stamp, c->dirty, &c->sweep->n_dirty);
 }
 
+// ---- after a thermal step: refresh only the rates whose temperatures changed -------------------------
+// A site's rates read T at the site itself, at its k +- 1 neighbours (grad_z of an empty site) and at its empty
+// neighbours among the 14 (the diffusion / attachment pair operand is then pairop = T).  The offsets are symmetric,
+// so a changed site x makes stale x, x +- 1 and x +- 2 in k, x + (0, +-1, +-1) and x + (+-1, +-1, 0), x + (+-2, 0, 0)
+// and x + (0, +-2, 0).  One thread per stamp word: the OR of the changed bitmap's words at those row offsets, shifted
+// by dk within the row (rows start on word boundaries: L % 32 == 0; rows outside the lattice contribute nothing).
+// Every word of the stamp bitmap is written; the stale sites are counted.
+__device__ __forceinline__ uint32_t kshift1(uint32_t w, uint32_t l, uint32_t r) { return (w >> 1 | r << 31) | (w << 1 | l >> 31); }
+__device__ __forceinline__ uint32_t kshift2(uint32_t w, uint32_t l, uint32_t r) { return (w >> 2 | r << 30) | (w << 2 | l >> 30); }
+
+__global__ void __launch_bounds__(256) thermal_stale_kernel(const uint32_t *__restrict__ chg, uint32_t *__restrict__ stamp, int L,
+                                                            int n0, int n_words, unsigned int *n_stale)
+{
+    const int wpr = L >> 5;                                       // words per row
+    unsigned cnt = 0;
+    for (int w = blockIdx.x * blockDim.x + threadIdx.x; w < n_words; w += gridDim.x * blockDim.x) {
+        const int r = w / wpr, kw = w - r * wpr;                  // row (plane * L + j), word within the row
+        const int p = r / L, j = r - p * L;
+        auto at = [&](int dp, int dj, int dw) -> uint32_t {
+            const int pp = p + dp, jj = j + dj, ww = kw + dw;
+            if (pp < 0 || pp >= n0 || jj < 0 || jj >= L || ww < 0 || ww >= wpr) return 0u;
+            return chg[((int64_t)pp * L + jj) * wpr + ww];
+        };
+        const uint32_t c = at(0, 0, 0);
+        uint32_t s = c | kshift1(c, at(0, 0, -1), at(0, 0, 1)) | kshift2(c, at(0, 0, -1), at(0, 0, 1));
+#pragma unroll
+        for (int dj = -1; dj <= 1; dj += 2) s |= kshift1(at(0, dj, 0), at(0, dj, -1), at(0, dj, 1));
+        s |= at(1, 1, 0) | at(1, -1, 0) | at(-1, 1, 0) | at(-1, -1, 0) | at(2, 0, 0) | at(-2, 0, 0) | at(0, 2, 0) | at(0, -2, 0);
+        stamp[w] = s;
+        cnt += __popc(s);
+    }
+    cnt = __reduce_add_sync(0xffffffffu, cnt);                   // one counter update per warp
+    if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(n_stale, cnt);
+}
+
+// Above this many stale sites the dense rebuild is the faster side.  Measured at 512^3 on a B200 (1000 W, 1965 MHz;
+// scripts/bench_thermal_refresh.py, profiles/thermal_refresh.json): the sweep holding the thermal step took 1.02 /
+// 1.21 / 1.49 / 2.06 / 2.63 ms on the refresh side at 1.6 / 5 / 10 / 20 / 30 % of the sites stale, about 5.8 ms
+// per unit of stale fraction, against 3.07-3.19 ms on the dense side, so the two meet near 40 %.  Both sides give
+// the same bits: the choice only costs time.
+static int64_t thermal_refresh_max(const cet_ctx *c) { return c->nloc / 8 * 3; }
+
+// The rates after a thermal step of the solo tiled path: the stencil has kept pairop (ThermalTrack); when the rates
+// were valid before it and L % 32 == 0 it has also marked its changed sites, and only the rates that read a changed
+// temperature are refreshed.  One host read of the counts per thermal step.  *done: the rates are current.
+static int thermal_refresh(cet_ctx *c, const SlabRanges &R, bool *done)
+{
+    *done = false;
+    ProfScope ps(c, PROF_REFRESH);
+    const int n_words = (int)(c->nloc >> 5);
+    thermal_stale_kernel<<<(int)std::min<int64_t>((n_words + 255) / 256, (int64_t)sm_count(c) * 8), 256, 0, c->stream>>>(
+        c->t_changed, c->stamp, (int)c->n1, (int)c->n0, n_words, &c->sweep->n_t_stale);
+    CET_CUDA(cudaGetLastError());
+    CET_CUDA(cudaMemcpyAsync(c->t_count_host, &c->sweep->n_t_changed, 2 * sizeof(unsigned int), cudaMemcpyDeviceToHost, c->stream));
+    CET_CUDA(cudaStreamSynchronize(c->stream));
+    if (c->t_count_host[0] == 0) { *done = true; return 0; }      // no temperature changed: every rate still holds
+    if ((int64_t)c->t_count_host[1] > thermal_refresh_max(c)) return 0;
+    CET_CUDA(cudaMemsetAsync(&c->sweep->n_dirty, 0, sizeof(unsigned int), c->stream));   // sweep_reset_kernel clears it again
+    if (int rc = rates_rows_dirty_compact(c, R.eval_lo, R.eval_hi, c->stamp, c->dirty, &c->sweep->n_dirty)) return rc;
+    *done = true;
+    return 0;
+}
+
 // One sweep.  tiled: the rate sums are kept current by the TMA tile kernel (sweep_tile.cu), which needs
 // the orientation invariant of tile_state.cuh; otherwise by the gather kernels of the first design
 // (stamp scan + list-driven re-evaluation, rates.cu).  Stream, pick and apply are the same either
@@ -806,10 +871,27 @@ static int refresh_tiled(cet_ctx *c, const SlabRanges &R)
 static int sweep_prepare(cet_ctx *c, const cet_sweep_params *sp, const cet_thermal_params *tp, const SlabRanges &R, bool tiled)
 {
     if (sp->thermal_every > 0 && c->sweep_index % sp->thermal_every == 0 && c->last_thermal_index != c->sweep_index) {
-        if (int rc = thermal_cet_step(c, tp, &c->sweep->terminated)) return rc;      // clears sweep_rates_valid
-        if (c->world > 1) if (int rc = comm_halo_exchange(c, 4)) return rc;
-        if (tiled) if (int rc = tile_pairop_T_update(c)) return rc;
+        // solo tiled path: the stencil keeps pairop itself (ThermalTrack); slabs run tile_pairop_T after the exchange
+        const bool solo = tiled && c->world == 1 && c->halo == 0 && c->tile_valid;
+        // the incremental refresh needs rates that were current before the stencil, the bitmap (L % 32 == 0), and the
+        // default rebuild (debug flags 8 / 32 / 65536 / 131072 select another rebuild kernel; 524288 forces the dense side)
+        const bool incremental = solo && c->sweep_rates_valid && c->t_changed && c->t_count_host &&
+                                 !(c->debug_flags & (8 | 32 | 65536 | 131072 | 524288));
+        if (solo) {
+            if (incremental) CET_CUDA(cudaMemsetAsync(&c->sweep->n_t_changed, 0, 2 * sizeof(unsigned int), c->stream));
+            if (int rc = thermal_cet_step_tracked(c, tp, &c->sweep->terminated, incremental ? c->t_changed : nullptr,
+                                                  &c->sweep->n_t_changed)) return rc;    // clears sweep_rates_valid
+        } else {
+            if (int rc = thermal_cet_step(c, tp, &c->sweep->terminated)) return rc;      // clears sweep_rates_valid
+            if (c->world > 1) if (int rc = comm_halo_exchange(c, 4)) return rc;
+            if (tiled) if (int rc = tile_pairop_T_update(c)) return rc;
+        }
         c->last_thermal_index = c->sweep_index;
+        if (incremental) {
+            bool done = false;
+            if (int rc = thermal_refresh(c, R, &done)) return rc;
+            c->sweep_rates_valid = done;
+        }
     }
     if (!c->sweep_rates_valid) {                     // new lattice, new T or new parameters: dense rebuild
         if (tiled && !(c->debug_flags & 8)) {
@@ -1040,6 +1122,11 @@ extern "C" int cet_sweep_run(cet_ctx *c, int64_t n_sweeps, const cet_sweep_param
         if (int rc = rate_tables_ensure(c)) return rc;      // the pick kernel reads the K_eff / E_tot tables
         c->nst_valid = false;                // the tile path keeps no neighbour cache
         if (c->world > 1) if (int rc = comm_delta_alloc(c)) return rc;
+        // the changed-site bitmap and the count buffer of the thermal refresh (sweep_prepare), outside the sweep loop
+        if (c->world == 1 && c->halo == 0 && c->n1 % 32 == 0 && sp->thermal_every > 0 && n_sweeps > 0) {
+            if (!c->t_changed) CET_CUDA(cudaMalloc(&c->t_changed, (size_t)c->nloc / 8));
+            if (!c->t_count_host) CET_CUDA(cudaMallocHost(&c->t_count_host, 2 * sizeof(unsigned int)));
+        }
     } else {
         c->tile_valid = false;               // the gather path's apply does not maintain cvox / pairop
         if (int rc = nst_ensure(c)) return rc;

@@ -65,11 +65,25 @@ __device__ __forceinline__ void thermal_fuse_site(const ThermalArgs &a, const Th
     if (x->cvox && (x->cvox[s] & 15u) == TC_EMPTY) x->pairop[s] = v;
 }
 
+// What cet_sweep_run fuses into update_temperature_cet on a whole-lattice context whose tile state is valid: a site
+// is *changed* when its new temperature differs in bit pattern from the value read (a NaN that nan_to_num replaced
+// counts).  A changed empty site's pair operand takes its new temperature: pairop == T held on every empty site
+// before the step, so pairop ends as tile_pairop_T would leave it.  With a bitmap (n2 % 32 == 0, the vector kernel
+// only) every word of it is written, one bit per local site, and the changed sites are counted.
+struct ThermalTrack {
+    const uint8_t *cvox;
+    double *pairop;
+    uint32_t *changed;               // NULL: no bitmap, no count
+    unsigned int *n_changed;
+};
+
 // The kernel bodies take their arguments by reference and the plane block `zb` (blockIdx.z of a solo launch): the
 // grouped launches of cet_sweep_run_group and cet_thermal_full_group run them for the table entry of their lattice.
 // FUSE (full variant, whole-lattice contexts, no stop flag): x holds the fused writes of ThermalFuse.
-template <bool FULL, bool FUSE = false>
-__device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb, const ThermalFuse *x = nullptr)
+// TRACK (CET variant): t holds the pair-operand writes of ThermalTrack (the scalar kernel keeps no bitmap).
+template <bool FULL, bool FUSE = false, bool TRACK = false>
+__device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb, const ThermalFuse *x = nullptr,
+                                             const ThermalTrack *t = nullptr)
 {
     const int k = blockIdx.x * TH_TK + threadIdx.x;
     const int j = blockIdx.y * TH_TJ + threadIdx.y;
@@ -120,12 +134,20 @@ __device__ __forceinline__ void thermal_body(const ThermalArgs &a, int zb, const
         if (v > a.hi) v = a.hi;
         a.Tout[(int64_t)p * plane + (int64_t)j * a.n2 + k] = v;
         if constexpr (FUSE) thermal_fuse_site(a, x, (int64_t)p * plane + (int64_t)j * a.n2 + k, v);
+        if constexpr (TRACK) {
+            const int64_t s = (int64_t)p * plane + (int64_t)j * a.n2 + k;
+            if (__double_as_longlong(v) != __double_as_longlong(a.Tin[s]) && (t->cvox[s] & 15u) == TC_EMPTY) t->pairop[s] = v;
+        }
         below = centre;
         centre = above;
     }
 }
 template <bool FULL>
 __global__ void __launch_bounds__(TH_TK *TH_TJ) thermal_kernel(ThermalArgs a) { thermal_body<FULL>(a, blockIdx.z); }
+__global__ void __launch_bounds__(TH_TK *TH_TJ) thermal_track_kernel(ThermalArgs a, const ThermalTrack t)
+{
+    thermal_body<false, false, true>(a, blockIdx.z, nullptr, &t);
+}
 
 // Fast path (n2 a multiple of V = 2 or 4): V consecutive k per thread with 16-byte loads/stores,
 // the k-neighbours exchanged by warp shuffles, the i-neighbours kept in a register queue while
@@ -152,8 +174,9 @@ struct RowVec {
     }
 };
 
-template <bool FULL, bool NANFIX, int V, bool FUSE = false>
-__device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb, const ThermalFuse *x = nullptr)
+template <bool FULL, bool NANFIX, int V, bool FUSE = false, bool TRACK = false>
+__device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb, const ThermalFuse *x = nullptr,
+                                                const ThermalTrack *t = nullptr)
 {
     const int lane = threadIdx.x;
     const int k0 = (blockIdx.x * 32 + lane) * V;
@@ -173,6 +196,7 @@ __device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb, con
     double *po = a.Tout + (int64_t)p0 * plane + (int64_t)j * a.n2 + kc;
     int gi = a.i_off + p0;
     RowVec<V, NANFIX> below, centre, above, l1, r1;
+    unsigned n_chg = 0;                                      // TRACK: changed sites seen by this lane
     below.load(gi > 0 ? pc - plane : pc, a.nan_value);
     centre.load(pc, a.nan_value);
     for (int p = p0; p < p1; ++p, ++gi) {
@@ -231,13 +255,49 @@ __device__ __forceinline__ void thermal_v2_body(const ThermalArgs a, int zb, con
                 for (int e = 0; e < V; ++e) thermal_fuse_site(a, x, (int64_t)p * plane + (int64_t)j * a.n2 + kc + e, out[e]);
             }
         }
+        if constexpr (TRACK) {
+            unsigned nib = 0;                                 // bit e: site kc + e changed (never on the stop path)
+#pragma unroll
+            for (int e = 0; e < V; ++e) {
+                const double raw = NANFIX ? pc[e] : centre.v[e];
+                if (__double_as_longlong(out[e]) != __double_as_longlong(raw)) nib |= 1u << e;
+            }
+            if (!in || stop) nib = 0;
+            if (nib) {
+                const int64_t s = (int64_t)p * plane + (int64_t)j * a.n2 + kc;
+#pragma unroll
+                for (int e = 0; e < V; ++e)
+                    if ((nib >> e & 1u) && (t->cvox[s + e] & 15u) == TC_EMPTY) t->pairop[s + e] = out[e];
+            }
+            if constexpr (V == 4) {
+                if (t->changed) {                             // n2 % 32 == 0: 8 lanes make one word of one row
+                    uint32_t word = nib << (4 * (lane & 7));
+                    word |= __shfl_xor_sync(0xffffffffu, word, 1);
+                    word |= __shfl_xor_sync(0xffffffffu, word, 2);
+                    word |= __shfl_xor_sync(0xffffffffu, word, 4);
+                    if (in && (lane & 7) == 0) t->changed[((int64_t)p * plane + (int64_t)j * a.n2 + k0) >> 5] = word;
+                    n_chg += __popc(nib);
+                }
+            }
+        }
         below = centre;
         centre = above;
         pc += plane; pm += plane; pp += plane; po += plane;
     }
+    if constexpr (TRACK && V == 4) {
+        if (t->changed) {                                     // one counter update per warp
+            n_chg = __reduce_add_sync(0xffffffffu, n_chg);
+            if (lane == 0 && n_chg) atomicAdd(t->n_changed, n_chg);
+        }
+    }
 }
 template <bool FULL, bool NANFIX, int V>
 __global__ void __launch_bounds__(32 * TH2_TJ) thermal_kernel_v2(const ThermalArgs a) { thermal_v2_body<FULL, NANFIX, V>(a, blockIdx.z); }
+template <bool NANFIX, int V>
+__global__ void __launch_bounds__(32 * TH2_TJ) thermal_track_kernel_v2(const ThermalArgs a, const ThermalTrack t)
+{
+    thermal_v2_body<false, NANFIX, V, false, true>(a, blockIdx.z, nullptr, &t);
+}
 
 // Grouped update_temperature_cet (cet_sweep_run_group): blockIdx.z = lattice * nzb + plane block.  V = 0: the
 // scalar kernel (odd n2).
@@ -287,8 +347,9 @@ static void thermal_done(cet_ctx *c, const ThermalArgs &a, bool full)
     c->rates_valid = false; c->sweep_rates_valid = false;
 }
 
+// track (CET variant only): the stencil's ThermalTrack writes (NULL: none)
 template <bool FULL>
-static int launch_thermal(cet_ctx *c, ThermalArgs &a)
+static int launch_thermal(cet_ctx *c, ThermalArgs &a, const ThermalTrack *track = nullptr)
 {
     thermal_geometry(c, a);
     if (a.p_hi <= a.p_lo) return 0;
@@ -301,7 +362,15 @@ static int launch_thermal(cet_ctx *c, ThermalArgs &a)
         dim3 grid((unsigned)((c->n2 / V + 31) / 32), (unsigned)((c->n1 + TH2_TJ - 1) / TH2_TJ),
                   (unsigned)((a.p_hi - a.p_lo + TH2_PLANES - 1) / TH2_PLANES));
         ProfScope ps(c, PROF_THERMAL);
-        if (V == 4) {
+        if (!FULL && track) {
+            if (V == 4) {
+                if (nanfix) thermal_track_kernel_v2<true, 4><<<grid, block, 0, c->stream>>>(a, *track);
+                else thermal_track_kernel_v2<false, 4><<<grid, block, 0, c->stream>>>(a, *track);
+            } else {
+                if (nanfix) thermal_track_kernel_v2<true, 2><<<grid, block, 0, c->stream>>>(a, *track);
+                else thermal_track_kernel_v2<false, 2><<<grid, block, 0, c->stream>>>(a, *track);
+            }
+        } else if (V == 4) {
             if (nanfix) thermal_kernel_v2<FULL, true, 4><<<grid, block, 0, c->stream>>>(a);
             else thermal_kernel_v2<FULL, false, 4><<<grid, block, 0, c->stream>>>(a);
         } else {
@@ -313,7 +382,8 @@ static int launch_thermal(cet_ctx *c, ThermalArgs &a)
         dim3 grid((unsigned)((c->n2 + TH_TK - 1) / TH_TK), (unsigned)((c->n1 + TH_TJ - 1) / TH_TJ),
                   (unsigned)((a.p_hi - a.p_lo + TH_PLANES - 1) / TH_PLANES));
         ProfScope ps(c, PROF_THERMAL);
-        thermal_kernel<FULL><<<grid, block, 0, c->stream>>>(a);
+        if (!FULL && track) thermal_track_kernel<<<grid, block, 0, c->stream>>>(a, *track);
+        else thermal_kernel<FULL><<<grid, block, 0, c->stream>>>(a);
     }
     CET_CUDA(cudaGetLastError());
     // planes outside [p_lo, p_hi) keep their previous contents: copy them so that the swap
@@ -343,6 +413,20 @@ int thermal_cet_step(cet_ctx *c, const cet_thermal_params *p, const int32_t *sto
 {
     ThermalArgs a = cet_step_args(p, stop_flag);
     return launch_thermal<false>(c, a);
+}
+
+// thermal_cet_step of a whole-lattice context with a valid tile state (cet_sweep_run): the stencil also keeps
+// pairop == T on the empty sites (ThermalTrack), so tile_pairop_T_update is not needed.  changed (n2 % 32 == 0, else
+// NULL): the bitmap of the changed sites, every word written; n_changed, which the caller has zeroed, gains their
+// number.
+int thermal_cet_step_tracked(cet_ctx *c, const cet_thermal_params *p, const int32_t *stop_flag, uint32_t *changed,
+                             unsigned int *n_changed)
+{
+    CET_REQUIRE(c->world == 1 && c->halo == 0 && c->tile_valid, "thermal_cet_step_tracked: whole-lattice context with a valid tile state");
+    CET_REQUIRE(!changed || c->n2 % 32 == 0, "thermal_cet_step_tracked: the changed bitmap needs n2 %% 32 == 0");
+    ThermalArgs a = cet_step_args(p, stop_flag);
+    const ThermalTrack t{c->cvox, c->pairop, changed, n_changed};
+    return launch_thermal<false>(c, a, &t);
 }
 
 template <bool NANFIX, int V, int CAP>

@@ -350,7 +350,10 @@ int cet_debug_nst_mismatches(cet_ctx *ctx, int64_t *n_bad);
  * the same bits).  Default: stamped sites are refreshed by the class-sorted list kernel on the compact tile
  * state (class codes + pair operands; rates_refresh.cu); the dense rebuild after a thermal step runs the
  * class-sorted tile kernel staged by 3-D TMA boxes (rates_dense.cu) when L % 16 == 0 and L >= 64, the dense
- * gather kernel on the compact state otherwise.
+ * gather kernel on the compact state otherwise.  After a thermal step of a whole-lattice context with L % 32 == 0
+ * and rates current before it, only the sites whose rates read a changed temperature are refreshed (the dense
+ * rebuild when they are more than three eighths of the lattice).
+ * 524288: the dense rebuild after every thermal step;
  * 262144: refresh by the pair-compacting list kernel (rates.cu); 131072: the dense tile kernel walks its sites by
  * class only, without the sort by pair count; 65536: dense rebuilds by the compact gather kernel;
  * 2: the gather refresh + dense kernel of the first design (neighbour-class cache + unit vectors);

@@ -140,6 +140,7 @@ SIGNATURES = {
                           C.POINTER(MetricsResult)],
     "cet_grain_profile_group": [C.POINTER(_VP), _I32, _I32, _F64, C.POINTER(_I64)],
     "cet_grain_shape_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, _I64, C.POINTER(_I64)],
+    "cet_front_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_I32), C.POINTER(_F64)],
     "cet_debug_nst_mismatches": [_VP, C.POINTER(_I64)],
     "cet_debug_flags": [_VP, C.c_int],
     "cet_profile_enable": [_VP, C.c_int],
@@ -718,6 +719,29 @@ def _shape_edges(fn, edges):
     if not np.all(np.diff(e) > 0.0):
         raise ValueError(f"{fn}: edges must ascend strictly, got {edges!r}")
     return e
+
+
+def front_group(ctxs, axis):
+    """The solidification front of every context of `ctxs` (whole-lattice Contexts of one L on one device) along the
+    growth axis `axis` (0, 1 or 2; growth from plane 0 toward plane L - 1), with one launch and two copies for the
+    group (include/cetkmc.h: cet_front_group).  Column c = u * L + w of the L^2 lines along the axis is indexed by
+    the other two coordinates, u the lower-numbered axis.  Returns a dict of four (n, L, L) arrays:
+        front     int32    consecutive occupied sites from plane 0 (0 .. L)
+        top       int32    1 + the highest occupied plane, 0 for an empty column
+        T_front   float64  T at plane `front` when front < L, else NaN
+        dT_front  float64  T[front] - T[front - 1] when 0 < front < L, else NaN
+    T is the context's current temperature (download(T=True)).  The call reads the lattice and T and changes nothing
+    the next sweep, metrics row, profile or shape reads."""
+    ctxs = list(ctxs)
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"front_group: axis must be 0, 1 or 2, got {axis!r}")
+    handles = _group_handles("front_group", ctxs)
+    L = ctxs[0].shape[2] if ctxs else 0
+    fr = np.zeros((len(ctxs), 2, L, L), np.int32)
+    tm = np.zeros((len(ctxs), 2, L, L), np.float64)
+    check(lib().cet_front_group(handles, len(ctxs), int(axis), fr.ctypes.data_as(C.POINTER(_I32)),
+                                tm.ctypes.data_as(C.POINTER(C.c_double))), "cet_front_group")
+    return {"front": fr[:, 0], "top": fr[:, 1], "T_front": tm[:, 0], "dT_front": tm[:, 1]}
 
 
 def comm_unique_id() -> bytes:

@@ -199,6 +199,45 @@ def grain_shape_summary(hist, edges, threshold=K.CET_AR_THRESHOLD):
             "ShapedGrains": shaped}
 
 
+FRONT_COLUMNS = ("FrontMean", "FrontRMS", "FrontMin", "FrontMax", "AheadMean", "AheadFraction", "FrontColumns",
+                 "T_Front", "Undercooling", "GradColumns", "G_Front")
+
+
+def front_summary(front, top, T_front, dT_front, t_melt=K.T_MELT, voxel_size=K.VOXEL_SIZE):
+    """The solidification conditions at the front of one lattice, from the four (L, L) column arrays of
+    cetkmc.front_group (front and top int, T_front and dT_front float; L the number of planes along the axis):
+        FrontMean, FrontRMS     mean and standard deviation (the front roughness, in planes) of `front`
+        FrontMin, FrontMax      its extremes
+        AheadMean               mean of top - front: planes of solid detached ahead of the front
+        AheadFraction           the fraction of columns with top > front
+        FrontColumns            columns whose front is inside the lattice (front < L)
+        T_Front, Undercooling   mean T_front over those columns, and t_melt - T_Front (K)
+        GradColumns             columns with 0 < front < L
+        G_Front                 mean dT_front over those columns / voxel_size: the gradient at the front (K/m)
+    A mean over no columns is "" (and so is what is derived from it)."""
+    h, t = np.asarray(front), np.asarray(top)
+    tf, dt = np.asarray(T_front, np.float64), np.asarray(dT_front, np.float64)
+    if h.ndim != 2 or h.shape[0] != h.shape[1] or any(a.shape != h.shape for a in (t, tf, dt)):
+        raise ValueError(f"front_summary: need four (L, L) arrays, got shapes {h.shape}, {t.shape}, {tf.shape}, {dt.shape}")
+    L = h.shape[0]
+    inside, grad = h < L, (h > 0) & (h < L)
+    ahead = t.astype(np.int64) - h.astype(np.int64)
+    n_in, n_grad = int(inside.sum()), int(grad.sum())
+    T_f = float(np.mean(tf[inside])) if n_in else ""
+    return {"FrontMean": float(np.mean(h)), "FrontRMS": float(np.std(h)), "FrontMin": int(h.min()), "FrontMax": int(h.max()),
+            "AheadMean": float(np.mean(ahead)), "AheadFraction": float(np.mean(t > h)),
+            "FrontColumns": n_in, "T_Front": T_f, "Undercooling": float(t_melt) - T_f if n_in else "",
+            "GradColumns": n_grad, "G_Front": float(np.mean(dt[grad])) / float(voxel_size) if n_grad else ""}
+
+
+def front_velocity(mean0, time0, mean1, time1, voxel_size=K.VOXEL_SIZE):
+    """The front velocity (m/s) between two metrics rows: (mean1 - mean0) * voxel_size / (time1 - time0), the means
+    FrontMean in planes and the times the driver's physical sweep clock (`Time`); "" when time1 <= time0."""
+    if not float(time1) > float(time0):
+        return ""
+    return (float(mean1) - float(mean0)) * float(voxel_size) / (float(time1) - float(time0))
+
+
 def grains_distributed(ctx, all_gather, theta_threshold=0.5):
     """Grains of a lattice that is split into z-slabs over several contexts (one per rank), in the form
     Context.grains() returns for a whole lattice — the reference's clusters (utils.py:28-84) in its

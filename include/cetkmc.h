@@ -339,6 +339,27 @@ int cet_grain_profile_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, d
  * table, one host synchronisation. */
 int cet_grain_shape_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, const double *edges, int32_t n_edges,
                           int64_t min_size, int64_t *out);
+/* ---- solidification conditions at the front of a group (front height, gradient, undercooling) ----
+ * A lattice grows along `axis` = a (0, 1 or 2) from plane 0 toward plane L - 1 (the generated lattices grow along 2).
+ * A column is one of the L^2 lines along a, indexed by the other two coordinates (u, w), u the lower-numbered axis:
+ * column c = u * L + w.  A site is occupied when (vox & 0x0F) != 0 (the grain labelling's predicate).  Per column:
+ *   front     int32  h = the number of consecutive occupied sites from plane 0 (0 .. L); the site at h is the
+ *                    liquid site at the front;
+ *   top       int32  1 + the plane of the highest occupied site, 0 for an empty column (top - front counts the planes
+ *                    of solid detached ahead of the front);
+ *   T_front   f64    T at plane h when h < L, else NaN;
+ *   dT_front  f64    T[h] - T[h - 1] (one IEEE subtraction) when 0 < h < L, else NaN; a NaN difference is NaN too.
+ * NaN is the one quiet NaN 0x7ff8000000000000; T is the context's current temperature (what the next sweep reads and
+ * cet_download returns), and a non-finite T at the front is returned as it is.
+ * front_out[(q * 2 + f) * L^2 + c]: f = 0 front, f = 1 top;  temp_out[(q * 2 + f) * L^2 + c]: f = 0 T_front,
+ * f = 1 dT_front.
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device, 1 <= n_ctx <= 64.
+ * Everything, the outputs included, is checked before anything is launched or written: a rejected call leaves every
+ * context and both outputs as they were.  The call is read-only on the lattice, T and every other field, so the next
+ * sweep, metrics row, profile and shape are what they would have been without it.  The work is ordered on the stream
+ * of ctxs[0] after the work already queued on every context's stream: one launch for the whole group, two D2H
+ * copies, one host synchronisation. */
+int cet_front_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, int32_t *front_out, double *temp_out);
 /* The same for global planes [i_lo, i_hi) within the labelled planes of a slab (owned + 2 ghost planes per
  * cut face): what two neighbouring slabs compare to join the grains that cross their cut. */
 int cet_grains_download_planes(cet_ctx *ctx, int64_t i_lo, int64_t i_hi, int32_t *labels);

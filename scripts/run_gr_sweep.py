@@ -14,6 +14,10 @@ lattice) and prints it, and with --replicas also cet_map_profile_ensemble.csv.
 --shape-axis a: every case also records the growth-axis elongation histogram of its grains along axis a in
 <case>/grain_shape.csv; rank 0 writes cet_map_shape.csv (columnar volume and grain fractions of every lattice) and
 prints it, and with --replicas also cet_map_shape_ensemble.csv.
+--front-axis a: every case also records the solidification conditions at its front along growth axis a (front height
+and roughness, gradient, undercooling, velocity) in <case>/front.csv; rank 0 writes cet_map_front.csv (the measured
+G_Front and V_Front of every lattice beside the nominal G and R) and prints it, and with --replicas also
+cet_map_front_ensemble.csv.
 """
 import argparse
 import csv
@@ -38,6 +42,7 @@ def main():
     ap.add_argument("--replicas", type=int, default=None)
     ap.add_argument("--profile-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--shape-axis", type=int, default=None, choices=(0, 1, 2))
+    ap.add_argument("--front-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     temps = [2600.0, 2800.0, 3000.0, 3200.0]                      # T_sub -> G = (T_MELT - T_sub) / (L dx)
@@ -46,7 +51,8 @@ def main():
     rows = campaign.run_gr_sweep(temps, nu_deps, L=args.L, n_sweeps=args.sweeps, n_seeds=20, defect_fraction=3e-3,
                                  impurity_c=0.1, output_root=args.out, metrics_every=100, batch=args.batch, replicas=args.replicas,
                                  **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}),
-                                 **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}))
+                                 **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}),
+                                 **({} if args.front_axis is None else {"front_axis": args.front_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -63,6 +69,11 @@ def main():
         for r in merged:
             print(f"case {int(r['case']):2d} T_sub {float(r['T_sub']):6.0f} NU_DEP {float(r['NU_DEP']):8.1e} G/R {float(r['G_over_R']):9.3e} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} {r['CET_Class']}")
+        if args.front_axis is not None:
+            for fn in ("cet_map_front.csv",) + (("cet_map_front_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.shape_axis is not None:
             for fn in ("cet_map_shape.csv",) + (("cet_map_shape_ensemble.csv",) if args.replicas is not None else ()):
                 with open(f"outputs/{args.out}/{fn}") as fh:

@@ -14,6 +14,10 @@ lattice) and prints it, and with --replicas also melt_pool_map_profile_ensemble.
 --shape-axis a: every case also records the growth-axis elongation histogram of its grains along axis a in
 <case>/grain_shape.csv; rank 0 writes melt_pool_map_shape.csv (columnar volume and grain fractions of every lattice) and
 prints it, and with --replicas also melt_pool_map_shape_ensemble.csv.
+--front-axis a: every case also records the solidification conditions at its front along growth axis a (front height
+and roughness, gradient, undercooling, velocity) in <case>/front.csv; rank 0 writes melt_pool_map_front.csv (the measured
+G_Front and V_Front of every lattice beside the nominal G and R) and prints it, and with --replicas also
+melt_pool_map_front_ensemble.csv.
 """
 import argparse
 import csv
@@ -37,6 +41,7 @@ def main():
     ap.add_argument("--replicas", type=int, default=None)
     ap.add_argument("--profile-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--shape-axis", type=int, default=None, choices=(0, 1, 2))
+    ap.add_argument("--front-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     powers = [100.0, 200.0, 300.0, 400.0]                         # W
@@ -46,7 +51,8 @@ def main():
                                n_seeds=20, defect_fraction=3e-3, impurity_c=0.1, output_root=args.out,
                                metrics_every=100, batch=args.batch, replicas=args.replicas,
                                **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}),
-                               **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}))
+                               **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}),
+                               **({} if args.front_axis is None else {"front_axis": args.front_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -64,6 +70,11 @@ def main():
             print(f"case {int(r['case']):2d} P {float(r['power']):6.1f} W V {float(r['speed']):5.2f} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} "
                   f"step {r['Step']} {r['CET_Class']}")
+        if args.front_axis is not None:
+            for fn in ("melt_pool_map_front.csv",) + (("melt_pool_map_front_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.shape_axis is not None:
             for fn in ("melt_pool_map_shape.csv",) + (("melt_pool_map_shape_ensemble.csv",) if args.replicas is not None else ()):
                 with open(f"outputs/{args.out}/{fn}") as fh:

@@ -141,6 +141,7 @@ SIGNATURES = {
     "cet_grain_profile_group": [C.POINTER(_VP), _I32, _I32, _F64, C.POINTER(_I64)],
     "cet_grain_shape_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, _I64, C.POINTER(_I64)],
     "cet_front_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_I32), C.POINTER(_F64)],
+    "cet_texture_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, C.POINTER(_I64)],
     "cet_debug_nst_mismatches": [_VP, C.POINTER(_I64)],
     "cet_debug_flags": [_VP, C.c_int],
     "cet_profile_enable": [_VP, C.c_int],
@@ -742,6 +743,56 @@ def front_group(ctxs, axis):
     check(lib().cet_front_group(handles, len(ctxs), int(axis), fr.ctypes.data_as(C.POINTER(_I32)),
                                 tm.ctypes.data_as(C.POINTER(C.c_double))), "cet_front_group")
     return {"front": fr[:, 0], "top": fr[:, 1], "T_front": tm[:, 0], "dT_front": tm[:, 1]}
+
+
+TEXTURE_EDGES_DEG = tuple(range(15, 180, 15))   # texture_group's default bin edges: 12 bins of 15 degrees
+TEXTURE_SCALE = 2 ** 32                           # the fixed-point scale of texture_group's sums
+TEXTURE_EDGES_MAX = 31
+
+
+def texture_group(ctxs, axis, edges_deg=TEXTURE_EDGES_DEG):
+    """Per-plane orientation histograms of every context of `ctxs` (whole-lattice Contexts of one L on one device)
+    along the growth axis `axis` (0, 1 or 2), with one launch and one copy for the group and no labelling
+    (include/cetkmc.h: cet_texture_group).  A site counts when it is occupied (state != 0, defects included); its angle
+    is the angle between its orientation vector and +axis, c = cos(angle) its component along the axis.
+    edges_deg: 1 to 31 angle edges in degrees, finite, strictly ascending, inside (0, 180).  The device bins c over the
+    edges cos(radians(edges_deg)) in ascending order; angle bin k holds edges_deg[k - 1] < angle <= edges_deg[k]
+    (edges_deg[-1] = 0, edges_deg[len] = 180).  That reading is exact only up to the rounding of those cosines: a site
+    whose c lies within an ulp of an edge's cosine falls on the side the rounded cosine puts it.
+    Returns (hist, sum_cos, sum_cos2): hist an (n, L, len(edges_deg) + 1) int64 array of the occupied sites of plane z
+    per angle bin, in ascending angle; sum_cos and sum_cos2 (n, L) int64 the exact fixed-point sums of c and of c^2
+    over those sites, each term rounded to the nearest integer multiple of 1 / TEXTURE_SCALE (half to even).  The call
+    changes nothing the next sweep, metrics row, profile, shape or front reads."""
+    ctxs = list(ctxs)
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"texture_group: axis must be 0, 1 or 2, got {axis!r}")
+    c = _texture_edges("texture_group", edges_deg)
+    handles = _group_handles("texture_group", ctxs)
+    m = c.size
+    L = ctxs[0].shape[2] if ctxs else 0
+    out = np.zeros((len(ctxs), L, m + 3), np.int64)
+    check(lib().cet_texture_group(handles, len(ctxs), int(axis), c.ctypes.data_as(C.POINTER(C.c_double)), m,
+                                  out.ctypes.data_as(C.POINTER(C.c_int64))), "cet_texture_group")
+    return np.ascontiguousarray(out[:, :, m::-1]), out[:, :, m + 1].copy(), out[:, :, m + 2].copy()
+
+
+def _texture_edges(fn, edges_deg):
+    """The ascending cosine edges of texture_group's angle edges (degrees): cos(radians(edges_deg[::-1])), refusing
+    what texture_group refuses."""
+    try:
+        e = np.asarray(edges_deg, dtype=np.float64)
+    except (TypeError, ValueError):
+        raise ValueError(f"{fn}: edges_deg must be numbers, got {edges_deg!r}") from None
+    if e.ndim != 1 or not 1 <= e.size <= TEXTURE_EDGES_MAX:
+        raise ValueError(f"{fn}: edges_deg must be 1 to {TEXTURE_EDGES_MAX} values, got shape {e.shape}")
+    if not np.all(np.isfinite(e)) or not np.all((e > 0.0) & (e < 180.0)):
+        raise ValueError(f"{fn}: edges_deg must be finite and inside (0, 180), got {edges_deg!r}")
+    if not np.all(np.diff(e) > 0.0):
+        raise ValueError(f"{fn}: edges_deg must ascend strictly, got {edges_deg!r}")
+    c = np.ascontiguousarray(np.cos(np.radians(e[::-1])))
+    if not np.all(np.diff(c) > 0.0):
+        raise ValueError(f"{fn}: the cosines of edges_deg {edges_deg!r} do not ascend strictly")
+    return c
 
 
 def comm_unique_id() -> bytes:

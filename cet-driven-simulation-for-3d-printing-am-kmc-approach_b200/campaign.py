@@ -31,6 +31,10 @@
                                      metrics.front_summary: front height and roughness, gradient G_Front,
                                      undercooling, velocity V_Front), and per map the measured G_Front and V_Front of
                                      every lattice beside the nominal G and R in <map>_front.csv
+    texture_axis=0|1|2               (run_cet_sublattice and the map drivers) the per-plane orientation histograms
+                                     along the growth axis of every metrics row in outputs/<prefix>/texture.csv
+                                     (cetkmc.texture_group), and per map the texture of every lattice
+                                     (metrics.texture_summary: MeanCos, Hermans, AlignedFraction) in <map>_texture.csv
 """
 from __future__ import annotations
 
@@ -186,7 +190,8 @@ def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_
                             all_gather=all_gather)
 
 
-def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shape_axis=None, front_axis=None):
+def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shape_axis=None, front_axis=None,
+                   texture_axis=None):
     """_cadence for every case of a group at once (cetkmc.metrics_group, one launch per kernel for the group): the
     defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  The Philox
     stream is keyed by r["seed"] where a case has one, else by `seed`.  With NumPy's
@@ -194,7 +199,8 @@ def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shap
     draws it.  profile_axis: one cetkmc.grain_profile_group call over the labelling the rows used appends each
     case's (step, profile) to r["profiles"]; shape_axis: one cetkmc.grain_shape_group call over that labelling appends
     each case's (step, histogram) to r["shapes"]; front_axis: one cetkmc.front_group call appends each case's (step,
-    time, metrics.front_summary) to r["fronts"]."""
+    time, metrics.front_summary) to r["fronts"]; texture_axis: one cetkmc.texture_group call appends each case's
+    (step, hist, sum_cos, sum_cos2) to r["textures"]."""
     ctxs = [r["ctx"] for r in runs]
     refresh = last % every == 0
     draws = None
@@ -227,6 +233,10 @@ def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shap
     if front_axis is not None:
         for r, s in zip(runs, _front_summaries(ctxs, front_axis)):
             r["fronts"].append((last, r["total_time"], s))
+    if texture_axis is not None:
+        hist, f1, f2 = _lib.texture_group(ctxs, texture_axis)
+        for q, r in enumerate(runs):
+            r["textures"].append((last, hist[q], f1[q], f2[q]))
 
 
 def _front_summaries(ctxs, axis):
@@ -239,13 +249,14 @@ def _front_summaries(ctxs, axis):
 PROFILE_CSV = "cet_profile.csv"
 SHAPE_CSV = "grain_shape.csv"
 FRONT_CSV = "front.csv"
+TEXTURE_CSV = "texture.csv"
 
 
 def _check_axis_kw(fn, name, axis, world=1, checkpoint_every=0, resume_from=None):
-    """Refuse what a run with per-plane grain profiles (name "profile_axis"), grain-shape histograms ("shape_axis") or
-    front conditions ("front_axis") does not take: an axis outside {0, 1, 2}, a lattice split into slabs (their labels
-    are slab-local, and a column crosses the cuts) and checkpoints (they do not carry the profile, shape or front
-    history)."""
+    """Refuse what a run with per-plane grain profiles (name "profile_axis"), grain-shape histograms ("shape_axis"),
+    front conditions ("front_axis") or texture ("texture_axis") does not take: an axis outside {0, 1, 2}, a lattice
+    split into slabs (their labels are slab-local, and a column crosses the cuts) and checkpoints (they do not carry
+    the profile, shape, front or texture history)."""
     if axis is None:
         return
     if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
@@ -315,6 +326,51 @@ def read_front_csv(path):
         return [{k: ("" if v == "" else int(v) if k in ints else float(v)) for k, v in r.items()} for r in csv.DictReader(fh)]
 
 
+def _texture_bin_names(edges_deg):
+    """The count columns of a texture.csv: one per angle bin, named "<lo>-<hi>" in degrees (the shortest positional
+    form that reads back exactly, never an exponent)."""
+    e = [float(x) for x in edges_deg]
+    name = [np.format_float_positional(x, trim="-") for x in [0.0] + e + [180.0]]
+    return [f"{name[b]}-{name[b + 1]}" for b in range(len(e) + 1)]
+
+
+def _write_texture_csv(textures, output_dir, edges_deg=_lib.TEXTURE_EDGES_DEG):
+    """outputs/<prefix>/texture.csv: one row per (metrics row, plane) of the (step, hist, sum_cos, sum_cos2) records of
+    cetkmc.texture_group: Step, Plane, Solid (the plane's occupied sites), SumCos, SumCos2 (the fixed-point sums), then
+    the sites of every angle bin in ascending angle.  Integers only."""
+    import csv
+    if not textures:
+        return
+    with open(os.path.join(output_dir, TEXTURE_CSV), "w", newline="") as fh:
+        w = csv.writer(fh)
+        w.writerow(["Step", "Plane", "Solid", "SumCos", "SumCos2"] + _texture_bin_names(edges_deg))
+        for step, hist, f1, f2 in textures:
+            for z in range(hist.shape[0]):
+                w.writerow([int(step), z, int(hist[z].sum()), int(f1[z]), int(f2[z])] + [int(v) for v in hist[z]])
+
+
+def read_texture_csv(path):
+    """The records of a texture.csv: (edges_deg, [(step, hist (L, m + 1), sum_cos (L,), sum_cos2 (L,)) per metrics
+    row]), the arrays int64 and the edges read back from the bin names."""
+    import csv
+    with open(path) as fh:
+        rd = csv.reader(fh)
+        head = next(rd)
+        rows = [[int(v) for v in r] for r in rd]
+    bins = head[5:]
+    edges = tuple(float(b.split("-")[1]) for b in bins[:-1])
+    out = []
+    for r in rows:
+        if not out or out[-1][0] != r[0]:
+            out.append((r[0], []))
+        out[-1][1].append(r)
+    recs = []
+    for step, rs in out:
+        a = np.array(rs, np.int64)
+        recs.append((step, a[:, 5:].copy(), a[:, 3].copy(), a[:, 4].copy()))
+    return edges, recs
+
+
 def read_shape_csv(path):
     """The last metrics row's histogram of a grain_shape.csv: (step, (2, n_edges + 2) int64 array, edges)."""
     import csv
@@ -343,7 +399,8 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
                        output_prefix="cet_sublattice", metrics_every=None, events_per_sweep=None, p_max=0.1,
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
                        checkpoint_every=0, resume_from=None, lattice=None, verbose=True, rank=0, world=1,
-                       mask_stream="numpy", init_seed=None, profile_axis=None, shape_axis=None, front_axis=None):
+                       mask_stream="numpy", init_seed=None, profile_axis=None, shape_axis=None, front_axis=None,
+                       texture_axis=None):
     """run_kmc's large-lattice sibling.  Same set-up (initialize_lattice + introduce_defects with the
     run's seed), same cadence and CSV; the steps are synchronous-sublattice sweeps (csrc/sweep.cu), so
     `Step` counts sweeps and `Time` is the accumulated sweep interval.
@@ -370,6 +427,11 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
            with the columns Step, Time, metrics.FRONT_COLUMNS and V_Front (metrics.front_velocity against the previous
            row, "" on the first).  Every other output is the same as without it.  Not with world > 1,
            checkpoint_every or resume_from.
+    texture_axis: None, or 0, 1 or 2: the growth axis; every metrics row also takes the per-plane orientation
+           histograms of the lattice along it (cetkmc.texture_group with its default edges), written to
+           outputs/<prefix>/texture.csv with the columns Step, Plane, Solid, SumCos, SumCos2 and one count per angle
+           bin, one row per (metrics row, plane).  Every other output is the same as without it.  Not with world > 1,
+           checkpoint_every or resume_from.
     world > 1: the lattice is split into z-slabs, one per rank / GPU (launch every rank with the same
            arguments plus its rank; torch.distributed.run provides the rendezvous).  The trajectory and
            the CSV do not depend on the number of slabs.  Rank 0 writes the CSV; every rank returns its
@@ -390,6 +452,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     _check_axis_kw("run_cet_sublattice", "profile_axis", profile_axis, world, checkpoint_every, resume_from)
     _check_axis_kw("run_cet_sublattice", "shape_axis", shape_axis, world, checkpoint_every, resume_from)
     _check_axis_kw("run_cet_sublattice", "front_axis", front_axis, world, checkpoint_every, resume_from)
+    _check_axis_kw("run_cet_sublattice", "texture_axis", texture_axis, world, checkpoint_every, resume_from)
     np.random.seed(seed)                                    # a resumed run restores the stream position below
     output_dir = f"outputs/{output_prefix}"
     os.makedirs(output_dir, exist_ok=True)
@@ -406,6 +469,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     try:
         ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
         sweep0, total_time, nucleation_count, cet_detected, rows, profiles, shapes, fronts = 0, 0.0, 0, False, [], [], [], []
+        textures = []
         if resume_from:
             meta = resume(ctx, resume_from)
             sweep0, total_time = int(meta.get("sweep", 0)), float(meta.get("time", 0.0))
@@ -460,6 +524,9 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
                 shapes.append((sweep - 1, _lib.grain_shape_group([ctx], shape_axis)[0]))
             if front_axis is not None:
                 fronts.append((sweep - 1, total_time, _front_summaries([ctx], front_axis)[0]))
+            if texture_axis is not None:
+                hist, f1, f2 = _lib.texture_group([ctx], texture_axis)
+                textures.append((sweep - 1, hist[0], f1[0], f2[0]))
             if checkpoint_every and (len(rows) % checkpoint_every == 0):
                 checkpoint(ctx, os.path.join(output_dir, "checkpoint"), sweep=sweep, time=total_time,
                            nucleation_count=nucleation_count, cet_detected=cet_detected,
@@ -469,6 +536,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             _write_profile_csv(profiles, output_dir)
             _write_shape_csv(shapes, output_dir)
             _write_front_csv(fronts, output_dir)
+            _write_texture_csv(textures, output_dir)
         f = ctx.download(state=True, atom_type=True, theta=True, phi=True)
     finally:
         ctx.close()
@@ -514,7 +582,9 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
     shape_axis=a (through **kw): every case writes outputs/<prefix>/grain_shape.csv (run_cet_sublattice), and each rank
     writes cet_map_shape_rank<r>.csv (_map_shape_rows); every other file is the same as without it.
     front_axis=a (through **kw): every case writes outputs/<prefix>/front.csv (run_cet_sublattice), and each rank
-    writes cet_map_front_rank<r>.csv (_map_front_rows); every other file is the same as without it."""
+    writes cet_map_front_rank<r>.csv (_map_front_rows); every other file is the same as without it.
+    texture_axis=a (through **kw): every case writes outputs/<prefix>/texture.csv (run_cet_sublattice), and each rank
+    writes cet_map_texture_rank<r>.csv (_map_texture_rows); every other file is the same as without it."""
     cases = [(float(t), float(r)) for t in temps for r in nu_deps]
 
     def case_row(q):
@@ -541,6 +611,7 @@ def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses
     _check_axis_kw(fn, "profile_axis", kw.get("profile_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_axis_kw(fn, "shape_axis", kw.get("shape_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_axis_kw(fn, "front_axis", kw.get("front_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
+    _check_axis_kw(fn, "texture_axis", kw.get("texture_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_mask_and_laser(fn, kw.get("mask_stream", "numpy"), lasers is not None or kw.get("laser"),
                           kw.get("thermal_every", _ks.THERMAL_EVERY))
     if batch is not None:
@@ -560,7 +631,7 @@ def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses
                                lasers=None if lasers is None else [lasers[lats[l][0]] for l in ls],
                                replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
     return _map_outputs(output_root, name, lats, [l for _d, ls in parts for l in ls], case_row, axes, replicas, rank,
-                        world, kw.get("profile_axis"), kw.get("shape_axis"), kw.get("front_axis"))
+                        world, kw.get("profile_axis"), kw.get("shape_axis"), kw.get("front_axis"), kw.get("texture_axis"))
 
 
 _MAP_FINAL = ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount",
@@ -596,12 +667,13 @@ def _replica_kw(kw, replicas, r):
 
 
 def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world, profile_axis=None,
-                 shape_axis=None, front_axis=None):
+                 shape_axis=None, front_axis=None, texture_axis=None):
     """The per-rank files of a map driver over the lattices `mine` (indices into `lats`) this rank ran:
     <name>_rank<rank>.csv (case, case_row(case), the final row's _MAP_FINAL columns) and the plot_cet tree from
     replica 0 of each case, with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica), with
     profile_axis <name>_profile_rank<rank>.csv (_map_profile_rows) and with shape_axis <name>_shape_rank<rank>.csv
-    (_map_shape_rows), with front_axis <name>_front_rank<rank>.csv (_map_front_rows).  Returns the map rows; with
+    (_map_shape_rows), with front_axis <name>_front_rank<rank>.csv (_map_front_rows), with texture_axis
+    <name>_texture_rank<rank>.csv (_map_texture_rows).  Returns the map rows; with
     replicas (map rows,
     ensemble_stats of the replica rows), the latter None when world > 1 (merge_* joins the ranks)."""
     import csv
@@ -623,6 +695,9 @@ def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, 
         _write_rows(_map_shape_rows(lats, sorted(mine), case_row, axes), os.path.join(out_dir, f"{name}_shape_rank{rank}.csv"))
     if front_axis is not None:
         _write_rows(_map_front_rows(lats, sorted(mine), case_row, axes), os.path.join(out_dir, f"{name}_front_rank{rank}.csv"))
+    if texture_axis is not None:
+        _write_rows(_map_texture_rows(lats, sorted(mine), case_row, axes),
+                    os.path.join(out_dir, f"{name}_texture_rank{rank}.csv"))
     write_plot_cet_tree([(row["case"], f"outputs/{lats[l][2]}/metrics.csv")
                          for row, l in zip(rows, sorted(l for l in mine if lats[l][1] == 0))],
                         os.path.join(out_dir, "plot_cet"))
@@ -725,6 +800,43 @@ def front_ensemble_stats(rows, axes):
     return out
 
 
+TEXTURE_ENSEMBLE = ("MeanCos", "Hermans", "AlignedFraction")
+
+
+def _map_texture_rows(lats, mine, case_row, axes):
+    """One row per lattice of `mine` (case, replica, the map's axis columns, and metrics.texture_summary of the final
+    row's histograms in outputs/<prefix>/texture.csv)."""
+    out = []
+    for l in mine:
+        q, r, p = lats[l]
+        edges, recs = read_texture_csv(f"outputs/{p}/{TEXTURE_CSV}")
+        _step, hist, f1, f2 = recs[-1]
+        c = case_row(q)
+        out.append({"case": q, "replica": r, **{k: c[k] for k in axes}, **_metrics.texture_summary(hist, f1, f2, edges)})
+    return out
+
+
+def texture_ensemble_stats(rows, axes):
+    """One row per case over the rows of a <map>_texture.csv (dicts with case, replica, the axis columns `axes` and
+    TEXTURE_ENSEMBLE; numbers or the strings a CSV gives back), in case order: case, the axes, replicas (n), and per
+    column of TEXTURE_ENSEMBLE <col>_mean and <col>_se over the replicas where it is defined (not ""): the mean, and
+    the sample standard deviation, ddof=1, over the square root of their number (empty below 2; the mean empty when
+    none)."""
+    by_case = {}
+    for r in rows:
+        by_case.setdefault(int(r["case"]), []).append(r)
+    out = []
+    for case in sorted(by_case):
+        rs = by_case[case]
+        e = {"case": case, **{k: rs[0][k] for k in axes}, "replicas": len(rs)}
+        for col in TEXTURE_ENSEMBLE:
+            v = np.array([float(r[col]) for r in rs if r[col] != ""])
+            e[f"{col}_mean"] = float(np.mean(v)) if v.size else ""
+            e[f"{col}_se"] = float(np.std(v, ddof=1) / np.sqrt(v.size)) if v.size > 1 else ""
+        out.append(e)
+    return out
+
+
 def profile_ensemble_stats(rows, axes):
     """One row per case over the rows of a <map>_profile.csv (dicts with case, replica, the axis columns `axes`,
     CET_Height; numbers or the strings a CSV gives back), in case order: case, the axes, replicas (n), p_cet_height
@@ -774,7 +886,8 @@ def ensemble_stats(rows, axes):
 
 def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
                        events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy",
-                       lasers=None, replicas=None, profile_axis=None, shape_axis=None, front_axis=None):
+                       lasers=None, replicas=None, profile_axis=None, shape_axis=None, front_axis=None,
+                       texture_axis=None):
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
@@ -791,11 +904,13 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     (_cadence_group), and each case writes the cet_profile.csv run_cet_sublattice(profile_axis=...) writes.
     shape_axis: the same with one cetkmc.grain_shape_group call per row, and the grain_shape.csv of
     run_cet_sublattice(shape_axis=...); front_axis: one cetkmc.front_group call per row, and the front.csv of
-    run_cet_sublattice(front_axis=...)."""
+    run_cet_sublattice(front_axis=...); texture_axis: one cetkmc.texture_group call per row, and the texture.csv of
+    run_cet_sublattice(texture_axis=...)."""
     _check_mask_and_laser("_run_cases_grouped", mask_stream, lasers is not None, thermal_every)
     _check_axis_kw("_run_cases_grouped", "profile_axis", profile_axis)
     _check_axis_kw("_run_cases_grouped", "shape_axis", shape_axis)
     _check_axis_kw("_run_cases_grouped", "front_axis", front_axis)
+    _check_axis_kw("_run_cases_grouped", "texture_axis", texture_axis)
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
     philox_mask = mask_stream == "philox"
@@ -810,7 +925,7 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
             ctx.init_seed = None if replicas is None else 42 + reps[q]
             ctx.init_nuclei = []
             r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], profiles=[], shapes=[], fronts=[],
-                     total_time=0.0,
+                     textures=[], total_time=0.0,
                      nucleation_count=0, cet_detected=False, terminated=False)
             runs.append(r)
             ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
@@ -842,15 +957,18 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
                 sweep += blk
                 stopped = [r for r in active if r["terminated"]]
                 if stopped:
-                    _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis, front_axis)
+                    _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis, front_axis,
+                                   texture_axis)
                     active = [r for r in active if not r["terminated"]]
             if active:
-                _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis, front_axis)
+                _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis, front_axis,
+                               texture_axis)
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
             _write_profile_csv(r["profiles"], f"outputs/{r['prefix']}")
             _write_shape_csv(r["shapes"], f"outputs/{r['prefix']}")
             _write_front_csv(r["fronts"], f"outputs/{r['prefix']}")
+            _write_texture_csv(r["textures"], f"outputs/{r['prefix']}")
     finally:
         for r in runs:
             r["ctx"].close()
@@ -907,7 +1025,9 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     writes melt_pool_map_shape_rank<r>.csv (_map_shape_rows); every other file is the same as without it.
     front_axis=a (through **kw): every case writes outputs/<prefix>/front.csv (run_cet_sublattice), and each rank
     writes melt_pool_map_front_rank<r>.csv (_map_front_rows) with the measured G_Front and V_Front of every lattice
-    beside the nominal G and R; every other file is the same as without it."""
+    beside the nominal G and R; every other file is the same as without it.
+    texture_axis=a (through **kw): every case writes outputs/<prefix>/texture.csv (run_cet_sublattice), and each rank
+    writes melt_pool_map_texture_rank<r>.csv (_map_texture_rows); every other file is the same as without it."""
     powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
     if not powers or not speeds:
         raise ValueError("run_melt_pool_map: needs at least one power and one speed")
@@ -983,6 +1103,9 @@ def _merge_map(output_root, name, axes):
     front = _merge_rank_files(output_root, f"{name}_front")
     if front and reps:
         _write_rows(front_ensemble_stats(front, axes), f"outputs/{output_root}/{name}_front_ensemble.csv")
+    texture = _merge_rank_files(output_root, f"{name}_texture")
+    if texture and reps:
+        _write_rows(texture_ensemble_stats(texture, axes), f"outputs/{output_root}/{name}_texture_ensemble.csv")
     return rows
 
 
@@ -992,7 +1115,8 @@ def merge_cet_map(output_root="gr_sweep"):
     with profile_axis also cet_map_profile.csv (sorted by case and replica), and with replicas
     cet_map_profile_ensemble.csv (profile_ensemble_stats); after a run with shape_axis also cet_map_shape.csv and, with
     replicas, cet_map_shape_ensemble.csv (shape_ensemble_stats); after a run with front_axis also cet_map_front.csv and,
-    with replicas, cet_map_front_ensemble.csv (front_ensemble_stats)."""
+    with replicas, cet_map_front_ensemble.csv (front_ensemble_stats); after a run with texture_axis also
+    cet_map_texture.csv and, with replicas, cet_map_texture_ensemble.csv (texture_ensemble_stats)."""
     return _merge_map(output_root, "cet_map", ("T_sub", "NU_DEP"))
 
 
@@ -1001,5 +1125,6 @@ def merge_melt_pool_map(output_root="melt_pool_map"):
     after a run with replicas also melt_pool_map_replicas.csv and melt_pool_map_ensemble.csv (ensemble_stats); after
     a run with profile_axis also melt_pool_map_profile.csv and, with replicas, melt_pool_map_profile_ensemble.csv;
     after a run with shape_axis also melt_pool_map_shape.csv and, with replicas, melt_pool_map_shape_ensemble.csv;
-    after a run with front_axis also melt_pool_map_front.csv and, with replicas, melt_pool_map_front_ensemble.csv."""
+    after a run with front_axis also melt_pool_map_front.csv and, with replicas, melt_pool_map_front_ensemble.csv;
+    after a run with texture_axis also melt_pool_map_texture.csv and, with replicas, melt_pool_map_texture_ensemble.csv."""
     return _merge_map(output_root, "melt_pool_map", ("power", "speed", "T_sub", "NU_DEP"))

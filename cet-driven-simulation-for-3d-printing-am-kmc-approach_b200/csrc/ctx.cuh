@@ -187,6 +187,8 @@ struct cet_ctx {
     size_t cap_shape_tab = 0;
     void *front_tab = nullptr;        // front columns (cet_front_group) of the groups this context leads, grow-only
     size_t cap_front_tab = 0;
+    void *texture_tab = nullptr;      // per-plane orientation histograms (cet_texture_group) of the groups this context leads, grow-only
+    size_t cap_texture_tab = 0;
 
     // per-kernel-kind device timing (cet_profile_*): event pairs recorded around the dominant
     // kernels on the context stream, resolved when the totals are read

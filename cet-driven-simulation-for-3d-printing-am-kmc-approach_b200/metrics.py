@@ -238,6 +238,43 @@ def front_velocity(mean0, time0, mean1, time1, voxel_size=K.VOXEL_SIZE):
     return (float(mean1) - float(mean0)) * float(voxel_size) / (float(time1) - float(time0))
 
 
+TEXTURE_COLUMNS = ("TexturedSolid", "MeanCos", "Hermans", "AlignedFraction")
+TEXTURE_SCALE = 2 ** 32                 # cetkmc.texture_group's fixed-point scale
+
+
+def texture_summary(hist, sum_cos, sum_cos2, edges_deg, aligned_deg=30):
+    """The texture along the growth axis of one lattice, over all its planes, from the arrays of cetkmc.texture_group
+    for that lattice: hist (L, len(edges_deg) + 1) sites per angle bin in ascending angle, sum_cos and sum_cos2 (L,)
+    the fixed-point sums F1 = sum c * 2^32 and F2 = sum c^2 * 2^32 (c the cosine between a site's orientation and the
+    axis).  `aligned_deg` must be one of `edges_deg`, so that a bin lies wholly on one side of it.
+        TexturedSolid    the occupied sites N
+        MeanCos          F1 / (N 2^32): the mean cosine
+        Hermans          (3 F2 / (N 2^32) - 1) / 2: the orientation factor, 1 fully aligned with the axis, -1/2
+                         perpendicular to it, 0 for orientations uniform on the sphere
+        AlignedFraction  the sites in the bins up to aligned_deg (angle <= aligned_deg, as the bins read it) / N
+    Each is one correctly rounded quotient of exact integers; "" where N = 0.
+    The null of the model's nucleation draw (theta ~ U(0, pi), phi ~ U(0, 2 pi), uniform in the angles rather than on
+    the sphere): along axis 2, where c = cos(theta), MeanCos 0, Hermans 1/4 (E[cos^2 theta] = 1/2), AlignedFraction
+    aligned_deg / 180 and every bin its width / 180 of the sites; along axes 0 and 1, where c = sin(theta) cos(phi) or
+    sin(theta) sin(phi), MeanCos 0 and Hermans -1/8 (E[c^2] = 1/4).  A lattice that only nucleated sits at that null;
+    growth that selects orientations along +axis raises MeanCos, Hermans and AlignedFraction above it."""
+    e = [float(x) for x in edges_deg]
+    h = np.asarray(hist)
+    f1, f2 = np.asarray(sum_cos), np.asarray(sum_cos2)
+    if h.ndim != 2 or h.shape[1] != len(e) + 1 or f1.shape != (h.shape[0],) or f2.shape != (h.shape[0],):
+        raise ValueError(f"texture_summary: need an (L, {len(e) + 1}) histogram and two (L,) sums, got shapes "
+                         f"{h.shape}, {f1.shape}, {f2.shape}")
+    if float(aligned_deg) not in e:
+        raise ValueError(f"texture_summary: aligned_deg {aligned_deg!r} must be one of the edges {tuple(e)}")
+    n = sum(int(x) for x in h.sum(axis=0))
+    if n == 0:
+        return {"TexturedSolid": 0, "MeanCos": "", "Hermans": "", "AlignedFraction": ""}
+    F1, F2 = sum(int(x) for x in f1), sum(int(x) for x in f2)
+    aligned = sum(int(x) for x in h[:, :e.index(float(aligned_deg)) + 1].sum(axis=0))
+    return {"TexturedSolid": n, "MeanCos": F1 / (n * TEXTURE_SCALE), "Hermans": (3 * F2 - n * TEXTURE_SCALE) / (2 * n * TEXTURE_SCALE),
+            "AlignedFraction": aligned / n}
+
+
 def grains_distributed(ctx, all_gather, theta_threshold=0.5):
     """Grains of a lattice that is split into z-slabs over several contexts (one per rank), in the form
     Context.grains() returns for a whole lattice — the reference's clusters (utils.py:28-84) in its

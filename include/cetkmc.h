@@ -360,6 +360,25 @@ int cet_grain_shape_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, con
  * of ctxs[0] after the work already queued on every context's stream: one launch for the whole group, two D2H
  * copies, one host synchronisation. */
 int cet_front_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, int32_t *front_out, double *temp_out);
+/* ---- texture along a growth axis: per-plane orientation histograms of a group ----
+ * A site is occupied when (vox & 0x0F) != 0 (the predicate of the labelling, the profile and the front, so defect
+ * sites count).  Its orientation is its resident unit vector v (cet_device_ptr field 5: 32-byte records x, y, z, pad,
+ * kept equal to unit_vec4(theta, phi) by every writer); x, y, z are axes 0, 1, 2.  For `axis` = a (0, 1 or 2),
+ * c = v[a] is the cosine of the angle between the orientation and +a.  The bins take the interior edges
+ * e_0 < ... < e_{m-1} on c (m = n_edges, 1 <= m <= 31; finite, within [-1, 1], strictly ascending): the bin of a site
+ * is b = #{i : e_i <= c} in 0 .. m, so bin b holds e_{b-1} <= c < e_b with e_{-1} = -inf and e_m = +inf.  The sums are
+ * exact fixed point: F1 = sum llrint(c * 2^32), F2 = sum llrint(fl(c * c) * 2^32), fl(c * c) one IEEE product (no
+ * contraction), llrint rounding half to even; a plane holds at most L^2 sites, so no sum overflows.
+ * out[((q * L) + z) * (n_edges + 3) + j] for context q and plane z along `axis`: j <= n_edges the occupied sites of
+ * plane z in bin j, j = n_edges + 1 their F1, j = n_edges + 2 their F2.
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device, 1 <= n_ctx <= 64.
+ * Everything, `out` included, is checked before anything is launched or written: a rejected call leaves every context
+ * and `out` as they were.  The call needs no labelling and is read-only on every field, so the next sweep, metrics
+ * row, profile, shape and front are what they would have been without it.  The work is ordered on the stream of
+ * ctxs[0] after the work already queued on every context's stream: one memset, one launch for the whole group, one
+ * D2H copy, one host synchronisation. */
+int cet_texture_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, const double *edges, int32_t n_edges,
+                      int64_t *out);
 /* The same for global planes [i_lo, i_hi) within the labelled planes of a slab (owned + 2 ghost planes per
  * cut face): what two neighbouring slabs compare to join the grains that cross their cut. */
 int cet_grains_download_planes(cet_ctx *ctx, int64_t i_lo, int64_t i_hi, int32_t *labels);

@@ -18,6 +18,9 @@ prints it, and with --replicas also melt_pool_map_shape_ensemble.csv.
 and roughness, gradient, undercooling, velocity) in <case>/front.csv; rank 0 writes melt_pool_map_front.csv (the measured
 G_Front and V_Front of every lattice beside the nominal G and R) and prints it, and with --replicas also
 melt_pool_map_front_ensemble.csv.
+--texture-axis a: every case also records the per-plane orientation histograms of its occupied sites along growth
+axis a in <case>/texture.csv; rank 0 writes melt_pool_map_texture.csv (mean cosine, Hermans factor and aligned fraction of every
+lattice) and prints it, and with --replicas also melt_pool_map_texture_ensemble.csv.
 """
 import argparse
 import csv
@@ -42,6 +45,7 @@ def main():
     ap.add_argument("--profile-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--shape-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--front-axis", type=int, default=None, choices=(0, 1, 2))
+    ap.add_argument("--texture-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     powers = [100.0, 200.0, 300.0, 400.0]                         # W
@@ -52,7 +56,8 @@ def main():
                                metrics_every=100, batch=args.batch, replicas=args.replicas,
                                **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}),
                                **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}),
-                               **({} if args.front_axis is None else {"front_axis": args.front_axis}))
+                               **({} if args.front_axis is None else {"front_axis": args.front_axis}),
+                               **({} if args.texture_axis is None else {"texture_axis": args.texture_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -70,6 +75,11 @@ def main():
             print(f"case {int(r['case']):2d} P {float(r['power']):6.1f} W V {float(r['speed']):5.2f} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} "
                   f"step {r['Step']} {r['CET_Class']}")
+        if args.texture_axis is not None:
+            for fn in ("melt_pool_map_texture.csv",) + (("melt_pool_map_texture_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.front_axis is not None:
             for fn in ("melt_pool_map_front.csv",) + (("melt_pool_map_front_ensemble.csv",) if args.replicas is not None else ()):
                 with open(f"outputs/{args.out}/{fn}") as fh:

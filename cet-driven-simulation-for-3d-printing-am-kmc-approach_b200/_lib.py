@@ -142,6 +142,7 @@ SIGNATURES = {
     "cet_grain_shape_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, _I64, C.POINTER(_I64)],
     "cet_front_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_I32), C.POINTER(_F64)],
     "cet_texture_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, C.POINTER(_I64)],
+    "cet_boundary_group": [C.POINTER(_VP), _I32, _I32, C.POINTER(_F64), _I32, C.POINTER(_I64)],
     "cet_debug_nst_mismatches": [_VP, C.POINTER(_I64)],
     "cet_debug_flags": [_VP, C.c_int],
     "cet_profile_enable": [_VP, C.c_int],
@@ -793,6 +794,43 @@ def _texture_edges(fn, edges_deg):
     if not np.all(np.diff(c) > 0.0):
         raise ValueError(f"{fn}: the cosines of edges_deg {edges_deg!r} do not ascend strictly")
     return c
+
+
+BOUNDARY_EDGES_DEG = tuple(range(10, 180, 10))  # boundary_group's default misorientation edges: 18 bins of 10 degrees
+BOUNDARY_SCALE = 2 ** 32                          # the fixed-point scale of boundary_group's sum
+BOUNDARY_OFFSETS = ((1, 1, 0), (1, -1, 0), (0, 1, 1), (0, 1, -1), (2, 0, 0), (0, 2, 0), (0, 0, 2))   # bond offset r
+BOUNDARY_CLASSES = ("Solid", "Boundary", "Interface")                                               # bond class f
+
+
+def boundary_group(ctxs, axis, edges_deg=BOUNDARY_EDGES_DEG):
+    """Per-plane bond counts and boundary misorientation of the last grain labelling (Context.grains(), metrics_group)
+    of every context of `ctxs` (whole-lattice Contexts of one L on one device) along the growth axis `axis` (0, 1 or 2),
+    with one launch and one copy for the group (include/cetkmc.h: cet_boundary_group).  A bond joins a site s to
+    s + BOUNDARY_OFFSETS[r] inside the lattice (no wrap; the labelling's neighbourhood, each bond counted once; the
+    offsets keep the parity of i + j + k, so a line along an axis steps by 2).  Its plane along the axis is the lower of
+    its ends' coordinates.  A bond is solid when both ends are labelled (occupied), boundary when they are solid with
+    different labels, interface when exactly one end is occupied.  The misorientation of a boundary bond is the angle
+    between its ends' orientation vectors, d = cos(angle) their dot product.
+    edges_deg: 1 to 31 angle edges in degrees, finite, strictly ascending, inside (0, 180), converted to cosine edges as
+    texture_group converts them; angle bin k holds edges_deg[k - 1] < angle <= edges_deg[k], up to the rounding of the
+    edges' cosines.
+    Returns (bonds, hist, sum_cos): bonds an (n, L, 7, 3) int64 array of the bonds of plane z of offset r and class f
+    (BOUNDARY_CLASSES); hist (n, L, len(edges_deg) + 1) int64 the boundary bonds of plane z per misorientation bin, in
+    ascending angle; sum_cos (n, L) int64 the exact fixed-point sum of d over those bonds, each term rounded to the
+    nearest integer multiple of 1 / BOUNDARY_SCALE (half to even).  The call does not relabel and changes nothing the
+    next sweep, metrics row, profile, shape, front or texture reads."""
+    ctxs = list(ctxs)
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"boundary_group: axis must be 0, 1 or 2, got {axis!r}")
+    c = _texture_edges("boundary_group", edges_deg)
+    handles = _group_handles("boundary_group", ctxs)
+    m = c.size
+    L = ctxs[0].shape[2] if ctxs else 0
+    out = np.zeros((len(ctxs), L, 21 + m + 2), np.int64)
+    check(lib().cet_boundary_group(handles, len(ctxs), int(axis), c.ctypes.data_as(C.POINTER(C.c_double)), m,
+                                   out.ctypes.data_as(C.POINTER(C.c_int64))), "cet_boundary_group")
+    return (out[:, :, :21].reshape(len(ctxs), L, 7, 3).copy(), np.ascontiguousarray(out[:, :, 21 + m:20:-1]),
+            out[:, :, 21 + m + 1].copy())
 
 
 def comm_unique_id() -> bytes:

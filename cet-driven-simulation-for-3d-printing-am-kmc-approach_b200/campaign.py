@@ -35,6 +35,11 @@
                                      along the growth axis of every metrics row in outputs/<prefix>/texture.csv
                                      (cetkmc.texture_group), and per map the texture of every lattice
                                      (metrics.texture_summary: MeanCos, Hermans, AlignedFraction) in <map>_texture.csv
+    boundary_axis=0|1|2              (run_cet_sublattice and the map drivers) the per-plane bond counts and boundary
+                                     misorientation histograms along the growth axis of every metrics row in
+                                     outputs/<prefix>/boundaries.csv (cetkmc.boundary_group), and per map the boundary
+                                     network of every lattice (metrics.boundary_summary: linear intercepts along and
+                                     across the axis, boundary fraction, mean misorientation) in <map>_boundary.csv
 """
 from __future__ import annotations
 
@@ -191,7 +196,7 @@ def _cadence(ctx, last, every, philox_mask, seed, world, total_time, nucleation_
 
 
 def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shape_axis=None, front_axis=None,
-                   texture_axis=None):
+                   texture_axis=None, boundary_axis=None):
     """_cadence for every case of a group at once (cetkmc.metrics_group, one launch per kernel for the group): the
     defect-mask refresh on multiples of `every` and each case's metrics row, appended to r["rows"].  The Philox
     stream is keyed by r["seed"] where a case has one, else by `seed`.  With NumPy's
@@ -200,7 +205,8 @@ def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shap
     case's (step, profile) to r["profiles"]; shape_axis: one cetkmc.grain_shape_group call over that labelling appends
     each case's (step, histogram) to r["shapes"]; front_axis: one cetkmc.front_group call appends each case's (step,
     time, metrics.front_summary) to r["fronts"]; texture_axis: one cetkmc.texture_group call appends each case's
-    (step, hist, sum_cos, sum_cos2) to r["textures"]."""
+    (step, hist, sum_cos, sum_cos2) to r["textures"]; boundary_axis: one cetkmc.boundary_group call over the labelling
+    the rows used appends each case's (step, bonds, hist, sum_cos) to r["boundaries"]."""
     ctxs = [r["ctx"] for r in runs]
     refresh = last % every == 0
     draws = None
@@ -237,6 +243,10 @@ def _cadence_group(runs, last, every, philox_mask, seed, profile_axis=None, shap
         hist, f1, f2 = _lib.texture_group(ctxs, texture_axis)
         for q, r in enumerate(runs):
             r["textures"].append((last, hist[q], f1[q], f2[q]))
+    if boundary_axis is not None:
+        bonds, hist, f = _lib.boundary_group(ctxs, boundary_axis)
+        for q, r in enumerate(runs):
+            r["boundaries"].append((last, bonds[q], hist[q], f[q]))
 
 
 def _front_summaries(ctxs, axis):
@@ -250,13 +260,14 @@ PROFILE_CSV = "cet_profile.csv"
 SHAPE_CSV = "grain_shape.csv"
 FRONT_CSV = "front.csv"
 TEXTURE_CSV = "texture.csv"
+BOUNDARY_CSV = "boundaries.csv"
 
 
 def _check_axis_kw(fn, name, axis, world=1, checkpoint_every=0, resume_from=None):
     """Refuse what a run with per-plane grain profiles (name "profile_axis"), grain-shape histograms ("shape_axis"),
-    front conditions ("front_axis") or texture ("texture_axis") does not take: an axis outside {0, 1, 2}, a lattice
-    split into slabs (their labels are slab-local, and a column crosses the cuts) and checkpoints (they do not carry
-    the profile, shape, front or texture history)."""
+    front conditions ("front_axis"), texture ("texture_axis") or grain boundaries ("boundary_axis") does not take: an
+    axis outside {0, 1, 2}, a lattice split into slabs (their labels are slab-local, and a column crosses the cuts) and
+    checkpoints (they do not carry the profile, shape, front, texture or boundary history)."""
     if axis is None:
         return
     if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
@@ -371,6 +382,50 @@ def read_texture_csv(path):
     return edges, recs
 
 
+def _boundary_bond_names():
+    """The 21 bond-count columns of a boundaries.csv, j = 3 r + f: "<class><r>" for offset r of
+    cetkmc._lib.BOUNDARY_OFFSETS and class f of cetkmc._lib.BOUNDARY_CLASSES."""
+    return [f"{cls}{r}" for r in range(7) for cls in _lib.BOUNDARY_CLASSES]
+
+
+def _write_boundary_csv(boundaries, output_dir, edges_deg=_lib.BOUNDARY_EDGES_DEG):
+    """outputs/<prefix>/boundaries.csv: one row per (metrics row, plane) of the (step, bonds, hist, sum_cos) records of
+    cetkmc.boundary_group: Step, Plane, the 21 bond counts (_boundary_bond_names), the boundary bonds of every
+    misorientation bin in ascending angle (named "<lo>-<hi>" in degrees), then SumCos (the fixed-point sum).  Integers
+    only."""
+    import csv
+    if not boundaries:
+        return
+    with open(os.path.join(output_dir, BOUNDARY_CSV), "w", newline="") as fh:
+        w = csv.writer(fh)
+        w.writerow(["Step", "Plane"] + _boundary_bond_names() + _texture_bin_names(edges_deg) + ["SumCos"])
+        for step, bonds, hist, f in boundaries:
+            for z in range(hist.shape[0]):
+                w.writerow([int(step), z] + [int(v) for v in bonds[z].reshape(21)] + [int(v) for v in hist[z]] + [int(f[z])])
+
+
+def read_boundary_csv(path):
+    """The records of a boundaries.csv: (edges_deg, [(step, bonds (L, 7, 3), hist (L, m + 1), sum_cos (L,)) per metrics
+    row]), the arrays int64 and the edges read back from the bin names."""
+    import csv
+    with open(path) as fh:
+        rd = csv.reader(fh)
+        head = next(rd)
+        rows = [[int(v) for v in r] for r in rd]
+    bins = head[23:-1]
+    edges = tuple(float(b.split("-")[1]) for b in bins[:-1])
+    out = []
+    for r in rows:
+        if not out or out[-1][0] != r[0]:
+            out.append((r[0], []))
+        out[-1][1].append(r)
+    recs = []
+    for step, rs in out:
+        a = np.array(rs, np.int64)
+        recs.append((step, a[:, 2:23].reshape(-1, 7, 3).copy(), a[:, 23:-1].copy(), a[:, -1].copy()))
+    return edges, recs
+
+
 def read_shape_csv(path):
     """The last metrics row's histogram of a grain_shape.csv: (step, (2, n_edges + 2) int64 array, edges)."""
     import csv
@@ -400,7 +455,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
                        nu_dep=None, laser=None, thermal_every=_ks.THERMAL_EVERY, device=0, seed=None,
                        checkpoint_every=0, resume_from=None, lattice=None, verbose=True, rank=0, world=1,
                        mask_stream="numpy", init_seed=None, profile_axis=None, shape_axis=None, front_axis=None,
-                       texture_axis=None):
+                       texture_axis=None, boundary_axis=None):
     """run_kmc's large-lattice sibling.  Same set-up (initialize_lattice + introduce_defects with the
     run's seed), same cadence and CSV; the steps are synchronous-sublattice sweeps (csrc/sweep.cu), so
     `Step` counts sweeps and `Time` is the accumulated sweep interval.
@@ -432,6 +487,11 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
            outputs/<prefix>/texture.csv with the columns Step, Plane, Solid, SumCos, SumCos2 and one count per angle
            bin, one row per (metrics row, plane).  Every other output is the same as without it.  Not with world > 1,
            checkpoint_every or resume_from.
+    boundary_axis: None, or 0, 1 or 2: the growth axis; every metrics row also takes the per-plane bond counts and
+           boundary misorientation histograms of the row's labelling along it (cetkmc.boundary_group with its default
+           edges), written to outputs/<prefix>/boundaries.csv with the columns Step, Plane, the 21 bond counts, one
+           count per misorientation bin and SumCos, one row per (metrics row, plane).  Every other output is the same
+           as without it.  Not with world > 1, checkpoint_every or resume_from.
     world > 1: the lattice is split into z-slabs, one per rank / GPU (launch every rank with the same
            arguments plus its rank; torch.distributed.run provides the rendezvous).  The trajectory and
            the CSV do not depend on the number of slabs.  Rank 0 writes the CSV; every rank returns its
@@ -453,6 +513,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     _check_axis_kw("run_cet_sublattice", "shape_axis", shape_axis, world, checkpoint_every, resume_from)
     _check_axis_kw("run_cet_sublattice", "front_axis", front_axis, world, checkpoint_every, resume_from)
     _check_axis_kw("run_cet_sublattice", "texture_axis", texture_axis, world, checkpoint_every, resume_from)
+    _check_axis_kw("run_cet_sublattice", "boundary_axis", boundary_axis, world, checkpoint_every, resume_from)
     np.random.seed(seed)                                    # a resumed run restores the stream position below
     output_dir = f"outputs/{output_prefix}"
     os.makedirs(output_dir, exist_ok=True)
@@ -469,7 +530,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
     try:
         ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
         sweep0, total_time, nucleation_count, cet_detected, rows, profiles, shapes, fronts = 0, 0.0, 0, False, [], [], [], []
-        textures = []
+        textures, boundaries = [], []
         if resume_from:
             meta = resume(ctx, resume_from)
             sweep0, total_time = int(meta.get("sweep", 0)), float(meta.get("time", 0.0))
@@ -527,6 +588,9 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             if texture_axis is not None:
                 hist, f1, f2 = _lib.texture_group([ctx], texture_axis)
                 textures.append((sweep - 1, hist[0], f1[0], f2[0]))
+            if boundary_axis is not None:
+                bonds, hist, f = _lib.boundary_group([ctx], boundary_axis)
+                boundaries.append((sweep - 1, bonds[0], hist[0], f[0]))
             if checkpoint_every and (len(rows) % checkpoint_every == 0):
                 checkpoint(ctx, os.path.join(output_dir, "checkpoint"), sweep=sweep, time=total_time,
                            nucleation_count=nucleation_count, cet_detected=cet_detected,
@@ -537,6 +601,7 @@ def run_cet_sublattice(L=None, n_sweeps=2000, temp=None, defect_fraction=0.0, n_
             _write_shape_csv(shapes, output_dir)
             _write_front_csv(fronts, output_dir)
             _write_texture_csv(textures, output_dir)
+            _write_boundary_csv(boundaries, output_dir)
         f = ctx.download(state=True, atom_type=True, theta=True, phi=True)
     finally:
         ctx.close()
@@ -584,7 +649,9 @@ def run_gr_sweep(temps, nu_deps, L=64, n_sweeps=400, impurity_c=0.0, n_seeds=20,
     front_axis=a (through **kw): every case writes outputs/<prefix>/front.csv (run_cet_sublattice), and each rank
     writes cet_map_front_rank<r>.csv (_map_front_rows); every other file is the same as without it.
     texture_axis=a (through **kw): every case writes outputs/<prefix>/texture.csv (run_cet_sublattice), and each rank
-    writes cet_map_texture_rank<r>.csv (_map_texture_rows); every other file is the same as without it."""
+    writes cet_map_texture_rank<r>.csv (_map_texture_rows); every other file is the same as without it.
+    boundary_axis=a (through **kw): every case writes outputs/<prefix>/boundaries.csv (run_cet_sublattice), and each
+    rank writes cet_map_boundary_rank<r>.csv (_map_boundary_rows); every other file is the same as without it."""
     cases = [(float(t), float(r)) for t in temps for r in nu_deps]
 
     def case_row(q):
@@ -612,6 +679,7 @@ def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses
     _check_axis_kw(fn, "shape_axis", kw.get("shape_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_axis_kw(fn, "front_axis", kw.get("front_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_axis_kw(fn, "texture_axis", kw.get("texture_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
+    _check_axis_kw(fn, "boundary_axis", kw.get("boundary_axis"), 1, kw.get("checkpoint_every"), kw.get("resume_from"))
     _check_mask_and_laser(fn, kw.get("mask_stream", "numpy"), lasers is not None or kw.get("laser"),
                           kw.get("thermal_every", _ks.THERMAL_EVERY))
     if batch is not None:
@@ -631,7 +699,8 @@ def _run_map(fn, name, axes, case_row, output_root, cases, lasers, batch_refuses
                                lasers=None if lasers is None else [lasers[lats[l][0]] for l in ls],
                                replicas=None if replicas is None else [lats[l][1] for l in ls], **kw)
     return _map_outputs(output_root, name, lats, [l for _d, ls in parts for l in ls], case_row, axes, replicas, rank,
-                        world, kw.get("profile_axis"), kw.get("shape_axis"), kw.get("front_axis"), kw.get("texture_axis"))
+                        world, kw.get("profile_axis"), kw.get("shape_axis"), kw.get("front_axis"), kw.get("texture_axis"),
+                        kw.get("boundary_axis"))
 
 
 _MAP_FINAL = ("Step", "Time", "AspectRatio", "EquiaxedFraction", "GrainCount", "AvgGrainSize", "NucleationCount",
@@ -667,13 +736,14 @@ def _replica_kw(kw, replicas, r):
 
 
 def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, world, profile_axis=None,
-                 shape_axis=None, front_axis=None, texture_axis=None):
+                 shape_axis=None, front_axis=None, texture_axis=None, boundary_axis=None):
     """The per-rank files of a map driver over the lattices `mine` (indices into `lats`) this rank ran:
     <name>_rank<rank>.csv (case, case_row(case), the final row's _MAP_FINAL columns) and the plot_cet tree from
     replica 0 of each case, with replicas <name>_replicas_rank<rank>.csv, one row per (case, replica), with
     profile_axis <name>_profile_rank<rank>.csv (_map_profile_rows) and with shape_axis <name>_shape_rank<rank>.csv
     (_map_shape_rows), with front_axis <name>_front_rank<rank>.csv (_map_front_rows), with texture_axis
-    <name>_texture_rank<rank>.csv (_map_texture_rows).  Returns the map rows; with
+    <name>_texture_rank<rank>.csv (_map_texture_rows), with boundary_axis <name>_boundary_rank<rank>.csv
+    (_map_boundary_rows).  Returns the map rows; with
     replicas (map rows,
     ensemble_stats of the replica rows), the latter None when world > 1 (merge_* joins the ranks)."""
     import csv
@@ -698,6 +768,9 @@ def _map_outputs(output_root, name, lats, mine, case_row, axes, replicas, rank, 
     if texture_axis is not None:
         _write_rows(_map_texture_rows(lats, sorted(mine), case_row, axes),
                     os.path.join(out_dir, f"{name}_texture_rank{rank}.csv"))
+    if boundary_axis is not None:
+        _write_rows(_map_boundary_rows(lats, sorted(mine), case_row, axes, boundary_axis),
+                    os.path.join(out_dir, f"{name}_boundary_rank{rank}.csv"))
     write_plot_cet_tree([(row["case"], f"outputs/{lats[l][2]}/metrics.csv")
                          for row, l in zip(rows, sorted(l for l in mine if lats[l][1] == 0))],
                         os.path.join(out_dir, "plot_cet"))
@@ -816,12 +889,38 @@ def _map_texture_rows(lats, mine, case_row, axes):
     return out
 
 
+BOUNDARY_ENSEMBLE = ("InterceptAlong", "InterceptAcross", "InterceptAnisotropy", "BoundaryFraction")
+
+
+def _map_boundary_rows(lats, mine, case_row, axes, axis):
+    """One row per lattice of `mine` (case, replica, the map's axis columns, and metrics.boundary_summary along the
+    growth axis `axis` of the final row's tables in outputs/<prefix>/boundaries.csv)."""
+    out = []
+    for l in mine:
+        q, r, p = lats[l]
+        edges, recs = read_boundary_csv(f"outputs/{p}/{BOUNDARY_CSV}")
+        _step, bonds, hist, f = recs[-1]
+        c = case_row(q)
+        out.append({"case": q, "replica": r, **{k: c[k] for k in axes},
+                    **_metrics.boundary_summary(bonds, hist, f, axis, edges)})
+    return out
+
+
+def boundary_ensemble_stats(rows, axes):
+    """texture_ensemble_stats over the columns BOUNDARY_ENSEMBLE of the rows of a <map>_boundary.csv."""
+    return _column_ensemble_stats(rows, axes, BOUNDARY_ENSEMBLE)
+
+
 def texture_ensemble_stats(rows, axes):
     """One row per case over the rows of a <map>_texture.csv (dicts with case, replica, the axis columns `axes` and
     TEXTURE_ENSEMBLE; numbers or the strings a CSV gives back), in case order: case, the axes, replicas (n), and per
     column of TEXTURE_ENSEMBLE <col>_mean and <col>_se over the replicas where it is defined (not ""): the mean, and
     the sample standard deviation, ddof=1, over the square root of their number (empty below 2; the mean empty when
     none)."""
+    return _column_ensemble_stats(rows, axes, TEXTURE_ENSEMBLE)
+
+
+def _column_ensemble_stats(rows, axes, columns):
     by_case = {}
     for r in rows:
         by_case.setdefault(int(r["case"]), []).append(r)
@@ -829,7 +928,7 @@ def texture_ensemble_stats(rows, axes):
     for case in sorted(by_case):
         rs = by_case[case]
         e = {"case": case, **{k: rs[0][k] for k in axes}, "replicas": len(rs)}
-        for col in TEXTURE_ENSEMBLE:
+        for col in columns:
             v = np.array([float(r[col]) for r in rs if r[col] != ""])
             e[f"{col}_mean"] = float(np.mean(v)) if v.size else ""
             e[f"{col}_se"] = float(np.std(v, ddof=1) / np.sqrt(v.size)) if v.size > 1 else ""
@@ -887,7 +986,7 @@ def ensemble_stats(rows, axes):
 def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction, device, metrics_every=None,
                        events_per_sweep=None, p_max=0.1, thermal_every=_ks.THERMAL_EVERY, seed=None, mask_stream="numpy",
                        lasers=None, replicas=None, profile_axis=None, shape_axis=None, front_axis=None,
-                       texture_axis=None):
+                       texture_axis=None, boundary_axis=None):
     """run_cet_sublattice(output_prefix=p, temp=t, nu_dep=r, ...) for every (p, t, r) of `cases` on one device, the
     lattices advancing together by sweep_run_group.  Each case has its own set-up, cadence and metrics.csv exactly as
     alone; with mask_stream="numpy" each case keeps its own position in NumPy's global stream (saved and restored
@@ -905,12 +1004,14 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
     shape_axis: the same with one cetkmc.grain_shape_group call per row, and the grain_shape.csv of
     run_cet_sublattice(shape_axis=...); front_axis: one cetkmc.front_group call per row, and the front.csv of
     run_cet_sublattice(front_axis=...); texture_axis: one cetkmc.texture_group call per row, and the texture.csv of
-    run_cet_sublattice(texture_axis=...)."""
+    run_cet_sublattice(texture_axis=...); boundary_axis: one cetkmc.boundary_group call per row, and the boundaries.csv
+    of run_cet_sublattice(boundary_axis=...)."""
     _check_mask_and_laser("_run_cases_grouped", mask_stream, lasers is not None, thermal_every)
     _check_axis_kw("_run_cases_grouped", "profile_axis", profile_axis)
     _check_axis_kw("_run_cases_grouped", "shape_axis", shape_axis)
     _check_axis_kw("_run_cases_grouped", "front_axis", front_axis)
     _check_axis_kw("_run_cases_grouped", "texture_axis", texture_axis)
+    _check_axis_kw("_run_cases_grouped", "boundary_axis", boundary_axis)
     seed = constants.RANDOM_SEED if seed is None else int(seed)
     every = constants.METRIC_UPDATE_STEP if metrics_every is None else int(metrics_every)
     philox_mask = mask_stream == "philox"
@@ -925,7 +1026,7 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
             ctx.init_seed = None if replicas is None else 42 + reps[q]
             ctx.init_nuclei = []
             r = dict(ctx=ctx, prefix=prefix, seed=seed_q, consts=_gr(L, temp, nu_dep), rows=[], profiles=[], shapes=[], fronts=[],
-                     textures=[], total_time=0.0,
+                     textures=[], boundaries=[], total_time=0.0,
                      nucleation_count=0, cet_detected=False, terminated=False)
             runs.append(r)
             ctx.set_rate_params(rate_params(impurity_c, 1, 2, 3, overrides={"NU_DEP": nu_dep}))
@@ -958,17 +1059,18 @@ def _run_cases_grouped(cases, L, n_sweeps, impurity_c, n_seeds, defect_fraction,
                 stopped = [r for r in active if r["terminated"]]
                 if stopped:
                     _cadence_group(stopped, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis, front_axis,
-                                   texture_axis)
+                                   texture_axis, boundary_axis)
                     active = [r for r in active if not r["terminated"]]
             if active:
                 _cadence_group(active, sweep - 1, every, philox_mask, seed, profile_axis, shape_axis, front_axis,
-                               texture_axis)
+                               texture_axis, boundary_axis)
         for r in runs:
             _ks._write_csv(r["rows"], f"outputs/{r['prefix']}")
             _write_profile_csv(r["profiles"], f"outputs/{r['prefix']}")
             _write_shape_csv(r["shapes"], f"outputs/{r['prefix']}")
             _write_front_csv(r["fronts"], f"outputs/{r['prefix']}")
             _write_texture_csv(r["textures"], f"outputs/{r['prefix']}")
+            _write_boundary_csv(r["boundaries"], f"outputs/{r['prefix']}")
     finally:
         for r in runs:
             r["ctx"].close()
@@ -1027,7 +1129,9 @@ def run_melt_pool_map(powers, speeds, L=64, n_sweeps=400, temp=None, nu_dep=None
     writes melt_pool_map_front_rank<r>.csv (_map_front_rows) with the measured G_Front and V_Front of every lattice
     beside the nominal G and R; every other file is the same as without it.
     texture_axis=a (through **kw): every case writes outputs/<prefix>/texture.csv (run_cet_sublattice), and each rank
-    writes melt_pool_map_texture_rank<r>.csv (_map_texture_rows); every other file is the same as without it."""
+    writes melt_pool_map_texture_rank<r>.csv (_map_texture_rows); every other file is the same as without it.
+    boundary_axis=a (through **kw): every case writes outputs/<prefix>/boundaries.csv (run_cet_sublattice), and each
+    rank writes melt_pool_map_boundary_rank<r>.csv (_map_boundary_rows); every other file is the same as without it."""
     powers, speeds = [float(p) for p in powers], [float(v) for v in speeds]
     if not powers or not speeds:
         raise ValueError("run_melt_pool_map: needs at least one power and one speed")
@@ -1106,6 +1210,9 @@ def _merge_map(output_root, name, axes):
     texture = _merge_rank_files(output_root, f"{name}_texture")
     if texture and reps:
         _write_rows(texture_ensemble_stats(texture, axes), f"outputs/{output_root}/{name}_texture_ensemble.csv")
+    boundary = _merge_rank_files(output_root, f"{name}_boundary")
+    if boundary and reps:
+        _write_rows(boundary_ensemble_stats(boundary, axes), f"outputs/{output_root}/{name}_boundary_ensemble.csv")
     return rows
 
 
@@ -1116,7 +1223,8 @@ def merge_cet_map(output_root="gr_sweep"):
     cet_map_profile_ensemble.csv (profile_ensemble_stats); after a run with shape_axis also cet_map_shape.csv and, with
     replicas, cet_map_shape_ensemble.csv (shape_ensemble_stats); after a run with front_axis also cet_map_front.csv and,
     with replicas, cet_map_front_ensemble.csv (front_ensemble_stats); after a run with texture_axis also
-    cet_map_texture.csv and, with replicas, cet_map_texture_ensemble.csv (texture_ensemble_stats)."""
+    cet_map_texture.csv and, with replicas, cet_map_texture_ensemble.csv (texture_ensemble_stats); after a run with
+    boundary_axis also cet_map_boundary.csv and, with replicas, cet_map_boundary_ensemble.csv (boundary_ensemble_stats)."""
     return _merge_map(output_root, "cet_map", ("T_sub", "NU_DEP"))
 
 
@@ -1126,5 +1234,7 @@ def merge_melt_pool_map(output_root="melt_pool_map"):
     a run with profile_axis also melt_pool_map_profile.csv and, with replicas, melt_pool_map_profile_ensemble.csv;
     after a run with shape_axis also melt_pool_map_shape.csv and, with replicas, melt_pool_map_shape_ensemble.csv;
     after a run with front_axis also melt_pool_map_front.csv and, with replicas, melt_pool_map_front_ensemble.csv;
-    after a run with texture_axis also melt_pool_map_texture.csv and, with replicas, melt_pool_map_texture_ensemble.csv."""
+    after a run with texture_axis also melt_pool_map_texture.csv and, with replicas, melt_pool_map_texture_ensemble.csv;
+    after a run with boundary_axis also melt_pool_map_boundary.csv and, with replicas,
+    melt_pool_map_boundary_ensemble.csv."""
     return _merge_map(output_root, "melt_pool_map", ("power", "speed", "T_sub", "NU_DEP"))

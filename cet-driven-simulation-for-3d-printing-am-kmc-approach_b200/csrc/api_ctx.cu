@@ -254,7 +254,7 @@ int cet_destroy(cet_ctx *c)
                     c->row_occ, c->row_emp, c->row_dep, c->row_depcnt, c->seg, c->total, c->q_top,
                     c->stage, c->kmc, c->d_py, c->d_np, c->d_sp, c->d_log, c->sweep, c->claim,
                     c->records, c->blk_sum, c->blk_max, c->plane_sum, c->stamp, c->t_changed, c->dirty, c->fired,
-                    c->grain_label, c->grain_gid, c->grain_st, c->group_tab, c->profile_tab, c->grain_mom, c->shape_tab, c->front_tab, c->texture_tab, c->rate_tab, c->cvox, c->pairop, c->tile_flag,
+                    c->grain_label, c->grain_gid, c->grain_st, c->group_tab, c->profile_tab, c->grain_mom, c->shape_tab, c->front_tab, c->texture_tab, c->boundary_tab, c->rate_tab, c->cvox, c->pairop, c->tile_flag,
                     c->delta_send[0], c->delta_send[1], c->delta_recv[0], c->delta_recv[1]};
     for (void *p : ptrs)
         if (p) cudaFree(p);

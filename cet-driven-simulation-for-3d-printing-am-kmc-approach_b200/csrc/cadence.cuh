@@ -231,6 +231,20 @@ __device__ __forceinline__ void grains_union_body(const uint8_t *__restrict__ vo
     }
 }
 
+// ---- caller-given histogram edges (texture_group.cu, boundary_group.cu) ----
+
+// b = #{i : e_i <= c} by bisection over the ascending edges
+__device__ __forceinline__ int tg_bin(const double *e, int n_edges, double c)
+{
+    int lo = 0, hi = n_edges;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (e[mid] <= c) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
 struct GrainStat { int root, size, lo[3], hi[3]; };
 
 // label[s] := root of s.  GID: roots are counted and given dense ids in order of arrival (the grouped path

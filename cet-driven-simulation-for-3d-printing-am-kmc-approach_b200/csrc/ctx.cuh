@@ -189,6 +189,8 @@ struct cet_ctx {
     size_t cap_front_tab = 0;
     void *texture_tab = nullptr;      // per-plane orientation histograms (cet_texture_group) of the groups this context leads, grow-only
     size_t cap_texture_tab = 0;
+    void *boundary_tab = nullptr;     // per-plane bond counts (cet_boundary_group) of the groups this context leads, grow-only
+    size_t cap_boundary_tab = 0;
 
     // per-kernel-kind device timing (cet_profile_*): event pairs recorded around the dominant
     // kernels on the context stream, resolved when the totals are read

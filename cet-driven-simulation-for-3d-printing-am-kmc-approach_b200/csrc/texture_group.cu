@@ -39,18 +39,6 @@ __device__ __forceinline__ int tg_plane(int s, int L, int axis)
     return axis == 0 ? s / (L * L) : axis == 1 ? (s / L) % L : s % L;
 }
 
-// b = #{i : e_i <= c} by bisection over the ascending edges
-__device__ __forceinline__ int tg_bin(const double *e, int n_edges, double c)
-{
-    int lo = 0, hi = n_edges;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (e[mid] <= c) lo = mid + 1;
-        else hi = mid;
-    }
-    return lo;
-}
-
 // dynamic shared memory: unsigned long long f[L][2] (F1, F2), double e[n_edges], unsigned h[L][n_edges + 1]
 template <int CAP>
 __global__ void __launch_bounds__(TG_THREADS) texture_group_kernel(const __grid_constant__ GroupArgs<TgArgs, CAP> g,

@@ -275,6 +275,58 @@ def texture_summary(hist, sum_cos, sum_cos2, edges_deg, aligned_deg=30):
             "AlignedFraction": aligned / n}
 
 
+BOUNDARY_COLUMNS = ("SolidBonds", "BoundaryBonds", "InterfaceBonds", "BoundaryFraction", "InterceptAlong",
+                    "InterceptAcross", "InterceptAnisotropy", "MeanMisorientationCos")
+BOUNDARY_SCALE = 2 ** 32                # cetkmc.boundary_group's fixed-point scale
+
+
+def boundary_summary(bonds, hist, sum_cos, axis, edges_deg, voxel_size=K.VOXEL_SIZE):
+    """The grain-boundary network of one lattice, over all its planes, from the arrays of cetkmc.boundary_group for
+    that lattice along the growth axis `axis`: bonds (L, 7, 3) the bonds per offset r (cetkmc._lib.BOUNDARY_OFFSETS)
+    and class (solid, boundary, interface), hist (L, len(edges_deg) + 1) the boundary bonds per misorientation bin,
+    sum_cos (L,) the fixed-point sum F = sum d * 2^32 of their misorientation cosines d.  S, B and I are the solid,
+    boundary and interface bonds over all offsets; S_x and B_x those of the axial offset along axis x (2 sites).
+        SolidBonds, BoundaryBonds, InterfaceBonds   S, B, I
+        BoundaryFraction       B / S: the share of solid bonds that cross a grain boundary
+        InterceptAlong         2 S_a / B_a * voxel_size (m): the mean linear intercept along the growth axis a (ASTM
+                               E112 on test lines along a through the solid; each axial bond is 2 voxels long)
+        InterceptAcross        2 (S_b + S_c) / (B_b + B_c) * voxel_size: the same on lines along the two other axes
+        InterceptAnisotropy    InterceptAlong / InterceptAcross = S_a (B_b + B_c) / (B_a (S_b + S_c)): above 1 for
+                               grains elongated along a (columnar), about 1 for equiaxed ones
+        MeanMisorientationCos  F / (B 2^32): the mean cosine of the boundary misorientation
+    Each ratio of bonds is one correctly rounded quotient of exact integers (the intercepts then times voxel_size);
+    "" where a denominator is 0.
+    The null of the model's nucleation draw: theta ~ U(0, pi) and phi ~ U(0, 2 pi) give E[v] = 0, so two independent
+    draws have mean cosine 0.  A boundary bond, though, joins two occupied sites the labelling left in different grains,
+    so its misorientation exceeds the labelling threshold (0.5 rad; d <= cos 0.5, to within the labelling's rounding):
+    the null of a boundary bond is that draw truncated to d <= cos 0.5, which keeps 91.76 % of the pairs and has mean
+    cosine -0.0847 and, over the default 10-degree bins in ascending angle, the shares 0, 0, 0.0072, 0.0593, 0.0679,
+    0.0746, 0.0794, 0.0825, 0.0841, 0.0841, 0.0825, 0.0794, 0.0746, 0.0679, 0.0593, 0.0483, 0.0342, 0.0145
+    (tests/test_boundary_host.py: Gauss-Legendre quadrature over theta and theta', the difference of the phi
+    integrated in closed form)."""
+    e = [float(x) for x in edges_deg]
+    bd, h, f = np.asarray(bonds), np.asarray(hist), np.asarray(sum_cos)
+    if bd.ndim != 3 or bd.shape[1:] != (7, 3) or h.shape != (bd.shape[0], len(e) + 1) or f.shape != (bd.shape[0],):
+        raise ValueError(f"boundary_summary: need (L, 7, 3) bonds, an (L, {len(e) + 1}) histogram and an (L,) sum, got "
+                         f"shapes {bd.shape}, {h.shape}, {f.shape}")
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or int(axis) not in (0, 1, 2):
+        raise ValueError(f"boundary_summary: axis must be 0, 1 or 2, got {axis!r}")
+    tot = [[int(x) for x in row] for row in bd.sum(axis=0)]                     # [r][class] over the planes
+    S, B, I = (sum(tot[r][f] for r in range(7)) for f in range(3))
+    if sum(int(x) for x in h.sum(axis=0)) != B:
+        raise ValueError("boundary_summary: the histogram does not hold the boundary bonds")
+    a = int(axis)
+    Sa, Ba = tot[4 + a][0], tot[4 + a][1]
+    Sx = sum(tot[4 + x][0] for x in range(3) if x != a)
+    Bx = sum(tot[4 + x][1] for x in range(3) if x != a)
+    return {"SolidBonds": S, "BoundaryBonds": B, "InterfaceBonds": I,
+            "BoundaryFraction": B / S if S else "",
+            "InterceptAlong": 2 * Sa / Ba * voxel_size if Ba else "",
+            "InterceptAcross": 2 * Sx / Bx * voxel_size if Bx else "",
+            "InterceptAnisotropy": Sa * Bx / (Ba * Sx) if Ba and Bx else "",
+            "MeanMisorientationCos": sum(int(x) for x in f) / (B * BOUNDARY_SCALE) if B else ""}
+
+
 def grains_distributed(ctx, all_gather, theta_threshold=0.5):
     """Grains of a lattice that is split into z-slabs over several contexts (one per rank), in the form
     Context.grains() returns for a whole lattice — the reference's clusters (utils.py:28-84) in its

@@ -379,6 +379,39 @@ int cet_front_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, int32_t *
  * D2H copy, one host synchronisation. */
 int cet_texture_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, const double *edges, int32_t n_edges,
                       int64_t *out);
+/* ---- grain boundaries along a growth axis: per-plane bond counts and boundary misorientation of a group ----
+ * Bonds.  The graph is the 14-offset neighbourhood of the labelling's union pass (grains_union_body; the reference's
+ * get_bcc_neighbors, kmc_event_rates.py:29-36).  Each unordered bond is counted once, from its site s through one of
+ * the 7 positive offsets in the labelling's order {0, 1, 4, 5, 8, 10, 12} of CET_NB_TABLE_INIT:
+ *   r = 0 .. 6 -> (1,1,0), (1,-1,0), (0,1,1), (0,1,-1), (2,0,0), (0,2,0), (0,0,2)   (di, dj, dk; s = (i L + j) L + k)
+ * A bond counts only when both ends are inside the lattice: there is no wrap, and the labelling has none either.
+ * Every offset keeps i + j + k even or odd, so the two parity classes of sites never share a bond, and a test line
+ * along an axis steps by 2.
+ * Occupancy and grains come from the last labelling (cet_grains_label[_ex] or cet_metrics_group), as in
+ * cet_grain_profile_group: a site is occupied when label[s] >= 0, and two occupied ends are in the same grain when
+ * their labels are equal.  The orientation is the resident unit vector v (cet_device_ptr field 5; x, y, z).
+ * Bond classes: solid, both ends occupied; boundary, solid and the labels differ; interface, exactly one end occupied
+ * (the solid-liquid surface).
+ * Misorientation of a boundary bond: d = clamp(fl(fl(fl(x x') + fl(y y')) + fl(z z')), -1, 1), every product and sum
+ * one round-to-nearest IEEE operation (no contraction), the clamp pymax(pymin(d, 1), -1).  It is binned over the
+ * interior cosine edges e_0 < ... < e_{m-1} (m = n_edges, 1 <= m <= 31; finite, within [-1, 1], strictly ascending)
+ * at b = #{i : e_i <= d}, as cet_texture_group bins; the exact fixed-point sum is F = sum llrint(d * 2^32) over the
+ * boundary bonds (round half to even).  The labelling decided "same grain" with its own dot product, which may be
+ * contracted, so a boundary bond's misorientation is at least the labelling's threshold only to within that rounding.
+ * Plane of a bond along axis a: min(c_a(s), c_a(t)), the lower of its ends' coordinates along a.
+ * out[((q * L) + z) * W + j] for context q and plane z along `axis`, W = 21 + (m + 1) + 1: j = 3 r + f the bonds of
+ * offset r in plane z of class f (0 solid, 1 boundary, 2 interface); j = 21 + b the boundary bonds of plane z (all
+ * offsets) in bin b; j = 21 + m + 1 their F.  A plane holds at most 7 L^2 bonds and a whole lattice has L < 1291, so no
+ * count or sum overflows.
+ * The contexts must be distinct whole-lattice contexts (no slabs) of one cubic L on one device, 1 <= n_ctx <= 64, each
+ * labelled over the whole lattice, and the per-CTA table of 8 L + 8 m + 4 L (22 + m) bytes must fit the device's
+ * opt-in shared memory per block.  Everything is checked before anything is launched or written: a rejected call leaves
+ * every context and `out` as they were.  The call is read-only on every field, the labels and the mask, so the next
+ * sweep, metrics row, profile, shape, front and texture are what they would have been without it.  The work is ordered
+ * on the stream of ctxs[0] after the work already queued on every context's stream: one memset, one launch for the
+ * whole group, one D2H copy, one host synchronisation. */
+int cet_boundary_group(cet_ctx *const *ctxs, int32_t n_ctx, int32_t axis, const double *edges, int32_t n_edges,
+                       int64_t *out);
 /* The same for global planes [i_lo, i_hi) within the labelled planes of a slab (owned + 2 ghost planes per
  * cut face): what two neighbouring slabs compare to join the grains that cross their cut. */
 int cet_grains_download_planes(cet_ctx *ctx, int64_t i_lo, int64_t i_hi, int32_t *labels);

@@ -21,6 +21,10 @@ cet_map_front_ensemble.csv.
 --texture-axis a: every case also records the per-plane orientation histograms of its occupied sites along growth
 axis a in <case>/texture.csv; rank 0 writes cet_map_texture.csv (mean cosine, Hermans factor and aligned fraction of every
 lattice) and prints it, and with --replicas also cet_map_texture_ensemble.csv.
+--boundary-axis a: every case also records the per-plane bond counts and boundary misorientation histograms of its
+labelling along growth axis a in <case>/boundaries.csv; rank 0 writes cet_map_boundary.csv (linear intercepts along and
+across the axis, their ratio, boundary fraction and mean misorientation of every lattice) and prints it, and with
+--replicas also cet_map_boundary_ensemble.csv.
 """
 import argparse
 import csv
@@ -47,6 +51,7 @@ def main():
     ap.add_argument("--shape-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--front-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--texture-axis", type=int, default=None, choices=(0, 1, 2))
+    ap.add_argument("--boundary-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     temps = [2600.0, 2800.0, 3000.0, 3200.0]                      # T_sub -> G = (T_MELT - T_sub) / (L dx)
@@ -57,7 +62,8 @@ def main():
                                  **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}),
                                  **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}),
                                  **({} if args.front_axis is None else {"front_axis": args.front_axis}),
-                                 **({} if args.texture_axis is None else {"texture_axis": args.texture_axis}))
+                                 **({} if args.texture_axis is None else {"texture_axis": args.texture_axis}),
+                                 **({} if args.boundary_axis is None else {"boundary_axis": args.boundary_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -74,6 +80,11 @@ def main():
         for r in merged:
             print(f"case {int(r['case']):2d} T_sub {float(r['T_sub']):6.0f} NU_DEP {float(r['NU_DEP']):8.1e} G/R {float(r['G_over_R']):9.3e} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} {r['CET_Class']}")
+        if args.boundary_axis is not None:
+            for fn in ("cet_map_boundary.csv",) + (("cet_map_boundary_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.texture_axis is not None:
             for fn in ("cet_map_texture.csv",) + (("cet_map_texture_ensemble.csv",) if args.replicas is not None else ()):
                 with open(f"outputs/{args.out}/{fn}") as fh:

@@ -21,6 +21,10 @@ melt_pool_map_front_ensemble.csv.
 --texture-axis a: every case also records the per-plane orientation histograms of its occupied sites along growth
 axis a in <case>/texture.csv; rank 0 writes melt_pool_map_texture.csv (mean cosine, Hermans factor and aligned fraction of every
 lattice) and prints it, and with --replicas also melt_pool_map_texture_ensemble.csv.
+--boundary-axis a: every case also records the per-plane bond counts and boundary misorientation histograms of its
+labelling along growth axis a in <case>/boundaries.csv; rank 0 writes melt_pool_map_boundary.csv (linear intercepts along and
+across the axis, their ratio, boundary fraction and mean misorientation of every lattice) and prints it, and with
+--replicas also melt_pool_map_boundary_ensemble.csv.
 """
 import argparse
 import csv
@@ -46,6 +50,7 @@ def main():
     ap.add_argument("--shape-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--front-axis", type=int, default=None, choices=(0, 1, 2))
     ap.add_argument("--texture-axis", type=int, default=None, choices=(0, 1, 2))
+    ap.add_argument("--boundary-axis", type=int, default=None, choices=(0, 1, 2))
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     powers = [100.0, 200.0, 300.0, 400.0]                         # W
@@ -57,7 +62,8 @@ def main():
                                **({} if args.profile_axis is None else {"profile_axis": args.profile_axis}),
                                **({} if args.shape_axis is None else {"shape_axis": args.shape_axis}),
                                **({} if args.front_axis is None else {"front_axis": args.front_axis}),
-                               **({} if args.texture_axis is None else {"texture_axis": args.texture_axis}))
+                               **({} if args.texture_axis is None else {"texture_axis": args.texture_axis}),
+                               **({} if args.boundary_axis is None else {"boundary_axis": args.boundary_axis}))
     dt = time.perf_counter() - t0
     # replicas only: the one rendezvous is "everybody is done" before rank 0 merges the per-rank files
     if world > 1:
@@ -75,6 +81,11 @@ def main():
             print(f"case {int(r['case']):2d} P {float(r['power']):6.1f} W V {float(r['speed']):5.2f} "
                   f"AR {float(r['AspectRatio']):.3f} eq {float(r['EquiaxedFraction']):.3f} grains {int(float(r['GrainCount']))} "
                   f"step {r['Step']} {r['CET_Class']}")
+        if args.boundary_axis is not None:
+            for fn in ("melt_pool_map_boundary.csv",) + (("melt_pool_map_boundary_ensemble.csv",) if args.replicas is not None else ()):
+                with open(f"outputs/{args.out}/{fn}") as fh:
+                    for e in csv.DictReader(fh):
+                        print(json.dumps(e))
         if args.texture_axis is not None:
             for fn in ("melt_pool_map_texture.csv",) + (("melt_pool_map_texture_ensemble.csv",) if args.replicas is not None else ()):
                 with open(f"outputs/{args.out}/{fn}") as fh:
